@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — env-actions/sec of the batched env dynamics on N B200s (one process per GPU).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--env shkadov] [--batch B] [--extras all|none|a,b]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--env shkadov] [--batch B] [--extras all|none|a,b] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference ...      # the UNMODIFIED reference (numpy + numba) on the host cores
 
@@ -52,7 +52,9 @@ DEFAULT_EXTRAS = ("rayleigh", "shkadov_b4096", "shkadov_separable", "mixing", "b
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=None)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps of the headline workload; the other batched workloads time at most this many "
+                         "(the burgers and VectorEnv episodes keep their episode lengths)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--env", default="shkadov", choices=sorted(WORKLOADS))
@@ -62,7 +64,34 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-gather", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step of the headline workload returned (rank 0) as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the CUDA path: it needs --impl b200")
+    return args
+
+
+DUMP_LIMIT = 64 * 1024 * 1024
+
+
+def dump_outputs(path, obs, rwd, done, trunc):
+    """obs / reward / done / truncated of one batched step as float64 (flags as float32) .npy files.  A batch whose
+    arrays exceed DUMP_LIMIT is written as a fixed sample of env rows, listed in sample_rows.npy."""
+    arrs = {"obs": obs.double(), "reward": rwd.double(), "done": done.float(), "truncated": trunc.float()}
+    arrs = {k: a.cpu().numpy() for k, a in arrs.items()}
+    B = obs.shape[0]
+    row_bytes = sum(a[0].nbytes for a in arrs.values())
+    os.makedirs(path, exist_ok=True)
+    if B * row_bytes > DUMP_LIMIT:
+        n = (DUMP_LIMIT - 4096) // (row_bytes + 8)                  # 4096: room for the .npy headers
+        rows = np.sort(np.random.default_rng(0).choice(B, n, replace=False))
+        np.save(os.path.join(path, "sample_rows.npy"), rows.astype(np.float64))
+        arrs = {k: a[rows] for k, a in arrs.items()}
+    for k, a in arrs.items():
+        np.save(os.path.join(path, k + ".npy"), a)
 
 
 # --------------------------------------------------------------------------------------------
@@ -398,7 +427,7 @@ def run_workload(wl, B, K, W, cx, args, headline):
         for k in range(K):
             cx.flush.zero_()                                 # L2 flush between timed iterations (untimed)
             ev[k][0].record()
-            env.step(actions[W + k], want_iters=want_iters)
+            last = env.step(actions[W + k], want_iters=want_iters)
             ev[k][1].record()
             if want_iters:
                 it_sum += env.last_iters.sum()
@@ -412,6 +441,8 @@ def run_workload(wl, B, K, W, cx, args, headline):
             if k % 8 == 0:
                 torch.cuda.synchronize()
         torch.cuda.synchronize()
+    if headline and args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *last)
     ms = [a.elapsed_time(b) for a, b in ev]
     total_ms = float(sum(ms))
     t = torch.tensor([total_ms], device=dev, dtype=torch.float64)
@@ -680,14 +711,9 @@ def main():
                     workloads["shkadov_vector_env_episode"] = {"error": repr(e)[:300]}
             continue
         K2 = min(K2, args.steps) if args.steps else K2
-        K2 = max(K2, 3)
         r = run_workload(w2, B2, K2, W, cx, args, False)
         if rank == 0:
             workloads[w2] = r
-    if wl == "shkadov" and names and K < 200:
-        r = run_workload("shkadov", B, 400, W, cx, argparse.Namespace(**{**vars(args), "no_e2e": True, "no_gather": True}), False)
-        if rank == 0:
-            workloads["shkadov_400_steps"] = {k: r[k] for k in ("value", "ms_per_step", "steps", "clocks")}
 
     if rank == 0:
         line = {

@@ -162,6 +162,12 @@ def test_vortex(golden):
         np.testing.assert_allclose(env.x, g["x"][k], rtol=1e-13, atol=0)
         np.testing.assert_allclose(obs, g["obs"][k], rtol=1e-12, atol=1e-18)
         assert rwd == pytest.approx(g["rwd"][k], rel=1e-9, abs=1e-18)
+    env.reset()
+    sr = sum(env.step(np.array([0.5, -0.25]))[1] for _ in range(10))
+    # SURVEY.md §4 KAT
+    np.testing.assert_allclose(env.x, [-0.010474204824095492, -0.0044519423003400675, -0.0003076860892504164,
+                                       -0.0028289435961359756], rtol=1e-13, atol=0)
+    assert sr == pytest.approx(-0.0021355829919963414, rel=1e-9, abs=1e-18)
 
 
 @pytest.mark.parametrize("name,scal", [("rayleigh", "T"), ("mixing", "C")])

@@ -1,6 +1,7 @@
-"""Live A/B of the oracle against the unmodified reference (only where /root/reference
-exists, i.e. the build container; skipped on the GPU box).  Longer random sequences than
-the golden files; fields bit-exact."""
+"""Live A/B of the oracle against the unmodified reference, wherever oracle/refload.py finds a
+jviquerat/beacon checkout (REF_ROOT: BEACON_REFERENCE, else its default checkout location, else
+the copy oracle/make_ref.py stages under oracle/_ref/); skipped without one.  Longer random
+sequences than the golden files; fields bit-exact."""
 import warnings
 
 import numpy as np
@@ -9,7 +10,7 @@ import pytest
 from oracle import beacon_oracle as bo
 from oracle import refload
 
-pytestmark = pytest.mark.skipif(not refload.available(), reason="reference checkout not present")
+pytestmark = pytest.mark.skipif(not refload.available(), reason=f"no reference checkout at {refload.REF_ROOT} (set BEACON_REFERENCE to a jviquerat/beacon checkout)")
 warnings.simplefilter("ignore")
 
 
