@@ -130,6 +130,7 @@ def test_shkadov_vs_oracle_resync():
     (dict(n_jets=4, jet_space=5.0), False),      # dense jets (spacing 25 < chunk + jet width): per-point jet table
     (dict(n_jets=4, jet_space=3.0, L0=200.0), False),   # overlapping jets (spacing 15 < 21): generic per-jet loop
     (dict(n_jets=10), True),                     # outlet not aligned to a chunk end: per-point index tests
+    (dict(n_jets=20), True),                     # the same on the 10,192,2 instance (nx 1850)
 ])
 def test_shkadov_general_paths_vs_oracle(kw, noalign, monkeypatch):
     """The general (per-point index test) path of the kernel, which the standard configurations no
