@@ -44,7 +44,8 @@ VortexParams = _struct("VortexParams", ("ndt_act", "n_act"),
 MacParams = _struct("MacParams",
                     ("nx", "ny", "ndt_act", "n_act", "n_sgts", "nx_sgts", "nx_obs_pts", "ny_obs_pts", "n_obs_steps",
                      "nx_obs", "ny_obs", "itmax"),
-                    ("dx", "dy", "dt", "pr", "ra", "Tc", "Th", "C", "re", "pe", "u_max", "ref_c", "tol"))
+                    ("dx", "dy", "dt", "pr", "ra", "Tc", "Th", "C", "re", "pe", "u_max", "ref_c", "tol"),
+                    (("ctas_per_env", _i32),))
 
 
 class EnvInfo(C.Structure):

@@ -29,16 +29,23 @@ class BatchedEnv:
     step(actions, noise=None)     -> obs [B, n_obs], rwd [B] (or [B, n_jets]), done [B], trunc [B]
     step_fused(actions[K,B,...])  -> same with a leading K axis: K consecutive actions, one launch
     get_state(name) / set_state(name, tensor)
+
+    ctas_per_env (rayleigh / mixing): how many SMs one environment may occupy.  1 runs each env on one
+    CTA (grids up to ~100x100 cells); 2..8 split each env over a thread-block cluster of that many CTAs,
+    which reaches larger grids (DESIGN.md §3.6).  The state layout is the same for every value.
     """
 
-    def __init__(self, name, batch, device=0, dtype=torch.float64, seed=0, env_index_base=0, init_state=None, **kwargs):
+    def __init__(self, name, batch, device=0, dtype=torch.float64, seed=0, env_index_base=0, init_state=None,
+                 ctas_per_env=1, **kwargs):
         if name not in CFG:
             raise ValueError(f"unknown env '{name}' (have {sorted(CFG)})")
         if dtype not in (torch.float64, torch.float32):
             raise ValueError(f"dtype must be torch.float64 or torch.float32 (the arithmetic types of the kernels), got {dtype}")
+        if ctas_per_env != 1 and name not in ("rayleigh", "mixing"):
+            raise ValueError(f"ctas_per_env applies to the MAC-grid envs (rayleigh, mixing), not to {name}")
         if not torch.cuda.is_available():
             raise capi.BeaconError("beacon_b200 needs a CUDA device (B200, sm_100a); there is no CPU fallback")
-        self.name, self.batch, self.dtype = name, int(batch), dtype
+        self.name, self.batch, self.dtype, self.ctas_per_env = name, int(batch), dtype, int(ctas_per_env)
         self.device = torch.device("cuda", device)
         self.cfg = CFG[name](**kwargs)
         d = self.cfg.d
@@ -88,13 +95,14 @@ class BatchedEnv:
                 c = self.cfg
                 p = capi.MacParams(d["nx"], d["ny"], d["ndt_act"], d["n_act"], c.n_sgts, d["nx_sgts"], d["nx_obs_pts"],
                                    d["ny_obs_pts"], d["n_obs_steps"], d["nx_obs"], d["ny_obs"], d["itmax"], d["dx"],
-                                   d["dy"], d["dt"], d["pr"], d["ra"], d["Tc"], d["Th"], d["C"], 0.0, 0.0, 0.0, 0.0, d["tol"])
+                                   d["dy"], d["dt"], d["pr"], d["ra"], d["Tc"], d["Th"], d["C"], 0.0, 0.0, 0.0, 0.0, d["tol"],
+                                   self.ctas_per_env)
                 arrs = [np.ascontiguousarray(d[k + "_init"], dtype=np.float64) for k in "uvpT"]
                 capi.check(L.beacon_rayleigh_create(C.byref(com), C.byref(p), *[_dp(a) for a in arrs], C.byref(h)))
             elif name == "mixing":
                 p = capi.MacParams(d["nx"], d["ny"], d["ndt_act"], d["n_act"], 0, 0, d["nx_obs_pts"], d["ny_obs_pts"],
                                    d["n_obs_steps"], d["nx_obs"], d["ny_obs"], d["itmax"], d["dx"], d["dy"], d["dt"],
-                                   0.0, 0.0, 0.0, 0.0, 0.0, d["re"], d["pe"], d["u_max"], d["ref_c"], d["tol"])
+                                   0.0, 0.0, 0.0, 0.0, 0.0, d["re"], d["pe"], d["u_max"], d["ref_c"], d["tol"], self.ctas_per_env)
                 Ci = np.ascontiguousarray(d["C_init"], dtype=np.float64)
                 capi.check(L.beacon_mixing_create(C.byref(com), C.byref(p), _dp(Ci), C.byref(h)))
         self._h = h

@@ -8,8 +8,8 @@
 // predictor :382-416, poisson :421-465, corrector :470-473, transport :478-495,
 // get_obs :237-256, get_rwd :259-264.
 //
-// B200 design: ONE CTA PER ENVIRONMENT runs every sub-step of every fused action without
-// returning to the host.  Three kernels (DESIGN.md 3.4 / 3.5):
+// B200 design: ONE CTA PER ENVIRONMENT (or one cluster, mac_cluster_kernel) runs every sub-step of
+// every fused action without returning to the host.  Four kernels (DESIGN.md 3.4 - 3.6):
 //   * mac_reg_kernel  — rayleigh 50x50: phi and the Poisson right-hand side of a 2x5 tile in
 //     REGISTERS, in-place Jacobi sweeps over two strided exchange planes (one barrier per sweep),
 //     convergence test two sweeps behind and interleaved with the next sweep (exact sweep counts),
@@ -18,7 +18,11 @@
 //     planes in L2/HBM, tile copies of p, us, vs in a thread-interleaved scratch, u / v staged in
 //     the exchange planes for the predictor (TMA bulk copies), transport in two row passes;
 //   * mac_kernel      — generic fallback for any other grid up to ~100x100 cells: phi ping-pongs
-//     between two shared-memory planes, right-hand side in registers, fields in global memory.
+//     between two shared-memory planes, right-hand side in registers, fields in global memory;
+//   * mac_cluster_kernel — only with ctas_per_env = G in 2..8, on any grid whose row slabs fit
+//     (DESIGN.md 3.6): one env over a cluster of G CTAs, phi slabs in each CTA's shared memory,
+//     halo rows and residual partials through DSMEM, one cluster barrier per sweep, the transport
+//     wavefront chained from rank to rank.
 // Common to all:
 //   * the residual reproduces the reference's: sum over the whole ghost-inclusive array after
 //     the ghost update (ghost copies re-count the wall-adjacent cells; mixing's top ghost is 0);
@@ -39,7 +43,9 @@
 //   MAC_CLUSTER_BARRIER_TEST rayleigh: cluster barrier in place of the CTA barrier of a sweep (cost measurement)
 #include <cstdio>
 #include <cstdlib>
+#include <algorithm>
 #include <cstring>
+#include <string>
 #include <type_traits>
 
 #include "common.cuh"
@@ -58,6 +64,7 @@ template <typename R> struct MacArgs {
     int nx_obs_pts, ny_obs_pts, n_obs_steps, nx_obs, ny_obs, n_obs, tr_pass;
     R dx, dy, dt, inv_dx, inv_dy, inv_dx2, inv_dy2, dx2, dy2, inv_den, pk1, pk2, cscale, dcoef, tcoef, Tc, Th, Cmax, u_max, ref_c, tol;
     int B, mode, n_fused;
+    int G, slab_rows;                  // mac_cluster_kernel: CTAs per env, rows of a phi slab plane (halos included)
     R *u, *v, *p, *s, *us, *vs, *cc;   // [B, n] planes (s = T or C); us/vs/cc are workspaces
     R *a_cur, *obs_hist;
     int32_t *stp, *a_int;
@@ -442,6 +449,434 @@ __global__ void __launch_bounds__(T) mac_kernel(const MacArgs<R> a)
         for (int e = tid; e < n; e += T) { gu[e] = u[e]; gv[e] = v[e]; gp[e] = p[e]; gs[e] = s[e]; a.us[row + e] = us[e]; a.vs[row + e] = vs[e]; }
     }
     if (tid == 0) { a.stp[b] = stp; if (a.status) a.status[b] = status; }
+#undef CELL_LOOP
+#undef CELL_OK
+}
+
+// ---------------------------------------------------------------------------------------
+// mac_cluster_kernel — one environment split over a thread-block cluster of G = a.G CTAs
+// (DESIGN.md 3.6).  Rank g owns the interior rows ib..ie of a balanced slab; the left wall and
+// ghost row 0 go to rank 0, the right wall and ghost row nx+1 to rank G-1.  Fields stay in their
+// global planes as in mac_kernel; each CTA keeps only its slab of the two phi planes (one halo
+// row on each side) in shared memory.  A Jacobi sweep pushes its first and last rows into the
+// neighbours' halo rows through DSMEM and ends in one cluster barrier, where every CTA also
+// receives the per-warp residual partials of every rank.  Phases that read rows written by
+// another CTA follow a cluster barrier (release / acquire).  The transport wavefront of rank
+// g + 1 starts on the new values of rank g's last row, handed over through DSMEM in chunks of
+// MAC_CLUSTER_CHUNK columns, each published with a cluster-scope release / acquire flag.
+// ---------------------------------------------------------------------------------------
+#define MAC_CLUSTER_MAX 8          // portable cluster size
+#define MAC_CLUSTER_MIN_ROWS 4     // rows of the thinnest slab: one tile height
+#define MAC_CLUSTER_MAX_LD 512     // columns (ny + 2) of the wavefront hand-off buffers
+#define MAC_CLUSTER_CHUNK 8        // columns per hand-off flag: a cluster-scope release per chunk, not per column
+#define MAC_CLUSTER_SMEM (200 * 1024)   // dynamic shared memory; the static arrays take the rest of 227 KB
+
+__device__ __forceinline__ void cluster_barrier()
+{
+    asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
+}
+__device__ __forceinline__ unsigned cluster_rank()
+{
+    unsigned r;
+    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
+    return r;
+}
+// generic address of the same shared-memory object in CTA `rank` of the cluster
+template <typename P> __device__ __forceinline__ P *cluster_map(P *p, unsigned rank)
+{
+    uint64_t r;
+    asm volatile("mapa.u64 %0, %1, %2;" : "=l"(r) : "l"(p), "r"(rank));
+    return reinterpret_cast<P *>(r);
+}
+__device__ __forceinline__ void st_release_cluster(int *p, int v)
+{
+    asm volatile("st.release.cluster.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
+}
+__device__ __forceinline__ int ld_acquire_cluster(const int *p)
+{
+    int v;
+    asm volatile("ld.acquire.cluster.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
+    return v;
+}
+
+template <typename R, int TI, int TJ, int T>
+__global__ void __launch_bounds__(T) mac_cluster_kernel(const MacArgs<R> a)
+{
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    __shared__ R s_part[2][MAC_CLUSTER_MAX][T / 32];   // residual partials of every rank, by sweep parity
+    __shared__ R s_red[T / 32];
+    __shared__ R s_rank[MAC_CLUSTER_MAX];             // per-rank reward partials (mixing)
+    __shared__ int s_bad[MAC_CLUSTER_MAX];            // per-rank non-finite flags
+    __shared__ R s_seg[128];
+    __shared__ R s_act[128];
+    __shared__ R s_west[MAC_CLUSTER_MAX_LD];          // new values of rank g-1's last row, by column
+    __shared__ int s_flag[MAC_CLUSTER_MAX_LD / MAC_CLUSTER_CHUNK];   // == substep sequence: chunk of s_west ready
+    const int tid = threadIdx.x, G = a.G;
+    const unsigned rank = cluster_rank();
+    const int b = blockIdx.x / G;
+    const int nx = a.nx, ny = a.ny, ld = a.ld;
+    const bool resetting = a.mode == 1;
+    if (resetting && a.mask && !a.mask[b]) return;     // uniform over the cluster: no DSMEM access yet
+    const bool ray = a.kind == BEACON_RAYLEIGH;
+    const bool first = rank == 0, last = rank == (unsigned)G - 1;
+
+    // ---- slab: rows ib..ie (S rows), balanced to within one row --------------------------------
+    const int base = nx / G, rem = nx % G;
+    const int S = base + ((int)rank < rem), ib = 1 + (int)rank * base + min((int)rank, rem), ie = ib + S - 1;
+    const int S_left = rank > 0 ? base + ((int)rank - 1 < rem) : 0;
+    const int r0 = first ? 0 : ib, r1 = last ? nx + 1 : ie;   // rows of the whole-array passes (ghost rows included)
+    const int e0 = r0 * ld, e1 = (r1 + 1) * ld;
+
+    // ---- planes: phi slabs [S + 2][ld] (local row li = i - ib + 1), fields in global memory --------
+    const int slab = a.slab_rows * ld;
+    R *phiA = reinterpret_cast<R *>(smem_raw), *phiB = phiA + slab;
+    R *lA = nullptr, *lB = nullptr, *rA = nullptr, *rB = nullptr;   // neighbours' halo rows, same planes
+    if (!first) { lA = cluster_map(phiA, rank - 1) + (S_left + 1) * ld; lB = cluster_map(phiB, rank - 1) + (S_left + 1) * ld; }
+    if (!last) { rA = cluster_map(phiA, rank + 1); rB = cluster_map(phiB, rank + 1); }
+    const size_t row = (size_t)b * a.n;
+    R *u = a.u + row, *v = a.v + row, *p = a.p + row, *s = a.s + row, *us = a.us + row, *vs = a.vs + row;
+
+    const int tiles_i = (S + TI - 1) / TI;
+    const bool has_tile = tid < tiles_i * a.tiles_j;
+    const int ti = tid / a.tiles_j, tj = tid - ti * a.tiles_j;
+    const int i0 = ib + ti * TI, j0 = 1 + tj * TJ;
+#define CELL_LOOP                                       \
+    _Pragma("unroll") for (int r = 0; r < TI; r++)      \
+    _Pragma("unroll") for (int k = 0; k < TJ; k++)
+#define CELL_OK(i, j) (has_tile && (i) <= ie && (j) <= ny)
+
+    for (int e = tid; e < MAC_CLUSTER_MAX_LD / MAC_CLUSTER_CHUNK; e += T) s_flag[e] = 0;
+
+    // ---- load / reset (own rows) -----------------------------------------------------------------
+    if (resetting) {
+        for (int e = e0 + tid; e < e1; e += T) {
+            u[e] = ray ? a.u0[e] : R(0); v[e] = ray ? a.v0[e] : R(0); p[e] = ray ? a.p0[e] : R(0); s[e] = a.s0[e];
+            us[e] = R(0); vs[e] = R(0);
+        }
+        if (first) {
+            for (int e = tid; e < a.n_obs; e += T) a.obs_hist[(size_t)b * a.n_obs + e] = R(0);
+            for (int e = tid; e < (ray ? a.n_sgts : 0); e += T) a.a_cur[(size_t)b * a.n_sgts + e] = R(0);
+            if (tid == 0) { a.stp[b] = 0; if (!ray) a.a_int[b] = 1; }
+        }
+        cluster_barrier();
+        if (first) {                                           // history zero, newest slot from the init state
+            R *hist = a.obs_hist + (size_t)b * a.n_obs;
+            const int per_step = 3 * a.nx_obs_pts * a.ny_obs_pts;
+            for (int e = tid; e < a.n_obs; e += T) {
+                int st = e / per_step, rm = e - st * per_step;
+                R val = R(0);
+                if (st == a.n_obs_steps - 1) {
+                    int f = rm / (a.nx_obs_pts * a.ny_obs_pts), q = rm - f * (a.nx_obs_pts * a.ny_obs_pts);
+                    int pi = q / a.ny_obs_pts, pj = q - pi * a.ny_obs_pts;
+                    int x = a.nx_obs / 2 + pi * a.nx_obs, y = a.ny_obs / 2 + pj * a.ny_obs;
+                    val = (f == 0) ? s[x * ld + y] : (f == 1 ? u[x * ld + y] : v[x * ld + y]);
+                }
+                hist[e] = val;
+                a.obs[(size_t)b * a.n_obs + e] = val;
+            }
+        }
+        return;                                                // no DSMEM access after the barrier
+    }
+    int stp = a.stp[b];
+    int status = 0, seq = 0;
+    cluster_barrier();                                         // s_flag cleared in every rank
+
+    for (int act = 0; act < a.n_fused; act++) {
+        const size_t orow = (size_t)act * a.B + b;
+        // ---- action conditioning: every rank computes it, rank 0 stores it -------------------------
+        if (ray) {
+            const R *ain = (const R *)a.actions + orow * a.n_sgts;
+            if (tid == 0) {                                        // rayleigh.py:164-171
+                const int ns = a.n_sgts;
+                for (int j = 0; j < ns; j++) s_act[j] = ain[j];
+                R mean = np_pairwise_small(s_act, ns) / R(ns);
+                R m = R(1);
+                for (int j = 0; j < ns; j++) { s_act[j] = s_act[j] - mean; m = np_max(m, rabs(s_act[j]) / a.Cmax); }
+                for (int j = 0; j < ns; j++) {
+                    s_act[j] = s_act[j] / m; s_seg[j] = a.Th + s_act[j];
+                    if (first) a.a_cur[(size_t)b * ns + j] = s_act[j];
+                }
+            }
+        } else if (tid == 0) {                                     // get_control, mixing.py:212-234
+            int ai = ((const int32_t *)a.actions)[orow];
+            R ut = 0, ub = 0, vl = 0, vr = 0;
+            if (ai == 0) { ub = a.u_max; ut = -a.u_max; }
+            if (ai == 1) { ub = -a.u_max; ut = a.u_max; }
+            if (ai == 2) { vr = a.u_max; vl = -a.u_max; }
+            if (ai == 3) { vr = -a.u_max; vl = a.u_max; }
+            s_seg[0] = ut; s_seg[1] = ub; s_seg[2] = vl; s_seg[3] = vr;
+            if (first) a.a_int[b] = ai;
+        }
+        __syncthreads();
+        long long it_total = 0;
+
+        for (int it = 0; it < a.ndt_act; it++) {
+            seq += 1;
+            // ---- boundary conditions (as mac_kernel), own walls and own i range --------------------
+            {
+                const int nl = first ? ny + 2 : 0, nr = last ? ny + 2 : 0;
+                const int ihi = last ? nx + 1 : ie, ni = ihi - ib + 1;
+                for (int k = tid; k < nl + nr + 2 * ni; k += T) {
+                    if (k < nl) {                                      // left wall (i = 0/1)
+                        int j = k;
+                        if (j >= 1 && j <= ny) { u[1 * ld + j] = R(0); s[0 * ld + j] = s[1 * ld + j]; }
+                        if (j >= 2 && j <= ny) v[0 * ld + j] = ray ? -v[1 * ld + j] : R(2) * s_seg[2] - v[1 * ld + j];
+                    } else if (k < nl + nr) {                          // right wall
+                        int j = k - nl;
+                        if (j >= 1 && j <= ny) { u[(nx + 1) * ld + j] = R(0); s[(nx + 1) * ld + j] = s[nx * ld + j]; }
+                        if (j >= 2 && j <= ny) v[(nx + 1) * ld + j] = ray ? -v[nx * ld + j] : R(2) * s_seg[3] - v[nx * ld + j];
+                    } else if (k < nl + nr + ni) {                     // top wall (j = ny+1)
+                        int i = ib + k - nl - nr;
+                        R ui = (i == 1 || i == nx + 1) ? R(0) : u[i * ld + ny];
+                        u[i * ld + ny + 1] = ray ? -ui : R(2) * s_seg[0] - ui;
+                        if (i <= nx) {
+                            v[i * ld + ny + 1] = R(0);
+                            s[i * ld + ny + 1] = ray ? R(2) * a.Tc - s[i * ld + ny] : s[i * ld + ny];
+                        }
+                    } else {                                           // bottom wall (j = 0/1)
+                        int i = ib + k - nl - nr - ni;
+                        R ui = (i == 1 || i == nx + 1) ? R(0) : u[i * ld + 1];
+                        u[i * ld + 0] = ray ? -ui : R(2) * s_seg[1] - ui;
+                        if (i <= nx) {
+                            v[i * ld + 1] = R(0);
+                            if (ray) {
+                                int sg = (i - 1) / a.nx_sgts;
+                                if (sg < a.n_sgts) s[i * ld + 0] = R(2) * s_seg[sg] - s[i * ld + 1];
+                            } else s[i * ld + 0] = s[i * ld + 1];
+                        }
+                    }
+                }
+            }
+            for (int e = tid; e < 2 * slab; e += T) phiA[e] = R(0);   // both planes: they doubled as transport scratch
+            cluster_barrier();                                 // walls of the neighbours; zeroed halos before any push
+
+            // ---- predictor (own rows; reads the neighbours' wall rows) ---------------------------------
+            CELL_LOOP {
+                const int i = i0 + r, j = j0 + k;
+                if (CELL_OK(i, j)) {
+                    const R uc = u[i * ld + j], vc = v[i * ld + j];
+                    if (i >= 2) {
+                        R uE = R(0.5) * (u[(i + 1) * ld + j] + uc), uW = R(0.5) * (uc + u[(i - 1) * ld + j]);
+                        R uN = R(0.5) * (u[i * ld + j + 1] + uc), uS = R(0.5) * (uc + u[i * ld + j - 1]);
+                        R vN = R(0.5) * (v[i * ld + j + 1] + v[(i - 1) * ld + j + 1]), vS = R(0.5) * (vc + v[(i - 1) * ld + j]);
+                        R conv = (uE * uE - uW * uW) * a.inv_dx + (uN * vN - uS * vS) * a.inv_dy;
+                        R diff = ((u[(i + 1) * ld + j] - R(2) * uc + u[(i - 1) * ld + j]) * a.inv_dx2 +
+                                  (u[i * ld + j + 1] - R(2) * uc + u[i * ld + j - 1]) * a.inv_dy2) * a.dcoef;
+                        R pres = (p[i * ld + j] - p[(i - 1) * ld + j]) * a.inv_dx;
+                        us[i * ld + j] = uc + a.dt * (diff - conv - pres);
+                    }
+                    if (j >= 2) {
+                        R vE = R(0.5) * (v[(i + 1) * ld + j] + vc), vW = R(0.5) * (vc + v[(i - 1) * ld + j]);
+                        R uE = R(0.5) * (u[(i + 1) * ld + j] + u[(i + 1) * ld + j - 1]), uW = R(0.5) * (uc + u[i * ld + j - 1]);
+                        R vN = R(0.5) * (v[i * ld + j + 1] + vc), vS = R(0.5) * (vc + v[i * ld + j - 1]);
+                        R conv = (uE * vE - uW * vW) * a.inv_dx + (vN * vN - vS * vS) * a.inv_dy;
+                        R diff = ((v[(i + 1) * ld + j] - R(2) * vc + v[(i - 1) * ld + j]) * a.inv_dx2 +
+                                  (v[i * ld + j + 1] - R(2) * vc + v[i * ld + j - 1]) * a.inv_dy2) * a.dcoef;
+                        R pres = (p[i * ld + j] - p[i * ld + j - 1]) * a.inv_dy;
+                        R rhs = diff - conv - pres;
+                        if (ray) rhs += s[i * ld + j];
+                        vs[i * ld + j] = vc + a.dt * rhs;
+                    }
+                }
+            }
+            cluster_barrier();                                 // us of row ie + 1 comes from rank g + 1
+
+            // ---- Poisson right-hand side into registers --------------------------------------------------
+            R c[TI][TJ];
+            CELL_LOOP {
+                const int i = i0 + r, j = j0 + k;
+                c[r][k] = R(0);
+                if (CELL_OK(i, j))
+                    c[r][k] = ((us[(i + 1) * ld + j] - us[i * ld + j]) * a.inv_dx + (vs[i * ld + j + 1] - vs[i * ld + j]) * a.inv_dy) * a.cscale;
+            }
+            // ---- Jacobi sweeps: halo rows pushed to the neighbours, one cluster barrier per sweep ------
+            R *pin = phiA, *pout = phiB;
+            R err = R(1.0e10);
+            int itp = 0;
+            while (err > a.tol) {
+                R acc = R(0);
+                R *lout = (itp & 1) ? lA : lB, *rout = (itp & 1) ? rA : rB;   // the neighbours' copies of pout
+                if (has_tile) {
+#pragma unroll
+                    for (int r = 0; r < TI; r++) {
+                        const int i = i0 + r;
+                        if (i <= ie) {
+                            const int li = i - ib + 1;
+                            const R *rc = pin + li * ld + j0, *rw = rc - ld, *re = rc + ld;
+                            R *po = pout + li * ld;
+                            R west = rc[-1], cen = rc[0];
+#pragma unroll
+                            for (int k = 0; k < TJ; k++) {
+                                const int j = j0 + k;
+                                if (j <= ny) {
+                                    const R east = rc[k + 1];
+                                    R nv = ((re[k] + rw[k]) * a.dy2 + (east + west) * a.dx2 - c[r][k]) * a.inv_den;
+                                    R d = nv - cen;
+                                    R w = R(1);
+                                    if (i == 1) { w += R(1); po[j - ld] = nv; }
+                                    if (i == nx) { w += R(1); po[j + ld] = nv; }
+                                    if (j == 1) { w += R(1); po[0] = nv; }
+                                    if (j == ny) { if (ray) { w += R(1); po[ny + 1] = nv; } }
+                                    if (i == ib && lout) lout[j] = nv;     // halo row S_left + 1 of rank g - 1
+                                    if (i == ie && rout) rout[j] = nv;     // halo row 0 of rank g + 1
+                                    acc += w * (d * d);
+                                    po[j] = nv;
+                                    west = cen; cen = east;
+                                }
+                            }
+                        }
+                    }
+                }
+                acc = warp_sum(acc);
+                const int lane = tid & 31, warp = tid >> 5;
+                if (lane < G) cluster_map(&s_part[itp & 1][rank][warp], lane)[0] = acc;
+                cluster_barrier();
+                err = R(0);
+                for (int g = 0; g < G; g++) {                  // same partials, same order in every thread of the cluster
+                    R eg = s_part[itp & 1][g][0];
+#pragma unroll
+                    for (int w = 1; w < T / 32; w++) eg += s_part[itp & 1][g][w];
+                    err += eg;
+                }
+                R *t = pin; pin = pout; pout = t;
+                itp += 1;
+                if (itp > a.itmax) { status |= BEACON_STATUS_POISSON_OVERFLOW; break; }
+            }
+            it_total += itp;
+            const R *phi = pin;
+
+            // ---- p += phi (own rows, ghost rows at the ends) and corrector --------------------------------
+            for (int e = e0 + tid; e < e1; e += T) p[e] += phi[e - (ib - 1) * ld];
+            CELL_LOOP {
+                const int i = i0 + r, j = j0 + k;
+                if (CELL_OK(i, j)) {
+                    const int li = i - ib + 1;
+                    if (i >= 2) u[i * ld + j] = us[i * ld + j] - a.dt * (phi[li * ld + j] - phi[(li - 1) * ld + j]) * a.inv_dx;
+                    if (j >= 2) v[i * ld + j] = vs[i * ld + j] - a.dt * (phi[li * ld + j] - phi[li * ld + j - 1]) * a.inv_dy;
+                }
+            }
+            cluster_barrier();                                 // u of row ie + 1 comes from rank g + 1
+
+            // ---- transport: coefficients per pass in the phi planes, wavefront chained over the ranks -----
+            {
+                const int passes = a.tr_pass, rows = (S + passes - 1) / passes;
+                R *cA = phiA, *cW = phiA + rows * ld, *cS = phiA + 2 * rows * ld;
+                const R kx = a.tcoef * a.inv_dx2, ky = a.tcoef * a.inv_dy2;
+                int *right_flag = last ? nullptr : cluster_map(s_flag, rank + 1);
+                R *right_west = last ? nullptr : cluster_map(s_west, rank + 1);
+                for (int ps = 0; ps < passes; ps++) {
+                    const int pb = ib + ps * rows, pe = min(ie, pb + rows - 1);
+                    // old values of row ie + 1 (rank g + 1) are read here, before this rank's last pass
+                    // hands over the columns that rank g + 1 needs before it overwrites that row
+                    CELL_LOOP {
+                        const int i = i0 + r, j = j0 + k;
+                        if (CELL_OK(i, j) && i >= pb && i <= pe) {
+                            const R uE = u[(i + 1) * ld + j], uW = u[i * ld + j], vN = v[i * ld + j + 1], vS = v[i * ld + j];
+                            const R sc = s[i * ld + j], sE = s[(i + 1) * ld + j], sN = s[i * ld + j + 1];
+                            R diff0 = ((sE - R(2) * sc) * a.inv_dx2 + (sN - R(2) * sc) * a.inv_dy2) * a.tcoef;
+                            R conv0 = (uE * (R(0.5) * (sE + sc)) - uW * (R(0.5) * sc)) * a.inv_dx +
+                                      (vN * (R(0.5) * (sN + sc)) - vS * (R(0.5) * sc)) * a.inv_dy;
+                            const int e = (i - pb) * ld + j;
+                            cA[e] = sc + a.dt * (diff0 - conv0);
+                            cW[e] = a.dt * (kx + R(0.5) * uW * a.inv_dx);
+                            cS[e] = a.dt * (ky + R(0.5) * vS * a.inv_dy);
+                        }
+                    }
+                    __syncthreads();
+                    if (tid < 32) {
+                        constexpr int RPL = MAC_RPL;
+                        const int lanes = (pe - pb + 1 + RPL - 1) / RPL;
+                        const int lane = tid;
+                        const int rb = pb + lane * RPL;
+                        const bool from_left = ps == 0 && !first;        // row pb - 1 is rank g - 1's last row
+                        const bool to_right = ps == passes - 1 && !last;  // row pe = ie feeds rank g + 1
+                        R prev[RPL];
+#pragma unroll
+                        for (int q = 0; q < RPL; q++) prev[q] = (rb + q <= pe) ? s[(rb + q) * ld + 0] : R(0);
+                        R last_new = R(0);
+                        const int steps = ny + lanes - 1;
+                        for (int t = 0; t < steps; t++) {
+                            R wv = __shfl_up_sync(0xffffffffu, last_new, 1);
+                            const int j = t - lane + 1;
+                            if (lane < lanes && j >= 1 && j <= ny) {
+                                if (lane == 0) {
+                                    if (from_left) {
+                                        if ((j - 1) % MAC_CLUSTER_CHUNK == 0)
+                                            while (ld_acquire_cluster(&s_flag[(j - 1) / MAC_CLUSTER_CHUNK]) != seq) {}
+                                        wv = s_west[j];
+                                    } else wv = s[(pb - 1) * ld + j];
+                                }
+#pragma unroll
+                                for (int q = 0; q < RPL; q++) {
+                                    const int i = rb + q;
+                                    if (i <= pe) {
+                                        const int e = (i - pb) * ld + j;
+                                        R nv = (cA[e] + cS[e] * prev[q]) + cW[e] * wv;
+                                        s[i * ld + j] = nv;
+                                        prev[q] = nv;
+                                        wv = nv;
+                                        if (to_right && i == pe) {
+                                            right_west[j] = nv;
+                                            if (j % MAC_CLUSTER_CHUNK == 0 || j == ny) st_release_cluster(&right_flag[(j - 1) / MAC_CLUSTER_CHUNK], seq);
+                                        }
+                                    }
+                                }
+                                last_new = wv;
+                            }
+                        }
+                    }
+                    __syncthreads();
+                }
+            }
+        }   // sub-steps
+        cluster_barrier();                                     // every rank's rows done
+
+        // ---- observations and reward: rank 0 writes, every rank contributes its rows -----------------
+        R part = R(0);
+        if (!ray) for (int e = e0 + tid; e < e1; e += T) part += rabs(s[e] - a.ref_c);
+        part = block_sum(part, s_red);
+        bool nonfinite = false;
+        for (int e = e0 + tid; e < e1; e += T) nonfinite |= !finite_(s[e]) | !finite_(u[e]) | !finite_(v[e]);
+        const int bad = __syncthreads_or(nonfinite ? 1 : 0);
+        if (tid < G) { cluster_map(s_rank, tid)[rank] = part; cluster_map(s_bad, tid)[rank] = bad; }
+        if (first) {
+            R *hist = a.obs_hist + (size_t)b * a.n_obs;
+            const int per_step = 3 * a.nx_obs_pts * a.ny_obs_pts;
+            R *out = a.obs + orow * a.n_obs;
+            for (int e = tid; e < a.n_obs; e += T) {
+                int st = e / per_step, rm = e - st * per_step;
+                R val;
+                if (st < a.n_obs_steps - 1) val = hist[e + per_step];
+                else {
+                    int f = rm / (a.nx_obs_pts * a.ny_obs_pts), q = rm - f * (a.nx_obs_pts * a.ny_obs_pts);
+                    int pi = q / a.ny_obs_pts, pj = q - pi * a.ny_obs_pts;
+                    int x = a.nx_obs / 2 + pi * a.nx_obs, y = a.ny_obs / 2 + pj * a.ny_obs;
+                    val = (f == 0) ? s[x * ld + y] : (f == 1 ? u[x * ld + y] : v[x * ld + y]);
+                }
+                out[e] = val;
+            }
+            __syncthreads();
+            for (int e = tid; e < a.n_obs; e += T) hist[e] = out[e];
+        }
+        R nu = R(0);
+        if (first && ray && tid == 0)                          // rayleigh.py:265-275 (sequential sum over i)
+            for (int i = 1; i <= nx; i++) nu -= (s[i * ld + 1] - a.Th) / (R(0.5) * a.dy);
+        cluster_barrier();                                     // partials in place; obs read before the next walls
+        int any_bad = 0;
+        R total = R(0);
+        for (int g = 0; g < G; g++) { any_bad |= s_bad[g]; total += s_rank[g]; }   // rank order
+        if (any_bad) status |= BEACON_STATUS_NONFINITE;
+        if (first && tid == 0) {
+            a.rwd[orow] = ray ? -(nu / R(nx)) : -(total / R(a.n));
+            bool horizon = stp == a.n_act - 1;
+            a.done[orow] = horizon; a.trunc[orow] = horizon;
+            if (a.iters) a.iters[orow] = it_total;
+        }
+        stp += 1;
+    }   // actions
+
+    if (first && tid == 0) { a.stp[b] = stp; if (a.status) a.status[b] = status; }
+    cluster_barrier();                                         // no CTA leaves while a neighbour may write its shared memory
 #undef CELL_LOOP
 #undef CELL_OK
 }
@@ -1910,9 +2345,33 @@ __global__ void __launch_bounds__(T, MINB) mac_big_kernel(const MacArgs<R> a)
 }
 
 // ---------------------------------------------------------------------------------------
+// Capacity of mac_cluster_kernel with G CTAs per env: "" when (nx, ny) fits, else the reason.
+// Slabs of at least MAC_CLUSTER_MIN_ROWS rows; 4x5 tiles of the thickest slab within 512 threads; two phi
+// slab planes of (rows + 2) x (ny + 2) in the shared-memory budget; ny + 2 within the hand-off buffers.
+// The transport coefficients take 3 planes of a pass of at most 32 * MAC_RPL rows (cluster_passes).
+template <typename R> static std::string cluster_misfit(int nx, int ny, int G)
+{
+    const int ld = ny + 2, Smax = (nx + G - 1) / G;
+    if (G > MAC_CLUSTER_MAX) return "at most " + std::to_string(MAC_CLUSTER_MAX) + " CTAs per env (portable cluster size)";
+    if (nx / G < MAC_CLUSTER_MIN_ROWS)
+        return "slabs of " + std::to_string(nx / G) + " rows, fewer than " + std::to_string(MAC_CLUSTER_MIN_ROWS);
+    if (ld > MAC_CLUSTER_MAX_LD) return "ny + 2 = " + std::to_string(ld) + " columns, more than " + std::to_string(MAC_CLUSTER_MAX_LD);
+    if (((Smax + 3) / 4) * ((ny + 4) / 5) > 512) return "slab of " + std::to_string(Smax) + " rows needs more than 512 tiles of 4x5 cells";
+    if (2 * (size_t)(Smax + 2) * ld * sizeof(R) > MAC_CLUSTER_SMEM || 3 * (size_t)ld * sizeof(R) > MAC_CLUSTER_SMEM)
+        return "two phi slab planes of " + std::to_string(Smax + 2) + " rows exceed " + std::to_string(MAC_CLUSTER_SMEM / 1024) + " KB";
+    return "";
+}
+// transport passes of a slab: at most 32 * MAC_RPL rows each (one warp), 3 coefficient planes in the budget
+template <typename R> static int cluster_passes(int Smax, int ld)
+{
+    int ps = 1;
+    while ((Smax + ps - 1) / ps > 32 * MAC_RPL || 3 * (size_t)((Smax + ps - 1) / ps) * ld * sizeof(R) > MAC_CLUSTER_SMEM) ps++;
+    return ps;
+}
+
 template <typename R> class MacEnv : public Env {
     beacon_mac_params p;
-    int kind;
+    int kind, G = 1;
     DeviceBuffer u, v, pp, s, us, vs, cc, a_cur, a_int, obs_hist, stp, u0, v0, p0, s0, dbgbuf;
     MacArgs<R> base{};
     void (*kernel)(const MacArgs<R>) = nullptr;
@@ -1943,11 +2402,20 @@ public:
         info.rwd_dim = 1; info.n_act = p.n_act; info.noise_dim = 0;
 
         MacArgs<R> &a = base;
-        // kernel variant: all planes in shared memory when 8 planes fit, else phi planes only
+        // kernel variant: all planes in shared memory when 8 planes fit, else phi planes only;
+        // ctas_per_env = G > 1 selects mac_cluster_kernel on any grid
         const size_t plane = (size_t)n * sizeof(R);
         int TI, TJ;
+        G = p.ctas_per_env;
+        BEACON_REQUIRE(G >= 0, "mac2d: ctas_per_env must be >= 0 (0 and 1: one CTA per env)");
+        if (G > 1) {
+            const std::string why = cluster_misfit<R>(nx, ny, G);
+            if (why.size()) throw Error(BEACON_ERR_UNSUPPORTED, "mac2d: ctas_per_env=" + std::to_string(G) + ": " + why);
+        }
         reg_variant = false;
-        if (ray && nx == 50 && ny == 50 && p.n_sgts <= 32 && !getenv("BEACON_MAC_V1")) {
+        if (G > 1) {
+            // selected below, after the transport passes
+        } else if (ray && nx == 50 && ny == 50 && p.n_sgts <= 32 && !getenv("BEACON_MAC_V1")) {
             // five planes fit twice per SM: register-resident phi tiles, 2 CTAs/SM
             const char *tile = getenv("BEACON_MAC_TILE");              // tuning: "5x5" = 100 threads with 25 cells each
             if (tile && !strcmp(tile, "5x5")) {
@@ -1967,13 +2435,38 @@ public:
             smem = sizeof(R) * 2 * (size_t)((102 * 105 + 3) / 4 * 4);
         } else if (2 * plane + 1024 <= 220 * 1024 && ((nx + 3) / 4) * ((ny + 4) / 5) <= 512) {
             kernel = mac_kernel<R, 4, 5, 512, false>; T = 512; TI = 4; TJ = 5; smem = 2 * plane;
-        } else
-            throw Error(BEACON_ERR_UNSUPPORTED, "mac2d: grid too large for the one-CTA-per-env kernel (max ~100x100 cells)");
+        } else {
+            std::string msg = "mac2d: grid too large for the one-CTA-per-env kernel (max ~100x100 cells)";
+            for (int g = 2; g <= MAC_CLUSTER_MAX; g++)
+                if (!cluster_misfit<R>(nx, ny, g).size()) { msg += " (ctas_per_env=" + std::to_string(g) + " would fit)"; break; }
+            throw Error(BEACON_ERR_UNSUPPORTED, msg);
+        }
         // transport scratch = 3 planes of ceil(nx/passes) rows inside the two phi planes
         a.tr_pass = 1;
         while (3 * (size_t)((nx + a.tr_pass - 1) / a.tr_pass) * ld > 2 * (size_t)n || (nx + a.tr_pass - 1) / a.tr_pass > 32 * MAC_RPL)
             a.tr_pass++;
+        if (G > 1) {
+            // one cluster of G CTAs per env: slab rows, phi slab planes + transport passes (cluster_misfit)
+            const int Smax = (nx + G - 1) / G;
+            a.G = G; a.slab_rows = Smax + 2;
+            a.tr_pass = cluster_passes<R>(Smax, ld);
+            const int rows = (Smax + a.tr_pass - 1) / a.tr_pass;
+            kernel = mac_cluster_kernel<R, 4, 5, 512>; T = 512; TI = 4; TJ = 5;
+            smem = sizeof(R) * (size_t)ld * std::max(2 * a.slab_rows, 3 * rows);
+        }
         BEACON_CUDA_CHECK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        if (G > 1) {
+            cudaLaunchConfig_t cfg = {};
+            cudaLaunchAttribute at[1];
+            cfg.gridDim = dim3(B * G); cfg.blockDim = dim3(T); cfg.dynamicSmemBytes = smem;
+            at[0].id = cudaLaunchAttributeClusterDimension; at[0].val.clusterDim.x = G; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
+            cfg.attrs = at; cfg.numAttrs = 1;
+            int clusters = 0;
+            BEACON_CUDA_CHECK(cudaOccupancyMaxActiveClusters(&clusters, kernel, &cfg));
+            if (clusters < 1)
+                throw Error(BEACON_ERR_UNSUPPORTED, "mac2d: no cluster of " + std::to_string(G) + " CTAs of " + std::to_string(smem) +
+                                                        " B shared memory fits this device");
+        }
 
         const size_t nb = (size_t)B * plane;
         u.alloc(nb); v.alloc(nb); pp.alloc(nb); s.alloc(nb); us.alloc(nb); vs.alloc(nb);
@@ -2015,6 +2508,14 @@ public:
             BEACON_CUDA_CHECK(cudaMemsetAsync(dbgbuf.ptr, 0, 64, st));
             a.dbg = dbgbuf.as<unsigned long long>();
         }
+        if (G > 1) {
+            cudaLaunchConfig_t cfg = {};
+            cfg.gridDim = dim3(a.B * G); cfg.blockDim = dim3(T); cfg.dynamicSmemBytes = smem; cfg.stream = st;
+            cudaLaunchAttribute at[1];
+            at[0].id = cudaLaunchAttributeClusterDimension; at[0].val.clusterDim.x = G; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
+            cfg.attrs = at; cfg.numAttrs = 1;
+            BEACON_CUDA_CHECK(cudaLaunchKernelEx(&cfg, kernel, a));
+        } else
 #ifdef MAC_CLUSTER_BARRIER_TEST
         {
             cudaLaunchConfig_t cfg = {};

@@ -310,9 +310,9 @@ class rayleigh(_Mac):
     _name = "rayleigh"
     _fields = ("u", "v", "p", "T", "a")
 
-    def __init__(self, cpu=0, init=True, L=1.0, H=1.0, n_sgts=10, ra=1.0e4, device=0, dtype=torch.float64):
+    def __init__(self, cpu=0, init=True, L=1.0, H=1.0, n_sgts=10, ra=1.0e4, device=0, dtype=torch.float64, ctas_per_env=1):
         self.n_sgts = n_sgts
-        self._make(device=device, dtype=dtype, init=init, L=L, H=H, n_sgts=n_sgts, ra=ra)
+        self._make(device=device, dtype=dtype, init=init, L=L, H=H, n_sgts=n_sgts, ra=ra, ctas_per_env=ctas_per_env)
         n = self._env.n_obs
         self.action_space = _Box(-0.75, 0.75, (n_sgts,))
         self.observation_space = _Box(-np.ones(n), np.ones(n), (n,))
@@ -335,8 +335,9 @@ class mixing(_Mac):
     _name = "mixing"
     _fields = ("u", "v", "p", "C", "us", "vs")
 
-    def __init__(self, cpu=0, L=1.0, H=1.0, re=100.0, pe=10000.0, side=0.5, C0=1.0, device=0, dtype=torch.float64):
-        self._make(device=device, dtype=dtype, L=L, H=H, re=re, pe=pe, side=side, C0=C0)
+    def __init__(self, cpu=0, L=1.0, H=1.0, re=100.0, pe=10000.0, side=0.5, C0=1.0, device=0, dtype=torch.float64,
+                 ctas_per_env=1):
+        self._make(device=device, dtype=dtype, L=L, H=H, re=re, pe=pe, side=side, C0=C0, ctas_per_env=ctas_per_env)
         n = self._env.n_obs
         self.action_space = _Discrete(4)
         self.observation_space = _Box(-np.ones(n), np.ones(n), (n,))

@@ -134,6 +134,10 @@ typedef struct {
     double pr, ra, Tc, Th, C;                 /* rayleigh */
     double re, pe, u_max, ref_c;              /* mixing; ref_c = side^2/(L*H)*C0 (mixing.py:261) */
     double tol;                               /* 1e-8 rayleigh.py:414 / 1e-4 mixing.py:423 */
+    /* How many SMs one environment may occupy.  0 or 1: one CTA per env (grids up to ~100x100
+     * cells).  2..8: one thread-block cluster of exactly that many CTAs per env, each owning a slab of
+     * >= 4 rows of i, on any grid whose slab fits (DESIGN.md 3.6); anything else is rejected at create. */
+    int32_t ctas_per_env;
 } beacon_mac_params;
 
 /* What a handle looks like from outside. */
