@@ -315,6 +315,17 @@ public:
                    int32_t *status, cudaStream_t stream);
 };
 
+// Let `kernel` launch with `bytes` of dynamic shared memory.  The limit is an attribute of the kernel
+// function, shared by every env of the process on that instance, so it is only ever raised: lowering it
+// to a smaller env's size would make the next launch of a larger env fail.
+template <typename K> inline void raise_dynamic_smem_limit(K kernel, size_t bytes)
+{
+    cudaFuncAttributes fa;
+    BEACON_CUDA_CHECK(cudaFuncGetAttributes(&fa, (const void *)kernel));
+    if ((size_t)fa.maxDynamicSharedSizeBytes < bytes)
+        BEACON_CUDA_CHECK(cudaFuncSetAttribute((const void *)kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
+}
+
 // upload a host float64 array as `R`
 template <typename R> inline void upload_as(DeviceBuffer &dst, const double *src, size_t n)
 {

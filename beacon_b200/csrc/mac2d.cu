@@ -8,8 +8,8 @@
 // predictor :382-416, poisson :421-465, corrector :470-473, transport :478-495,
 // get_obs :237-256, get_rwd :259-264.
 //
-// B200 design: ONE CTA PER ENVIRONMENT (or one cluster, mac_cluster_kernel) runs every sub-step of
-// every fused action without returning to the host.  Four kernels (DESIGN.md 3.4 - 3.6):
+// B200 design: ONE CTA PER ENVIRONMENT (or one cluster, mac_kernel with ctas_per_env > 1) runs every
+// sub-step of every fused action without returning to the host.  Three kernels (DESIGN.md 3.4 - 3.6):
 //   * mac_reg_kernel  — rayleigh 50x50: phi and the Poisson right-hand side of a 2x5 tile in
 //     REGISTERS, in-place Jacobi sweeps over two strided exchange planes (one barrier per sweep),
 //     convergence test two sweeps behind and interleaved with the next sweep (exact sweep counts),
@@ -17,12 +17,12 @@
 //   * mac_big_kernel  — mixing 100x100: the same register-resident Poisson with 4x5 tiles, field
 //     planes in L2/HBM, tile copies of p, us, vs in a thread-interleaved scratch, u / v staged in
 //     the exchange planes for the predictor (TMA bulk copies), transport in two row passes;
-//   * mac_kernel      — generic fallback for any other grid up to ~100x100 cells: phi ping-pongs
-//     between two shared-memory planes, right-hand side in registers, fields in global memory;
-//   * mac_cluster_kernel — only with ctas_per_env = G in 2..8, on any grid whose row slabs fit
-//     (DESIGN.md 3.6): one env over a cluster of G CTAs, phi slabs in each CTA's shared memory,
-//     halo rows and residual partials through DSMEM, one cluster barrier per sweep, the transport
-//     wavefront chained from rank to rank.
+//   * mac_kernel      — generic kernel for any other grid: one env over G = ctas_per_env CTAs
+//     (1 by default, 2..8 as a thread-block cluster, DESIGN.md 3.6), each with its slab of rows of
+//     the two phi planes in shared memory, right-hand side in registers, fields in global memory;
+//     at G > 1 halo rows and residual partials go through DSMEM, one cluster barrier per sweep, the
+//     transport wavefront chained from rank to rank.  At G = 1 the slab is the whole array (grids
+//     up to ~100x100 cells) and every barrier is a CTA barrier.
 // Common to all:
 //   * the residual reproduces the reference's: sum over the whole ghost-inclusive array after
 //     the ghost update (ghost copies re-count the wall-adjacent cells; mixing's top ghost is 0);
@@ -32,19 +32,9 @@
 //     update that only involves OLD values plus the coefficients multiplying the new neighbours;
 //     then one warp runs the remaining 2-FMA recurrence as a skewed wavefront, rows across lanes,
 //     the new west value travelling by warp shuffle (no barriers).
-//
-// Build switches (tuning aids; `python -m beacon_b200.build --tag=x -DNAME=1` + tools/ab.sh compare two libraries on the
-// same GPU box).  Each keeps the variant a measured change replaced, so that the A/B numbers of DESIGN.md 3.4 / 3.5 can
-// be reproduced; the product build defines none of them:
-//   MAC_REG_P_SCRATCH=0      rayleigh: pressure accessed tile-wise in its plane (47.0 k vs 50.7 k env-actions/s)
-//   MAC_BIG_DECIDE_LAST      mixing: convergence decision after the sweep, stores at its end (3.73 k vs 4.10 k)
-//   MAC_BIG_COPYOUT_BY_TILE  mixing: transported scalar copied back by tile (4.10 k vs 4.16 k)
-//   MAC_BIG_TRCOEF_BY_TILE   mixing: transport coefficients computed by tile (4.16 k vs 4.36 k)
-//   MAC_CLUSTER_BARRIER_TEST rayleigh: cluster barrier in place of the CTA barrier of a sweep (cost measurement)
 #include <cstdio>
 #include <cstdlib>
 #include <algorithm>
-#include <cstring>
 #include <string>
 #include <type_traits>
 
@@ -64,7 +54,7 @@ template <typename R> struct MacArgs {
     int nx_obs_pts, ny_obs_pts, n_obs_steps, nx_obs, ny_obs, n_obs, tr_pass;
     R dx, dy, dt, inv_dx, inv_dy, inv_dx2, inv_dy2, dx2, dy2, inv_den, pk1, pk2, cscale, dcoef, tcoef, Tc, Th, Cmax, u_max, ref_c, tol;
     int B, mode, n_fused;
-    int G, slab_rows;                  // mac_cluster_kernel: CTAs per env, rows of a phi slab plane (halos included)
+    int G, slab_rows;                  // mac_kernel: CTAs per env, rows of a phi slab plane (halos included)
     R *u, *v, *p, *s, *us, *vs, *cc;   // [B, n] planes (s = T or C); us/vs/cc are workspaces
     R *a_cur, *obs_hist;
     int32_t *stp, *a_int;
@@ -96,384 +86,38 @@ template <typename R> __device__ R np_pairwise_small(const R *a, int n)
     return res;
 }
 
-template <typename R, int TI, int TJ, int T, bool SMEM>
-__global__ void __launch_bounds__(T) mac_kernel(const MacArgs<R> a)
-{
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    __shared__ R s_part[2][T / 32];
-    __shared__ R s_red[T / 32];
-    __shared__ R s_seg[128];          // Th + a_j per segment (rayleigh) / wall speeds (mixing)
-    __shared__ R s_act[128];
-    const int tid = threadIdx.x, b = blockIdx.x;
-    const int nx = a.nx, ny = a.ny, ld = a.ld, n = a.n;
-    const bool resetting = a.mode == 1;
-    if (resetting && a.mask && !a.mask[b]) return;
-    const bool ray = a.kind == BEACON_RAYLEIGH;
-
-    // ---- planes ------------------------------------------------------------------------------
-    R *phiA = reinterpret_cast<R *>(smem_raw), *phiB = phiA + n;
-    R *u, *v, *p, *s, *us, *vs;
-    const size_t row = (size_t)b * n;
-    if (SMEM) { u = phiB + n; v = u + n; p = v + n; s = p + n; us = s + n; vs = us + n; }
-    else { u = a.u + row; v = a.v + row; p = a.p + row; s = a.s + row; us = a.us + row; vs = a.vs + row; }
-    R *gu = a.u + row, *gv = a.v + row, *gp = a.p + row, *gs = a.s + row;
-
-    // ---- tile ownership ------------------------------------------------------------------------
-    const bool has_tile = tid < a.tiles_i * a.tiles_j;
-    const int ti = tid / a.tiles_j, tj = tid - ti * a.tiles_j;
-    const int i0 = 1 + ti * TI, j0 = 1 + tj * TJ;
-#define CELL_LOOP                                       \
-    _Pragma("unroll") for (int r = 0; r < TI; r++)      \
-    _Pragma("unroll") for (int k = 0; k < TJ; k++)
-#define CELL_OK(i, j) (has_tile && (i) <= nx && (j) <= ny)
-
-    // ---- load / reset ----------------------------------------------------------------------------
-    if (resetting) {
-        for (int e = tid; e < n; e += T) {
-            R uu = ray ? a.u0[e] : R(0), vv = ray ? a.v0[e] : R(0), pp = ray ? a.p0[e] : R(0), ss = a.s0[e];
-            gu[e] = uu; gv[e] = vv; gp[e] = pp; gs[e] = ss;
-            a.us[row + e] = R(0); a.vs[row + e] = R(0);
-            if (SMEM) { u[e] = uu; v[e] = vv; s[e] = ss; }
-        }
-        for (int e = tid; e < a.n_obs; e += T) a.obs_hist[(size_t)b * a.n_obs + e] = R(0);
-        for (int e = tid; e < (ray ? a.n_sgts : 0); e += T) a.a_cur[(size_t)b * a.n_sgts + e] = R(0);
-        if (tid == 0) { a.stp[b] = 0; if (!ray) a.a_int[b] = 1; }
-        __syncthreads();
-    } else if (SMEM) {
-        for (int e = tid; e < n; e += T) { u[e] = gu[e]; v[e] = gv[e]; p[e] = gp[e]; s[e] = gs[e]; us[e] = a.us[row + e]; vs[e] = a.vs[row + e]; }
-        __syncthreads();
-    }
-    for (int e = tid; e < 2 * n; e += T) phiA[e] = R(0);
-    int stp = resetting ? 0 : a.stp[b];
-    int status = 0;
-    const int n_actions = resetting ? 0 : a.n_fused;
-
-    for (int act = 0; act < n_actions; act++) {
-        const size_t orow = (size_t)act * a.B + b;
-        __syncthreads();
-        // ---- action conditioning ----------------------------------------------------------------
-        if (ray) {
-            const R *ain = (const R *)a.actions + orow * a.n_sgts;
-            if (tid == 0) {                                        // rayleigh.py:164-171
-                const int ns = a.n_sgts;
-                for (int j = 0; j < ns; j++) s_act[j] = ain[j];
-                R mean = np_pairwise_small(s_act, ns) / R(ns);
-                R m = R(1);
-                for (int j = 0; j < ns; j++) { s_act[j] = s_act[j] - mean; m = np_max(m, rabs(s_act[j]) / a.Cmax); }
-                for (int j = 0; j < ns; j++) { s_act[j] = s_act[j] / m; s_seg[j] = a.Th + s_act[j]; a.a_cur[(size_t)b * ns + j] = s_act[j]; }
-            }
-        } else if (tid == 0) {                                     // get_control, mixing.py:212-234
-            int ai = ((const int32_t *)a.actions)[orow];
-            R ut = 0, ub = 0, vl = 0, vr = 0;
-            if (ai == 0) { ub = a.u_max; ut = -a.u_max; }
-            if (ai == 1) { ub = -a.u_max; ut = a.u_max; }
-            if (ai == 2) { vr = a.u_max; vl = -a.u_max; }
-            if (ai == 3) { vr = -a.u_max; vl = a.u_max; }
-            s_seg[0] = ut; s_seg[1] = ub; s_seg[2] = vl; s_seg[3] = vr;
-            a.a_int[b] = ai;
-        }
-        __syncthreads();
-        long long it_total = 0;
-
-        for (int it = 0; it < a.ndt_act; it++) {
-            // ---- boundary conditions: rayleigh.py:180-202, mixing.py:153-171 ---------------------
-            // (wall-normal velocities are zeroed first in the reference; the ghost formulas below
-            //  read them as zero, so one pass suffices)
-            for (int k = tid; k < 2 * (nx + 2) + 2 * (ny + 2); k += T) {
-                if (k < ny + 2) {                                  // left wall (i = 0/1), index j = k
-                    int j = k;
-                    if (j >= 1 && j <= ny) { u[1 * ld + j] = R(0); s[0 * ld + j] = s[1 * ld + j]; }
-                    if (j >= 2 && j <= ny) v[0 * ld + j] = ray ? -v[1 * ld + j] : R(2) * s_seg[2] - v[1 * ld + j];
-                } else if (k < 2 * (ny + 2)) {                     // right wall
-                    int j = k - (ny + 2);
-                    if (j >= 1 && j <= ny) { u[(nx + 1) * ld + j] = R(0); s[(nx + 1) * ld + j] = s[nx * ld + j]; }
-                    if (j >= 2 && j <= ny) v[(nx + 1) * ld + j] = ray ? -v[nx * ld + j] : R(2) * s_seg[3] - v[nx * ld + j];
-                } else if (k < 2 * (ny + 2) + (nx + 2)) {          // top wall (j = ny+1), index i
-                    int i = k - 2 * (ny + 2);
-                    if (i >= 1 && i <= nx + 1) {
-                        R ui = (i == 1 || i == nx + 1) ? R(0) : u[i * ld + ny];
-                        u[i * ld + ny + 1] = ray ? -ui : R(2) * s_seg[0] - ui;
-                    }
-                    if (i >= 1 && i <= nx) {
-                        v[i * ld + ny + 1] = R(0);
-                        s[i * ld + ny + 1] = ray ? R(2) * a.Tc - s[i * ld + ny] : s[i * ld + ny];
-                    }
-                } else {                                           // bottom wall (j = 0/1)
-                    int i = k - 2 * (ny + 2) - (nx + 2);
-                    if (i >= 1 && i <= nx + 1) {
-                        R ui = (i == 1 || i == nx + 1) ? R(0) : u[i * ld + 1];
-                        u[i * ld + 0] = ray ? -ui : R(2) * s_seg[1] - ui;
-                    }
-                    if (i >= 1 && i <= nx) {
-                        v[i * ld + 1] = R(0);
-                        if (ray) {
-                            int sg = (i - 1) / a.nx_sgts;
-                            if (sg < a.n_sgts) s[i * ld + 0] = R(2) * s_seg[sg] - s[i * ld + 1];
-                        } else s[i * ld + 0] = s[i * ld + 1];
-                    }
-                }
-            }
-            __syncthreads();
-
-            // ---- predictor: rayleigh.py:371-407, mixing.py:382-416 ------------------------------------
-            CELL_LOOP {
-                const int i = i0 + r, j = j0 + k;
-                if (CELL_OK(i, j)) {
-                    const R uc = u[i * ld + j], vc = v[i * ld + j];
-                    if (i >= 2) {
-                        R uE = R(0.5) * (u[(i + 1) * ld + j] + uc), uW = R(0.5) * (uc + u[(i - 1) * ld + j]);
-                        R uN = R(0.5) * (u[i * ld + j + 1] + uc), uS = R(0.5) * (uc + u[i * ld + j - 1]);
-                        R vN = R(0.5) * (v[i * ld + j + 1] + v[(i - 1) * ld + j + 1]), vS = R(0.5) * (vc + v[(i - 1) * ld + j]);
-                        R conv = (uE * uE - uW * uW) * a.inv_dx + (uN * vN - uS * vS) * a.inv_dy;
-                        R diff = ((u[(i + 1) * ld + j] - R(2) * uc + u[(i - 1) * ld + j]) * a.inv_dx2 +
-                                  (u[i * ld + j + 1] - R(2) * uc + u[i * ld + j - 1]) * a.inv_dy2) * a.dcoef;
-                        R pres = (p[i * ld + j] - p[(i - 1) * ld + j]) * a.inv_dx;
-                        us[i * ld + j] = uc + a.dt * (diff - conv - pres);
-                    }
-                    if (j >= 2) {
-                        R vE = R(0.5) * (v[(i + 1) * ld + j] + vc), vW = R(0.5) * (vc + v[(i - 1) * ld + j]);
-                        R uE = R(0.5) * (u[(i + 1) * ld + j] + u[(i + 1) * ld + j - 1]), uW = R(0.5) * (uc + u[i * ld + j - 1]);
-                        R vN = R(0.5) * (v[i * ld + j + 1] + vc), vS = R(0.5) * (vc + v[i * ld + j - 1]);
-                        R conv = (uE * vE - uW * vW) * a.inv_dx + (vN * vN - vS * vS) * a.inv_dy;
-                        R diff = ((v[(i + 1) * ld + j] - R(2) * vc + v[(i - 1) * ld + j]) * a.inv_dx2 +
-                                  (v[i * ld + j + 1] - R(2) * vc + v[i * ld + j - 1]) * a.inv_dy2) * a.dcoef;
-                        R pres = (p[i * ld + j] - p[i * ld + j - 1]) * a.inv_dy;
-                        R rhs = diff - conv - pres;
-                        if (ray) rhs += s[i * ld + j];
-                        vs[i * ld + j] = vc + a.dt * rhs;
-                    }
-                }
-            }
-            __syncthreads();
-
-            // ---- Poisson right-hand side into registers (b dx^2 dy^2, rayleigh.py:428-434) ----------
-            R c[TI][TJ];
-            CELL_LOOP {
-                const int i = i0 + r, j = j0 + k;
-                c[r][k] = R(0);
-                if (CELL_OK(i, j))
-                    c[r][k] = ((us[(i + 1) * ld + j] - us[i * ld + j]) * a.inv_dx + (vs[i * ld + j + 1] - vs[i * ld + j]) * a.inv_dy) * a.cscale;
-            }
-            // ---- Jacobi sweeps, poisson(): rayleigh.py:412-456 / mixing.py:421-465 -----------------------
-            R *pin = phiA, *pout = phiB;
-            for (int e = tid; e < 2 * n; e += T) phiA[e] = R(0);   // both planes: they doubled as transport scratch
-            __syncthreads();
-            R err = R(1.0e10);
-            int itp = 0;
-            while (err > a.tol) {
-                R acc = R(0);
-                if (has_tile) {
-#pragma unroll
-                    for (int r = 0; r < TI; r++) {
-                        const int i = i0 + r;
-                        if (i <= nx) {
-                            const R *rc = pin + i * ld + j0, *rw = rc - ld, *re = rc + ld;
-                            R west = rc[-1], cen = rc[0];
-#pragma unroll
-                            for (int k = 0; k < TJ; k++) {
-                                const int j = j0 + k;
-                                if (j <= ny) {
-                                    const R east = rc[k + 1];   // "north" in the reference's (i,j) naming: j+1
-                                    R nv = ((re[k] + rw[k]) * a.dy2 + (east + west) * a.dx2 - c[r][k]) * a.inv_den;
-                                    R d = nv - cen;
-                                    R w = R(1);
-                                    if (i == 1) { w += R(1); pout[j] = nv; }
-                                    if (i == nx) { w += R(1); pout[(nx + 1) * ld + j] = nv; }
-                                    if (j == 1) { w += R(1); pout[i * ld] = nv; }
-                                    if (j == ny) { if (ray) { w += R(1); pout[i * ld + ny + 1] = nv; } }
-                                    acc += w * (d * d);
-                                    pout[i * ld + j] = nv;
-                                    west = cen; cen = east;
-                                }
-                            }
-                        }
-                    }
-                }
-                acc = warp_sum(acc);
-                R *part = s_part[itp & 1];
-                if ((tid & 31) == 0) part[tid >> 5] = acc;
-                __syncthreads();
-                err = part[0];
-#pragma unroll
-                for (int w = 1; w < T / 32; w++) err += part[w];
-                R *t = pin; pin = pout; pout = t;
-                itp += 1;
-                if (itp > a.itmax) { status |= BEACON_STATUS_POISSON_OVERFLOW; break; }
-            }
-            it_total += itp;
-            const R *phi = pin;   // final iterate (mixing: its top ghost row is still 0)
-
-            // ---- p += phi (whole array, rayleigh.py:219) and corrector (:461-464) ---------------------
-            for (int e = tid; e < n; e += T) p[e] += phi[e];
-            CELL_LOOP {
-                const int i = i0 + r, j = j0 + k;
-                if (CELL_OK(i, j)) {
-                    if (i >= 2) u[i * ld + j] = us[i * ld + j] - a.dt * (phi[i * ld + j] - phi[(i - 1) * ld + j]) * a.inv_dx;
-                    if (j >= 2) v[i * ld + j] = vs[i * ld + j] - a.dt * (phi[i * ld + j] - phi[i * ld + j - 1]) * a.inv_dy;
-                }
-            }
-            __syncthreads();
-
-            // ---- transport: rayleigh.py:469-487 / mixing.py:478-495 -------------------------------------
-            // new(i,j) = A + BW*new(i-1,j) + BS*new(i,j-1); A, BW, BS from old values only.
-            // Scratch planes (3 per pass of `rows` rows) live in the phi planes (+ the Poisson-free
-            // us plane for rayleigh).
-            {
-                const int passes = a.tr_pass, rows = (nx + passes - 1) / passes;
-                R *cA = phiA, *cW = phiA + rows * ld, *cS = phiA + 2 * rows * ld;   // [rows][ld] each, row-local index
-                const R kx = a.tcoef * a.inv_dx2, ky = a.tcoef * a.inv_dy2;
-                for (int ps = 0; ps < passes; ps++) {
-                    const int ib = 1 + ps * rows, ie = min(nx, ib + rows - 1);
-                    CELL_LOOP {
-                        const int i = i0 + r, j = j0 + k;
-                        if (CELL_OK(i, j) && i >= ib && i <= ie) {
-                            const R uE = u[(i + 1) * ld + j], uW = u[i * ld + j], vN = v[i * ld + j + 1], vS = v[i * ld + j];
-                            const R sc = s[i * ld + j], sE = s[(i + 1) * ld + j], sN = s[i * ld + j + 1];
-                            // T += dt*(diff - conv), with TW = (Tw+Tc)/2 and TS = (Ts+Tc)/2 split off
-                            R diff0 = ((sE - R(2) * sc) * a.inv_dx2 + (sN - R(2) * sc) * a.inv_dy2) * a.tcoef;
-                            R conv0 = (uE * (R(0.5) * (sE + sc)) - uW * (R(0.5) * sc)) * a.inv_dx +
-                                      (vN * (R(0.5) * (sN + sc)) - vS * (R(0.5) * sc)) * a.inv_dy;
-                            const int e = (i - ib) * ld + j;
-                            cA[e] = sc + a.dt * (diff0 - conv0);
-                            cW[e] = a.dt * (kx + R(0.5) * uW * a.inv_dx);
-                            cS[e] = a.dt * (ky + R(0.5) * vS * a.inv_dy);
-                        }
-                    }
-                    __syncthreads();
-                    if (tid < 32) {
-                        // skewed wavefront: lane l owns rows ib + l*RPL .. ; at step t it does column t - l + 1
-                        constexpr int RPL = MAC_RPL;
-                        const int lanes = (ie - ib + 1 + RPL - 1) / RPL;
-                        const int lane = tid;
-                        const int rb = ib + lane * RPL;
-                        R prev[RPL];            // new values of my rows at column j-1
-#pragma unroll
-                        for (int q = 0; q < RPL; q++) prev[q] = (rb + q <= ie) ? s[(rb + q) * ld + 0] : R(0);
-                        R last_new = R(0);      // new value of my last row at the column just done
-                        const int steps = ny + lanes - 1;
-                        for (int t = 0; t < steps; t++) {
-                            // west value for my first row: lane-1's last row at the same column
-                            R wv = __shfl_up_sync(0xffffffffu, last_new, 1);
-                            const int j = t - lane + 1;
-                            if (lane < lanes && j >= 1 && j <= ny) {
-                                if (lane == 0) wv = s[(ib - 1) * ld + j];     // row ib-1: previous pass (new) or ghost
-#pragma unroll
-                                for (int q = 0; q < RPL; q++) {
-                                    const int i = rb + q;
-                                    if (i <= ie) {
-                                        const int e = (i - ib) * ld + j;
-                                        R nv = (cA[e] + cS[e] * prev[q]) + cW[e] * wv;
-                                        s[i * ld + j] = nv;
-                                        prev[q] = nv;
-                                        wv = nv;
-                                    }
-                                }
-                                last_new = wv;
-                            }
-                        }
-                    }
-                    __syncthreads();
-                }
-            }
-        }   // sub-steps
-
-        // ---- observations (probe history) and reward --------------------------------------------------
-        {
-            R *hist = a.obs_hist + (size_t)b * a.n_obs;
-            const int per_step = 3 * a.nx_obs_pts * a.ny_obs_pts;
-            R *out = a.obs + orow * a.n_obs;
-            for (int e = tid; e < a.n_obs; e += T) {              // rayleigh.py:243-262
-                int st = e / per_step, rem = e - st * per_step;
-                R val;
-                if (st < a.n_obs_steps - 1) val = hist[e + per_step];
-                else {
-                    int f = rem / (a.nx_obs_pts * a.ny_obs_pts), q = rem - f * (a.nx_obs_pts * a.ny_obs_pts);
-                    int pi = q / a.ny_obs_pts, pj = q - pi * a.ny_obs_pts;
-                    int x = a.nx_obs / 2 + pi * a.nx_obs, y = a.ny_obs / 2 + pj * a.ny_obs;
-                    val = (f == 0) ? s[x * ld + y] : (f == 1 ? u[x * ld + y] : v[x * ld + y]);
-                }
-                out[e] = val;
-            }
-            __syncthreads();
-            for (int e = tid; e < a.n_obs; e += T) hist[e] = out[e];
-            R rwd;
-            if (ray) {                                            // rayleigh.py:265-275 (sequential sum)
-                rwd = R(0);
-                if (tid == 0) {
-                    R nu = R(0);
-                    for (int i = 1; i <= nx; i++) nu -= (s[i * ld + 1] - a.Th) / (R(0.5) * a.dy);
-                    nu /= R(nx);
-                    rwd = -nu;
-                }
-            } else {                                              // mixing.py:259-264 (mean over the whole array)
-                R part = R(0);
-                for (int e = tid; e < n; e += T) part += rabs(s[e] - a.ref_c);
-                rwd = -(block_sum(part, s_red) / R(n));
-            }
-            bool nonfinite = false;
-            for (int e = tid; e < n; e += T) nonfinite |= !finite_(s[e]) | !finite_(u[e]) | !finite_(v[e]);
-            if (__syncthreads_or(nonfinite ? 1 : 0)) status |= BEACON_STATUS_NONFINITE;
-            if (tid == 0) {
-                a.rwd[orow] = rwd;
-                bool horizon = stp == a.n_act - 1;
-                a.done[orow] = horizon; a.trunc[orow] = horizon;
-                if (a.iters) a.iters[orow] = it_total;
-            }
-            stp += 1;
-        }
-    }   // actions
-
-    if (resetting) {
-        // reset observation: history is zero, newest slot sampled from the init state
-        __syncthreads();
-        R *hist = a.obs_hist + (size_t)b * a.n_obs;
-        const int per_step = 3 * a.nx_obs_pts * a.ny_obs_pts;
-        for (int e = tid; e < a.n_obs; e += T) {
-            int st = e / per_step, rem = e - st * per_step;
-            R val = R(0);
-            if (st == a.n_obs_steps - 1) {
-                int f = rem / (a.nx_obs_pts * a.ny_obs_pts), q = rem - f * (a.nx_obs_pts * a.ny_obs_pts);
-                int pi = q / a.ny_obs_pts, pj = q - pi * a.ny_obs_pts;
-                int x = a.nx_obs / 2 + pi * a.nx_obs, y = a.ny_obs / 2 + pj * a.ny_obs;
-                val = (f == 0) ? gs[x * ld + y] : (f == 1 ? gu[x * ld + y] : gv[x * ld + y]);
-            }
-            hist[e] = val;
-            a.obs[(size_t)b * a.n_obs + e] = val;
-        }
-        return;
-    }
-
-    // ---- store state -----------------------------------------------------------------------------------
-    __syncthreads();
-    if (SMEM) {
-        for (int e = tid; e < n; e += T) { gu[e] = u[e]; gv[e] = v[e]; gp[e] = p[e]; gs[e] = s[e]; a.us[row + e] = us[e]; a.vs[row + e] = vs[e]; }
-    }
-    if (tid == 0) { a.stp[b] = stp; if (a.status) a.status[b] = status; }
-#undef CELL_LOOP
-#undef CELL_OK
-}
-
 // ---------------------------------------------------------------------------------------
-// mac_cluster_kernel — one environment split over a thread-block cluster of G = a.G CTAs
-// (DESIGN.md 3.6).  Rank g owns the interior rows ib..ie of a balanced slab; the left wall and
-// ghost row 0 go to rank 0, the right wall and ghost row nx+1 to rank G-1.  Fields stay in their
-// global planes as in mac_kernel; each CTA keeps only its slab of the two phi planes (one halo
-// row on each side) in shared memory.  A Jacobi sweep pushes its first and last rows into the
+// mac_kernel — the generic kernel: one environment over G = a.G CTAs, a thread-block cluster
+// when G > 1 (DESIGN.md 3.6).  Rank g owns the interior rows ib..ie of a balanced slab; the left
+// wall and ghost row 0 go to rank 0, the right wall and ghost row nx+1 to rank G-1.  Fields stay
+// in their global planes; each CTA keeps only its slab of the two phi planes (one halo row on
+// each side) in shared memory.  A Jacobi sweep pushes its first and last rows into the
 // neighbours' halo rows through DSMEM and ends in one cluster barrier, where every CTA also
 // receives the per-warp residual partials of every rank.  Phases that read rows written by
 // another CTA follow a cluster barrier (release / acquire).  The transport wavefront of rank
 // g + 1 starts on the new values of rank g's last row, handed over through DSMEM in chunks of
 // MAC_CLUSTER_CHUNK columns, each published with a cluster-scope release / acquire flag.
+// CLUSTER = false is the G = 1 instance (a plain launch): the slab is the whole array, nothing goes
+// through DSMEM, every barrier is a CTA barrier (env_barrier) and the neighbour tests of the sweep and
+// the wavefront fold away.  With G a run-time value these cost 25 % per sweep at G = 1 (B200).
 // ---------------------------------------------------------------------------------------
 #define MAC_CLUSTER_MAX 8          // portable cluster size
 #define MAC_CLUSTER_MIN_ROWS 4     // rows of the thinnest slab: one tile height
 #define MAC_CLUSTER_MAX_LD 512     // columns (ny + 2) of the wavefront hand-off buffers
 #define MAC_CLUSTER_CHUNK 8        // columns per hand-off flag: a cluster-scope release per chunk, not per column
-#define MAC_CLUSTER_SMEM (200 * 1024)   // dynamic shared memory; the static arrays take the rest of 227 KB
+#define MAC_CLUSTER_SMEM (200 * 1024)   // phi slabs and transport planes; the hand-off buffers and static arrays take the rest of 227 KB
+// bytes of the wavefront hand-off buffers (G > 1 only), after the phi slabs in dynamic shared memory
+#define MAC_HANDOFF_BYTES(R) (MAC_CLUSTER_MAX_LD * sizeof(R) + MAC_CLUSTER_MAX_LD / MAC_CLUSTER_CHUNK * sizeof(int))
 
 __device__ __forceinline__ void cluster_barrier()
 {
     asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
+}
+// barrier of the CTAs of one env
+template <bool CLUSTER> __device__ __forceinline__ void env_barrier()
+{
+    if (CLUSTER) cluster_barrier();
+    else __syncthreads();
 }
 __device__ __forceinline__ unsigned cluster_rank()
 {
@@ -499,8 +143,20 @@ __device__ __forceinline__ int ld_acquire_cluster(const int *p)
     return v;
 }
 
-template <typename R, int TI, int TJ, int T>
-__global__ void __launch_bounds__(T) mac_cluster_kernel(const MacArgs<R> a)
+// G > 1: the wavefront hand-off buffers, after the phi slabs and transport planes in dynamic shared memory
+// (MacEnv sizes both): new values of rank g-1's last row by column, and one flag per chunk of it that holds
+// the sub-step sequence number once the chunk is ready
+template <typename R> __device__ __forceinline__ R *handoff_west(R *phiA, const MacArgs<R> &a)
+{
+    return phiA + a.ld * max(2 * a.slab_rows, 3 * ((a.slab_rows - 2 + a.tr_pass - 1) / a.tr_pass));
+}
+template <typename R> __device__ __forceinline__ int *handoff_flags(R *phiA, const MacArgs<R> &a)
+{
+    return reinterpret_cast<int *>(handoff_west(phiA, a) + MAC_CLUSTER_MAX_LD);
+}
+
+template <typename R, int TI, int TJ, int T, bool CLUSTER>
+__global__ void __launch_bounds__(T) mac_kernel(const MacArgs<R> a)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     __shared__ R s_part[2][MAC_CLUSTER_MAX][T / 32];   // residual partials of every rank, by sweep parity
@@ -509,10 +165,8 @@ __global__ void __launch_bounds__(T) mac_cluster_kernel(const MacArgs<R> a)
     __shared__ int s_bad[MAC_CLUSTER_MAX];            // per-rank non-finite flags
     __shared__ R s_seg[128];
     __shared__ R s_act[128];
-    __shared__ R s_west[MAC_CLUSTER_MAX_LD];          // new values of rank g-1's last row, by column
-    __shared__ int s_flag[MAC_CLUSTER_MAX_LD / MAC_CLUSTER_CHUNK];   // == substep sequence: chunk of s_west ready
-    const int tid = threadIdx.x, G = a.G;
-    const unsigned rank = cluster_rank();
+    const int tid = threadIdx.x, G = CLUSTER ? a.G : 1;
+    const unsigned rank = CLUSTER ? cluster_rank() : 0;
     const int b = blockIdx.x / G;
     const int nx = a.nx, ny = a.ny, ld = a.ld;
     const bool resetting = a.mode == 1;
@@ -545,7 +199,8 @@ __global__ void __launch_bounds__(T) mac_cluster_kernel(const MacArgs<R> a)
     _Pragma("unroll") for (int k = 0; k < TJ; k++)
 #define CELL_OK(i, j) (has_tile && (i) <= ie && (j) <= ny)
 
-    for (int e = tid; e < MAC_CLUSTER_MAX_LD / MAC_CLUSTER_CHUNK; e += T) s_flag[e] = 0;
+    if (CLUSTER)
+        for (int e = tid; e < MAC_CLUSTER_MAX_LD / MAC_CLUSTER_CHUNK; e += T) handoff_flags(phiA, a)[e] = 0;
 
     // ---- load / reset (own rows) -----------------------------------------------------------------
     if (resetting) {
@@ -558,7 +213,7 @@ __global__ void __launch_bounds__(T) mac_cluster_kernel(const MacArgs<R> a)
             for (int e = tid; e < (ray ? a.n_sgts : 0); e += T) a.a_cur[(size_t)b * a.n_sgts + e] = R(0);
             if (tid == 0) { a.stp[b] = 0; if (!ray) a.a_int[b] = 1; }
         }
-        cluster_barrier();
+        env_barrier<CLUSTER>();
         if (first) {                                           // history zero, newest slot from the init state
             R *hist = a.obs_hist + (size_t)b * a.n_obs;
             const int per_step = 3 * a.nx_obs_pts * a.ny_obs_pts;
@@ -579,7 +234,7 @@ __global__ void __launch_bounds__(T) mac_cluster_kernel(const MacArgs<R> a)
     }
     int stp = a.stp[b];
     int status = 0, seq = 0;
-    cluster_barrier();                                         // s_flag cleared in every rank
+    env_barrier<CLUSTER>();                                    // s_flag cleared in every rank
 
     for (int act = 0; act < a.n_fused; act++) {
         const size_t orow = (size_t)act * a.B + b;
@@ -612,7 +267,7 @@ __global__ void __launch_bounds__(T) mac_cluster_kernel(const MacArgs<R> a)
 
         for (int it = 0; it < a.ndt_act; it++) {
             seq += 1;
-            // ---- boundary conditions (as mac_kernel), own walls and own i range --------------------
+            // ---- boundary conditions: rayleigh.py:180-202, mixing.py:153-171, own walls and own i range ----
             {
                 const int nl = first ? ny + 2 : 0, nr = last ? ny + 2 : 0;
                 const int ihi = last ? nx + 1 : ie, ni = ihi - ib + 1;
@@ -648,7 +303,7 @@ __global__ void __launch_bounds__(T) mac_cluster_kernel(const MacArgs<R> a)
                 }
             }
             for (int e = tid; e < 2 * slab; e += T) phiA[e] = R(0);   // both planes: they doubled as transport scratch
-            cluster_barrier();                                 // walls of the neighbours; zeroed halos before any push
+            env_barrier<CLUSTER>();                            // walls of the neighbours; zeroed halos before any push
 
             // ---- predictor (own rows; reads the neighbours' wall rows) ---------------------------------
             CELL_LOOP {
@@ -679,7 +334,7 @@ __global__ void __launch_bounds__(T) mac_cluster_kernel(const MacArgs<R> a)
                     }
                 }
             }
-            cluster_barrier();                                 // us of row ie + 1 comes from rank g + 1
+            env_barrier<CLUSTER>();                            // us of row ie + 1 comes from rank g + 1
 
             // ---- Poisson right-hand side into registers --------------------------------------------------
             R c[TI][TJ];
@@ -729,8 +384,9 @@ __global__ void __launch_bounds__(T) mac_cluster_kernel(const MacArgs<R> a)
                 }
                 acc = warp_sum(acc);
                 const int lane = tid & 31, warp = tid >> 5;
-                if (lane < G) cluster_map(&s_part[itp & 1][rank][warp], lane)[0] = acc;
-                cluster_barrier();
+                if (!CLUSTER) { if (lane == 0) s_part[itp & 1][0][warp] = acc; }
+                else if (lane < G) cluster_map(&s_part[itp & 1][rank][warp], lane)[0] = acc;
+                env_barrier<CLUSTER>();
                 err = R(0);
                 for (int g = 0; g < G; g++) {                  // same partials, same order in every thread of the cluster
                     R eg = s_part[itp & 1][g][0];
@@ -755,13 +411,15 @@ __global__ void __launch_bounds__(T) mac_cluster_kernel(const MacArgs<R> a)
                     if (j >= 2) v[i * ld + j] = vs[i * ld + j] - a.dt * (phi[li * ld + j] - phi[li * ld + j - 1]) * a.inv_dy;
                 }
             }
-            cluster_barrier();                                 // u of row ie + 1 comes from rank g + 1
+            env_barrier<CLUSTER>();                            // u of row ie + 1 comes from rank g + 1
 
             // ---- transport: coefficients per pass in the phi planes, wavefront chained over the ranks -----
             {
                 const int passes = a.tr_pass, rows = (S + passes - 1) / passes;
                 R *cA = phiA, *cW = phiA + rows * ld, *cS = phiA + 2 * rows * ld;
                 const R kx = a.tcoef * a.inv_dx2, ky = a.tcoef * a.inv_dy2;
+                R *s_west = handoff_west(phiA, a);
+                int *s_flag = handoff_flags(phiA, a);
                 int *right_flag = last ? nullptr : cluster_map(s_flag, rank + 1);
                 R *right_west = last ? nullptr : cluster_map(s_west, rank + 1);
                 for (int ps = 0; ps < passes; ps++) {
@@ -829,7 +487,7 @@ __global__ void __launch_bounds__(T) mac_cluster_kernel(const MacArgs<R> a)
                 }
             }
         }   // sub-steps
-        cluster_barrier();                                     // every rank's rows done
+        env_barrier<CLUSTER>();                                // every rank's rows done
 
         // ---- observations and reward: rank 0 writes, every rank contributes its rows -----------------
         R part = R(0);
@@ -838,7 +496,8 @@ __global__ void __launch_bounds__(T) mac_cluster_kernel(const MacArgs<R> a)
         bool nonfinite = false;
         for (int e = e0 + tid; e < e1; e += T) nonfinite |= !finite_(s[e]) | !finite_(u[e]) | !finite_(v[e]);
         const int bad = __syncthreads_or(nonfinite ? 1 : 0);
-        if (tid < G) { cluster_map(s_rank, tid)[rank] = part; cluster_map(s_bad, tid)[rank] = bad; }
+        if (!CLUSTER) { if (tid == 0) { s_rank[0] = part; s_bad[0] = bad; } }
+        else if (tid < G) { cluster_map(s_rank, tid)[rank] = part; cluster_map(s_bad, tid)[rank] = bad; }
         if (first) {
             R *hist = a.obs_hist + (size_t)b * a.n_obs;
             const int per_step = 3 * a.nx_obs_pts * a.ny_obs_pts;
@@ -861,7 +520,7 @@ __global__ void __launch_bounds__(T) mac_cluster_kernel(const MacArgs<R> a)
         R nu = R(0);
         if (first && ray && tid == 0)                          // rayleigh.py:265-275 (sequential sum over i)
             for (int i = 1; i <= nx; i++) nu -= (s[i * ld + 1] - a.Th) / (R(0.5) * a.dy);
-        cluster_barrier();                                     // partials in place; obs read before the next walls
+        env_barrier<CLUSTER>();                                // partials in place; obs read before the next walls
         int any_bad = 0;
         R total = R(0);
         for (int g = 0; g < G; g++) { any_bad |= s_bad[g]; total += s_rank[g]; }   // rank order
@@ -876,7 +535,7 @@ __global__ void __launch_bounds__(T) mac_cluster_kernel(const MacArgs<R> a)
     }   // actions
 
     if (first && tid == 0) { a.stp[b] = stp; if (a.status) a.status[b] = status; }
-    cluster_barrier();                                         // no CTA leaves while a neighbour may write its shared memory
+    env_barrier<CLUSTER>();                                    // no CTA leaves while a neighbour may write its shared memory
 #undef CELL_LOOP
 #undef CELL_OK
 }
@@ -1012,14 +671,6 @@ __device__ __noinline__ bool residual_converged_exact(R mine, R *s_exact, R tol)
 // half-warp fall into 16 distinct 8-byte banks iff (TI * LDP) mod 16 == 2 (TI = 2: 57, TI = 5: 58).
 constexpr int mac_ldp(int ld, int ti) { int l = ld; while ((ti * l) % 16 != 2) l++; return l; }
 
-#ifdef MAC_CLUSTER_BARRIER_TEST
-#define SWEEP_BARRIER() asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory")
-#else
-#define SWEEP_BARRIER() __syncthreads()
-#endif
-#ifndef MAC_REG_P_SCRATCH
-#define MAC_REG_P_SCRATCH 1
-#endif
 template <typename R, int NX, int NY, int TI, int TJ, int T, bool DBG>
 __global__ void __launch_bounds__(T, 2) mac_reg_kernel(const MacArgs<R> a)
 {
@@ -1113,16 +764,10 @@ __global__ void __launch_bounds__(T, 2) mac_reg_kernel(const MacArgs<R> a)
     // the neighbour tile's cell is the same slot 1 / TILES_J threads away.  The plane keeps the launch-initial values
     // until the end: ghost cells of p only ever accumulate the same increments as their wall-adjacent cells (phi
     // ghosts are copies) and never feed back, so they are brought up to date once, at the end of the launch.
-    constexpr bool PSC = MAC_REG_P_SCRATCH && TI * TJ * T <= N;
+    static_assert(TI * TJ * T <= N, "the pressure scratch must fit the vs plane");
     R *const sp = a.vs + row + tid;
 #define PSCR(r, k) sp[((r) * TJ + (k)) * T]
-    if (PSC) {
-        if (has_tile) { TILE_LOOP { PSCR(r, k) = gp[o + r * LD + k]; } }
-    } else if (has_tile && (top || bot || lef || rig)) {
-        const R *p = gp + o;
-        R *sv = a.us + row + o;
-        TILE_LOOP { sv[r * LD + k] = p[r * LD + k]; }
-    }
+    if (has_tile) { TILE_LOOP { PSCR(r, k) = gp[o + r * LD + k]; } }
     int stp = a.stp[b];
     int status = 0;
     const R dt = a.dt, inv_dx = a.inv_dx, inv_dy = a.inv_dy;
@@ -1197,13 +842,15 @@ __global__ void __launch_bounds__(T, 2) mac_reg_kernel(const MacArgs<R> a)
         R us[TI][TJ], vs[TI][TJ];
         auto predictor = [&]() {
             const R2 *uv = UV + ou;
-            const R *p = gp + o;
+            // Not read (the pressure comes from the scratch).  It keeps gp and o among the lambda's captures, on which
+            // nvcc's code for this kernel depends: without it the fp64 instance spills 8 B more.
+            [[maybe_unused]] const R *p = gp + o;
             // (u, v) pairs of the tile and its one-cell ring are fetched as 16-byte words where they are used (equal
             // addresses are merged by the compiler)
             TILE_LOOP {
                 const R2 *q = uv + r * LDU + k;
                 const R2 c = q[0], E = q[LDU], W = q[-LDU], Nn = q[1], Ss = q[-1];
-                const R uc = c.x, vc = c.y, pc = PSC ? PSCR(r, k) : p[r * LD + k];
+                const R uc = c.x, vc = c.y, pc = PSCR(r, k);
                 us[r][k] = R(0); vs[r][k] = R(0);
                 if (r > 0 || !top) {               // i >= 2
                     R uE = R(0.5) * (E.x + uc), uW = R(0.5) * (uc + W.x);
@@ -1211,7 +858,7 @@ __global__ void __launch_bounds__(T, 2) mac_reg_kernel(const MacArgs<R> a)
                     R vN = R(0.5) * (Nn.y + q[-LDU + 1].y), vS = R(0.5) * (vc + W.y);
                     R conv = (uE * uE - uW * uW) * inv_dx + (uN * vN - uS * vS) * inv_dy;
                     R diff = ((E.x - R(2) * uc + W.x) * a.inv_dx2 + (Nn.x - R(2) * uc + Ss.x) * a.inv_dy2) * a.dcoef;
-                    const R pw = !PSC ? p[r * LD + k - LD] : (r > 0 ? PSCR(r - 1, k) : (sp - TILES_J)[((TI - 1) * TJ + k) * T]);
+                    const R pw = r > 0 ? PSCR(r - 1, k) : (sp - TILES_J)[((TI - 1) * TJ + k) * T];
                     R pres = (pc - pw) * inv_dx;
                     us[r][k] = diff - conv - pres;
                 }
@@ -1221,7 +868,7 @@ __global__ void __launch_bounds__(T, 2) mac_reg_kernel(const MacArgs<R> a)
                     R vN = R(0.5) * (Nn.y + vc), vS = R(0.5) * (vc + Ss.y);
                     R conv = (uE * vE - uW * vW) * inv_dx + (vN * vN - vS * vS) * inv_dy;
                     R diff = ((E.y - R(2) * vc + W.y) * a.inv_dx2 + (Nn.y - R(2) * vc + Ss.y) * a.inv_dy2) * a.dcoef;
-                    const R ps = !PSC ? p[r * LD + k - 1] : (k > 0 ? PSCR(r, k - 1) : (sp - 1)[(r * TJ + TJ - 1) * T]);
+                    const R ps = k > 0 ? PSCR(r, k - 1) : (sp - 1)[(r * TJ + TJ - 1) * T];
                     R pres = (pc - ps) * inv_dy;
                     vs[r][k] = diff - conv - pres;
                 }
@@ -1467,7 +1114,7 @@ __global__ void __launch_bounds__(T, 2) mac_reg_kernel(const MacArgs<R> a)
                     if (converged(err, accq)) { itp = k - 2; pf = pb; break; }
                     commit(phi, pb);
                     if ((tid & 31) == 0) s_part[0][tid >> 5] = ws;
-                    SWEEP_BARRIER();
+                    __syncthreads();
                     accq = accp; accp = acc;
                 }
                 {   // even k+1: phi_k (in PB) -> phi_{k+1}; decide on sweep k-1 (still in PA)
@@ -1478,7 +1125,7 @@ __global__ void __launch_bounds__(T, 2) mac_reg_kernel(const MacArgs<R> a)
                     if (converged(err, accq)) { itp = k - 1; pf = pa; break; }
                     commit(phi, pa);
                     if ((tid & 31) == 0) s_part[1][tid >> 5] = ws;
-                    SWEEP_BARRIER();
+                    __syncthreads();
                     accq = accp; accp = acc;
                 }
             }
@@ -1488,10 +1135,9 @@ __global__ void __launch_bounds__(T, 2) mac_reg_kernel(const MacArgs<R> a)
 
             // ---- p += phi (rayleigh.py:219; ghost cells: see the end of the launch) and in-place corrector (:461-464)
             if (has_tile) {
-                R *p = gp + o;
                 R2 *uv = UV + ou;
                 TILE_LOOP {
-                    if (PSC) PSCR(r, k) += phi[r][k]; else p[r * LD + k] += phi[r][k];
+                    PSCR(r, k) += phi[r][k];
                     R2 w = uv[r * LDU + k];
                     if (r > 0 || !top) { const R pw = (r > 0) ? phi[r - 1][k] : pf[-LDP + k]; w.x = w.x - dt * (phi[r][k] - pw) * inv_dx; }
                     if (k > 0 || !lef) { const R ps = (k > 0) ? phi[r][k - 1] : pf[r * LDP - 1]; w.y = w.y - dt * (phi[r][k] - ps) * inv_dy; }
@@ -1592,46 +1238,25 @@ __global__ void __launch_bounds__(T, 2) mac_reg_kernel(const MacArgs<R> a)
         const R2 w = UV[i * LDU + j];
         gu[e] = w.x; gv[e] = w.y; gs[e] = SS(i, j);
     }
-    if (PSC) {                                         // pressure back to its plane; ghost += adjacent(final) - adjacent(launch start)
-        if (has_tile) {
-            R *pp = gp + o;
-            if (top) {
-#pragma unroll
-                for (int k = 0; k < TJ; k++) pp[-LD + k] += PSCR(0, k) - pp[k];
-            }
-            if (bot) {
-#pragma unroll
-                for (int k = 0; k < TJ; k++) pp[TI * LD + k] += PSCR(TI - 1, k) - pp[(TI - 1) * LD + k];
-            }
-            if (lef) {
-#pragma unroll
-                for (int r = 0; r < TI; r++) pp[r * LD - 1] += PSCR(r, 0) - pp[r * LD];
-            }
-            if (rig) {
-#pragma unroll
-                for (int r = 0; r < TI; r++) pp[r * LD + TJ] += PSCR(r, TJ - 1) - pp[r * LD + TJ - 1];
-            }
-            TILE_LOOP { pp[r * LD + k] = PSCR(r, k); }
-        }
-    } else if (has_tile && (top || bot || lef || rig)) {      // ghost cells of p += this launch's increments of the adjacent cell
-        R *p = gp + o;
-        const R *sv = a.us + row + o;
+    if (has_tile) {                                    // pressure back to its plane; ghost += adjacent(final) - adjacent(launch start)
+        R *pp = gp + o;
         if (top) {
 #pragma unroll
-            for (int k = 0; k < TJ; k++) p[-LD + k] += p[k] - sv[k];
+            for (int k = 0; k < TJ; k++) pp[-LD + k] += PSCR(0, k) - pp[k];
         }
         if (bot) {
 #pragma unroll
-            for (int k = 0; k < TJ; k++) p[TI * LD + k] += p[(TI - 1) * LD + k] - sv[(TI - 1) * LD + k];
+            for (int k = 0; k < TJ; k++) pp[TI * LD + k] += PSCR(TI - 1, k) - pp[(TI - 1) * LD + k];
         }
         if (lef) {
 #pragma unroll
-            for (int r = 0; r < TI; r++) p[r * LD - 1] += p[r * LD] - sv[r * LD];
+            for (int r = 0; r < TI; r++) pp[r * LD - 1] += PSCR(r, 0) - pp[r * LD];
         }
         if (rig) {
 #pragma unroll
-            for (int r = 0; r < TI; r++) p[r * LD + TJ] += p[r * LD + TJ - 1] - sv[r * LD + TJ - 1];
+            for (int r = 0; r < TI; r++) pp[r * LD + TJ] += PSCR(r, TJ - 1) - pp[r * LD + TJ - 1];
         }
+        TILE_LOOP { pp[r * LD + k] = PSCR(r, k); }
     }
     if (tid == 0) { a.stp[b] = stp; if (a.status) a.status[b] = status; }
     if (DBG && dbg) { for (int n = 0; n < (DBG ? 8 : 1); n++) a.dbg[n] += (unsigned long long)tph[n]; }
@@ -1709,12 +1334,6 @@ __device__ __noinline__ void transport_wavefront3(uint32_t offA, uint32_t offW, 
 // L2-resident global memory (Poisson is > 90 % of the work: ~65 sweeps per sub-step), transport in
 // row passes through the three-plane wavefront above.  One CTA per SM.
 // ---------------------------------------------------------------------------------------
-#ifndef MAC_BIG_COPYOUT_BY_TILE
-#define MAC_BIG_COPYOUT_BY_TILE 0
-#endif
-#ifndef MAC_BIG_TRCOEF_BY_TILE
-#define MAC_BIG_TRCOEF_BY_TILE 0
-#endif
 template <typename R, int NX, int NY, int TI, int TJ, int T, int MINB, bool DBG>
 __global__ void __launch_bounds__(T, MINB) mac_big_kernel(const MacArgs<R> a)
 {
@@ -2041,32 +1660,6 @@ __global__ void __launch_bounds__(T, MINB) mac_big_kernel(const MacArgs<R> a)
             }
             int itp;
             const R *pf;                                  // plane holding the final iterate (tile-relative)
-#ifdef MAC_BIG_DECIDE_LAST
-            for (int k = 3;; k += 2) {
-                {   // odd k: phi_{k-1} (in PA) -> phi_k; decide on sweep k-2 (still in PB)
-                    float ws = (float)accp;
-                    const R acc = sweep(phi, pa, ws) * w_has;
-                    const float err = total32(s_part[1]);
-                    if (k - 2 > a.itmax) { status |= BEACON_STATUS_POISSON_OVERFLOW; itp = k - 2; pf = pb; break; }
-                    if (converged(err, accq)) { itp = k - 2; pf = pb; break; }
-                    commit(phi, pb);
-                    if ((tid & 31) == 0) s_part[0][tid >> 5] = ws;
-                    __syncthreads();
-                    accq = accp; accp = acc;
-                }
-                {   // even k+1: phi_k (in PB) -> phi_{k+1}; decide on sweep k-1 (still in PA)
-                    float ws = (float)accp;
-                    const R acc = sweep(phi, pb, ws) * w_has;
-                    const float err = total32(s_part[0]);
-                    if (k - 1 > a.itmax) { status |= BEACON_STATUS_POISSON_OVERFLOW; itp = k - 1; pf = pa; break; }
-                    if (converged(err, accq)) { itp = k - 1; pf = pa; break; }
-                    commit(phi, pa);
-                    if ((tid & 31) == 0) s_part[1][tid >> 5] = ws;
-                    __syncthreads();
-                    accq = accp; accp = acc;
-                }
-            }
-#else
             // One CTA per SM: nobody fills the gaps of a sweep, so the tile stores must overlap the arithmetic.  The
             // stores of sweep k overwrite phi_{k-2}, which a converged solve returns — hence the decision on sweep k-2
             // (partials published at the previous barrier) is taken FIRST, right after the west halo loads are issued,
@@ -2130,7 +1723,6 @@ __global__ void __launch_bounds__(T, MINB) mac_big_kernel(const MacArgs<R> a)
                 st = iter(pb, pa, s_part[0], s_part[1], k - 1);
                 if (st) { if (st == 2) status |= BEACON_STATUS_POISSON_OVERFLOW; itp = k - 1; pf = pa; break; }
             }
-#endif
             TILE_LOOP { phi[r][k] = pf[r * LDP + k]; }     // the converged iterate
             it_total += itp;
             PHASE(2);
@@ -2166,45 +1758,13 @@ __global__ void __launch_bounds__(T, MINB) mac_big_kernel(const MacArgs<R> a)
                 R *AA = PA, *WW = reinterpret_cast<R *>(smem_raw + PLANE_B), *SS = reinterpret_cast<R *>(smem_raw + 2 * PLANE_B);
                 for (int ps = 0; ps < PASSES; ps++) {
                     const int ib = 1 + ps * PASS_ROWS, ie = min(NX, ib + PASS_ROWS - 1);
-                    const bool mine = has_tile && i0 >= ib && i0 <= ie;       // passes are tile aligned
                     typedef typename vec2_of<R>::type R2;
-                    static_assert(TI % 2 == 0 && PASS_ROWS % 2 == 0, "row pairs of a tile are whole wavefront slots");
-                    // [row pair][column][row in pair]: the two rows of a pair are ONE 16-byte slot (tiles are an even number
-                    // of rows high and passes start on tile boundaries): half the store instructions, conflict free
-                    R2 *A2 = reinterpret_cast<R2 *>(AA) + ((i0 - ib) >> 1) * RS + j0, *W2 = reinterpret_cast<R2 *>(WW) + ((i0 - ib) >> 1) * RS + j0,
-                       *S2 = reinterpret_cast<R2 *>(SS) + ((i0 - ib) >> 1) * RS + j0;
-#if MAC_BIG_TRCOEF_BY_TILE
-                    if (mine) {
-                        const R *uu = u + o, *vv = v + o, *sc = s + o;
-#pragma unroll
-                        for (int rp = 0; rp < TI; rp += 2)
-#pragma unroll
-                            for (int k = 0; k < TJ; k++) {
-                                R2 xa, xw, xs;
-#pragma unroll
-                                for (int q = 0; q < 2; q++) {
-                                    const int r = rp + q, e = r * LD + k;
-                                    const R uE = uu[e + LD], uW = uu[e], vN = vv[e + 1], vS = vv[e];
-                                    const R s0 = sc[e], sE = sc[e + LD], sN = sc[e + 1];
-                                    R diff0 = ((sE - R(2) * s0) * a.inv_dx2 + (sN - R(2) * s0) * a.inv_dy2) * a.tcoef;
-                                    R conv0 = (uE * (R(0.5) * (sE + s0)) - uW * (R(0.5) * s0)) * inv_dx + (vN * (R(0.5) * (sN + s0)) - vS * (R(0.5) * s0)) * inv_dy;
-                                    R A = s0 + dt * (diff0 - conv0);
-                                    R BW = dt * (kx + R(0.5) * uW * inv_dx);
-                                    R BS = dt * (ky + R(0.5) * vS * inv_dy);
-                                    if (k == 0 && lef) { A = fma(BS, sc[e - 1], A); BS = R(0); }                 // south ghost column
-                                    if (r == 0 && i0 == ib) { A = fma(BW, sc[e - LD], A); BW = R(0); }           // row west of the pass
-                                    if (q == 0) { xa.x = A; xw.x = BW; xs.x = BS; } else { xa.y = A; xw.y = BW; xs.y = BS; }
-                                }
-                                A2[(rp >> 1) * RS + k] = xa; W2[(rp >> 1) * RS + k] = xw; S2[(rp >> 1) * RS + k] = xs;
-                            }
-                    }
-#else
+                    static_assert(PASS_ROWS % 2 == 0, "a pass is LANES_MAX whole row pairs");
                     // The coefficients are a pointwise function of old values, so for this phase the cells are dealt out
                     // row-contiguous instead of by tile: a thread takes row-pair slots (rows i, i + 1 at column j) with
                     // consecutive j across the lanes — every global load of u, v, C is coalesced (the tile-wise loads touched
                     // ~10 cache lines per warp instruction) and all 512 threads work in both passes.
                     {
-                        (void)mine; (void)A2; (void)W2; (void)S2;
                         const int nslots = ((ie - ib + 2) >> 1) * NY;
                         R2 *Ap = reinterpret_cast<R2 *>(AA), *Wp = reinterpret_cast<R2 *>(WW), *Sp = reinterpret_cast<R2 *>(SS);
                         constexpr int TRIPS = ((PASS_ROWS / 2) * NY + T - 1) / T;
@@ -2235,23 +1795,11 @@ __global__ void __launch_bounds__(T, MINB) mac_big_kernel(const MacArgs<R> a)
                             }
                         }
                     }
-#endif
                     __syncthreads();
                     PHASE(4);
                     if (tid < 32) transport_wavefront3<R, NY>(0u, PLANE_B, 2 * PLANE_B, (ie - ib + 2) / 2, tid);
                     __syncthreads();
                     PHASE(5);
-#if MAC_BIG_COPYOUT_BY_TILE
-                    if (mine) {
-#pragma unroll
-                        for (int rp = 0; rp < TI; rp += 2)
-#pragma unroll
-                            for (int k = 0; k < TJ; k++) {
-                                const R2 x = A2[(rp >> 1) * RS + k];
-                                s[o + rp * LD + k] = x.x; s[o + (rp + 1) * LD + k] = x.y;
-                            }
-                    }
-#else
                     // the transported rows back to the plane, by ALL threads and row-contiguous (a warp writes 32
                     // consecutive cells of one row: 2-3 cache lines instead of the ~10 a tile-wise store touches)
                     {
@@ -2262,7 +1810,6 @@ __global__ void __launch_bounds__(T, MINB) mac_big_kernel(const MacArgs<R> a)
                             s[(ib + ri) * LD + j] = AAs[(((ri >> 1) * RS + j) << 1) + (ri & 1)];
                         }
                     }
-#endif
                     __syncthreads();
                     PHASE(6);
                 }
@@ -2345,7 +1892,7 @@ __global__ void __launch_bounds__(T, MINB) mac_big_kernel(const MacArgs<R> a)
 }
 
 // ---------------------------------------------------------------------------------------
-// Capacity of mac_cluster_kernel with G CTAs per env: "" when (nx, ny) fits, else the reason.
+// Capacity of mac_kernel with G > 1 CTAs per env: "" when (nx, ny) fits, else the reason.
 // Slabs of at least MAC_CLUSTER_MIN_ROWS rows; 4x5 tiles of the thickest slab within 512 threads; two phi
 // slab planes of (rows + 2) x (ny + 2) in the shared-memory budget; ny + 2 within the hand-off buffers.
 // The transport coefficients take 3 planes of a pass of at most 32 * MAC_RPL rows (cluster_passes).
@@ -2402,12 +1949,12 @@ public:
         info.rwd_dim = 1; info.n_act = p.n_act; info.noise_dim = 0;
 
         MacArgs<R> &a = base;
-        // kernel variant: all planes in shared memory when 8 planes fit, else phi planes only;
-        // ctas_per_env = G > 1 selects mac_cluster_kernel on any grid
+        // kernel: mac_reg_kernel and mac_big_kernel for their grids, else mac_kernel with the whole array in
+        // one CTA; ctas_per_env = G > 1 selects mac_kernel over a cluster of G CTAs on any grid
         const size_t plane = (size_t)n * sizeof(R);
         int TI, TJ;
-        G = p.ctas_per_env;
-        BEACON_REQUIRE(G >= 0, "mac2d: ctas_per_env must be >= 0 (0 and 1: one CTA per env)");
+        BEACON_REQUIRE(p.ctas_per_env >= 0, "mac2d: ctas_per_env must be >= 0 (0 and 1: one CTA per env)");
+        G = std::max(p.ctas_per_env, 1);
         if (G > 1) {
             const std::string why = cluster_misfit<R>(nx, ny, G);
             if (why.size()) throw Error(BEACON_ERR_UNSUPPORTED, "mac2d: ctas_per_env=" + std::to_string(G) + ": " + why);
@@ -2417,16 +1964,10 @@ public:
             // selected below, after the transport passes
         } else if (ray && nx == 50 && ny == 50 && p.n_sgts <= 32 && !getenv("BEACON_MAC_V1")) {
             // five planes fit twice per SM: register-resident phi tiles, 2 CTAs/SM
-            const char *tile = getenv("BEACON_MAC_TILE");              // tuning: "5x5" = 100 threads with 25 cells each
-            if (tile && !strcmp(tile, "5x5")) {
-                kernel = mac_reg_kernel<R, 50, 50, 5, 5, 128, false>;
-                T = 128; TI = 5; TJ = 5;
-            } else {
-                if (getenv("BEACON_MAC_DEBUG")) kernel = mac_reg_kernel<R, 50, 50, 2, 5, 256, true>;
-                else kernel = mac_reg_kernel<R, 50, 50, 2, 5, 256, false>;
-                T = 256; TI = 2; TJ = 5; dbg_variant = true;
-            }
-            smem = sizeof(R) * (2 * (size_t)((51 * mac_ldp(52, TI) + 3) / 4 * 4) + 2 * 52 * 53 + 52 * mac_ldp(52, TI)); reg_variant = true;
+            if (getenv("BEACON_MAC_DEBUG")) kernel = mac_reg_kernel<R, 50, 50, 2, 5, 256, true>;
+            else kernel = mac_reg_kernel<R, 50, 50, 2, 5, 256, false>;
+            T = 256; TI = 2; TJ = 5; dbg_variant = true;
+            smem = sizeof(R) * (2 * (size_t)((51 * mac_ldp(52, 2) + 3) / 4 * 4) + 2 * 52 * 53 + 52 * mac_ldp(52, 2)); reg_variant = true;
         } else if (nx == 100 && ny == 100 && !getenv("BEACON_MAC_V1")) {
             // register-resident Poisson, fields in L2: one CTA of 500 tile threads per SM
             if (getenv("BEACON_MAC_DEBUG")) kernel = mac_big_kernel<R, 100, 100, 4, 5, 512, 1, true>;
@@ -2445,16 +1986,17 @@ public:
         a.tr_pass = 1;
         while (3 * (size_t)((nx + a.tr_pass - 1) / a.tr_pass) * ld > 2 * (size_t)n || (nx + a.tr_pass - 1) / a.tr_pass > 32 * MAC_RPL)
             a.tr_pass++;
+        a.G = G; a.slab_rows = nx + 2;                                  // mac_kernel at G = 1: the slab is the whole array
         if (G > 1) {
-            // one cluster of G CTAs per env: slab rows, phi slab planes + transport passes (cluster_misfit)
+            // one cluster of G CTAs per env: slab rows, phi slab planes + transport passes (cluster_misfit), hand-off buffers
             const int Smax = (nx + G - 1) / G;
-            a.G = G; a.slab_rows = Smax + 2;
+            a.slab_rows = Smax + 2;
             a.tr_pass = cluster_passes<R>(Smax, ld);
             const int rows = (Smax + a.tr_pass - 1) / a.tr_pass;
-            kernel = mac_cluster_kernel<R, 4, 5, 512>; T = 512; TI = 4; TJ = 5;
-            smem = sizeof(R) * (size_t)ld * std::max(2 * a.slab_rows, 3 * rows);
+            kernel = mac_kernel<R, 4, 5, 512, true>; T = 512; TI = 4; TJ = 5;
+            smem = sizeof(R) * (size_t)ld * std::max(2 * a.slab_rows, 3 * rows) + MAC_HANDOFF_BYTES(R);
         }
-        BEACON_CUDA_CHECK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        raise_dynamic_smem_limit(kernel, smem);
         if (G > 1) {
             cudaLaunchConfig_t cfg = {};
             cudaLaunchAttribute at[1];
@@ -2516,18 +2058,7 @@ public:
             cfg.attrs = at; cfg.numAttrs = 1;
             BEACON_CUDA_CHECK(cudaLaunchKernelEx(&cfg, kernel, a));
         } else
-#ifdef MAC_CLUSTER_BARRIER_TEST
-        {
-            cudaLaunchConfig_t cfg = {};
-            cfg.gridDim = dim3(a.B); cfg.blockDim = dim3(T); cfg.dynamicSmemBytes = smem; cfg.stream = st;
-            cudaLaunchAttribute at[1];
-            at[0].id = cudaLaunchAttributeClusterDimension; at[0].val.clusterDim.x = 4; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-            cfg.attrs = at; cfg.numAttrs = 1;
-            BEACON_CUDA_CHECK(cudaLaunchKernelEx(&cfg, kernel, a));
-        }
-#else
-        kernel<<<a.B, T, smem, st>>>(a);
-#endif
+            kernel<<<a.B, T, smem, st>>>(a);
         BEACON_CUDA_CHECK(cudaGetLastError());
         launches++;
         if (debug && dbg_variant && a.mode == 0) {

@@ -580,7 +580,7 @@ public:
         smem = sizeof(R) * ((size_t)2 * XN * T + 2 * (size_t)nx + 2 * (size_t)p.ndt_act + 6 * (size_t)(nj ? nj : 1) + a.jz_len + 2 * C) +
                sizeof(short) * (size_t)a.jz_len + 16;
         BEACON_REQUIRE(smem <= 227 * 1024, "shkadov: shared-memory budget exceeded");
-        BEACON_CUDA_CHECK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        raise_dynamic_smem_limit(kernel, smem);
     }
 
     void launch(const ShkArgs<R> &a, cudaStream_t s)

@@ -1,6 +1,7 @@
-"""rayleigh / mixing with one environment split over a thread-block cluster (ctas_per_env = G > 1,
-mac_cluster_kernel, DESIGN.md §3.6): grids no single CTA holds against the oracle, the cluster path against
-the single-CTA kernels on the same grid, determinism, plumbing, fp32 and the host-side capacity rule."""
+"""rayleigh / mixing with one environment split over a thread-block cluster (ctas_per_env = G > 1: the generic
+mac_kernel over G CTAs, DESIGN.md §3.6): grids no single CTA holds against the oracle, the cluster path against
+the single-CTA kernels on the same grid (for 100x50 that is the same mac_kernel at G = 1), determinism, plumbing,
+fp32 and the host-side capacity rule."""
 import math
 
 import numpy as np

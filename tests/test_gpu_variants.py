@@ -479,8 +479,8 @@ def test_sloshing_capacity_rejected():
 # ============================================================================= mac2d
 def mac_dispatch(kind, nx, ny, n_sgts=0, real_bytes=8):
     """Mirror of MacEnv: (kernel, tiles of 4x5 cells, transport passes).  rayleigh 50x50 with n_sgts <= 32:
-    mac_reg_kernel; any 100x100 grid: mac_big_kernel; else the generic mac_kernel when two planes fit
-    in shared memory and the 4x5 tiles in 512 threads; else None (rejected)."""
+    mac_reg_kernel; any 100x100 grid: mac_big_kernel; else the generic mac_kernel on one CTA per env (G = 1)
+    when two planes fit in shared memory and the 4x5 tiles in 512 threads; else None (rejected)."""
     ld, n = ny + 2, (nx + 2) * (ny + 2)
     tiles = ((nx + 3) // 4) * ((ny + 4) // 5)
     if kind == "rayleigh" and nx == ny == 50 and n_sgts <= 32:
@@ -574,6 +574,26 @@ def test_rayleigh_segment_layouts(n_sgts, kernel, n_actions):
         close(obs, np.stack([r[0] for r in ref]), what="obs")
         close(rwd, np.array([r[1] for r in ref]), rtol=1e-12, what="rwd")
     assert int(env.status.max()) == 0
+
+
+def test_smaller_env_keeps_the_shared_memory_limit():
+    """The dynamic shared-memory limit is an attribute of the kernel function, shared by every env on that
+    instance: creating a smaller env after a larger one must not lower it below what the larger env launches
+    with.  mac_kernel: rayleigh 200x50 (168,064 B), then 75x61 (77,616 B); shkadov 6,256,2: nx 1536, then 1350.
+    Both envs of each pair are reset and stepped after both were created."""
+    assert mac_dispatch("rayleigh", 200, 50, 5)[0] == mac_dispatch("rayleigh", 75, 61, 5)[0] == "mac_kernel"
+    kws = [dict(init=False, L=4.0, H=1.0, n_sgts=5), dict(init=False, L=1.5, H=1.22, n_sgts=5)]
+    envs = [make("rayleigh", 2, **kw) for kw in kws]
+    for env in envs:
+        env.reset()
+        env.step(torch.zeros(2, 5, dtype=torch.float64))
+        assert int(env.status.max()) == 0
+    assert shk_dispatch(1536)[0] == shk_dispatch(1350)[0] == V6
+    envs = [make("shkadov", 2, init="rest", L0=shk_l0(nx), n_jets=10) for nx in (1536, 1350)]
+    for env in envs:
+        obs0 = env.reset()
+        obs, rwd, d, t = env.step(torch.zeros(2, 10, dtype=torch.float64))
+        assert obs.shape == obs0.shape and bool(torch.isfinite(obs).all())
 
 
 def test_mac2d_grids_rejected():

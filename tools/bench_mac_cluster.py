@@ -7,9 +7,12 @@ Cases:
     B * G a multiple of the B200's 148 SMs, so that the GPU is full;
   * mixing 100x100 at small batches (8, 16, 37 envs) on one CTA per env (mac_big_kernel) against 2 and 4:
     whether spreading an env over idle SMs lowers the latency of a step;
-  * rayleigh 100x50 from rest, 16 envs, on the generic one-CTA mac_kernel (G = 1) and on 2, 4, 8 CTAs: the
-    same grid and the same sweep counts, so the difference of the time per sweep isolates what the cluster
-    path adds per sweep (its cluster barrier and DSMEM exchange) net of the work the split saves.
+  * rayleigh 100x50 from rest, 16 envs, on the generic mac_kernel at G = 1 (one CTA per env) and on 2, 4, 8
+    CTAs: the same grid and the same sweep counts, so the difference of the time per sweep isolates what the
+    cluster path adds per sweep (its cluster barrier and DSMEM exchange) net of the work the split saves;
+  * the generic mac_kernel at G = 1 on a full GPU (148 envs, one per SM) on rayleigh 100x50, 75x61 (partial
+    tiles) and 200x50 (500 tile threads, four transport passes), from rest: the one-CTA throughput of the
+    kernel that also runs the clusters, tight enough to show a small change.
 Each case: reset, one warm-up action, then `--repeats` windows of `--steps` actions timed with CUDA events
 (random actions, one launch each; actions differ between windows).  Per window:
   env_actions_per_s = B * steps / time;
@@ -40,6 +43,8 @@ CASES = (
     + [("mixing 200x200", "mixing", dict(L=2.0, H=2.0), 8, 37)]
     + [("mixing 100x100", "mixing", dict(), G, B) for B in (8, 16, 37) for G in (1, 2, 4)]
     + [(PAIR, "rayleigh", dict(init=False, L=2.0, n_sgts=5), G, 16) for G in (1, 2, 4, 8)]
+    + [(label, "rayleigh", dict(init=False, L=L, H=H, n_sgts=5), 1, 148)
+       for label, L, H in ((PAIR, 2.0, 1.0), ("rayleigh 75x61", 1.5, 1.22), ("rayleigh 200x50", 4.0, 1.0))]
 )
 
 
@@ -101,8 +106,9 @@ def main():
         rows.append(r)
         print(json.dumps(r), flush=True)
     # same grid, same sweep counts: extra time per sweep of the cluster path over the generic one-CTA kernel
-    base = next(r for r in rows if r["case"] == PAIR and r["G"] == 1)["us_per_sweep"]["median"]
-    extra = {r["G"]: r["us_per_sweep"]["median"] - base for r in rows if r["case"] == PAIR and r["G"] > 1}
+    pair = [r for r in rows if r["case"] == PAIR and r["B"] == 16]
+    base = next(r for r in pair if r["G"] == 1)["us_per_sweep"]["median"]
+    extra = {r["G"]: r["us_per_sweep"]["median"] - base for r in pair if r["G"] > 1}
     print(json.dumps({"case": PAIR, "extra_us_per_sweep_vs_G1": extra}), flush=True)
     if args.out:
         with open(args.out, "w") as f:
