@@ -125,13 +125,14 @@ def _cfg_env(variant):
     return ",".join(str(x) for x in variant)
 
 
-def shk_vs_oracle(envs, nx, n_jets, C, n_actions=3, rtol=1e-10, per_jet=False, seed=0):
+def shk_vs_oracle(envs, nx, n_jets, C, n_actions=3, rtol=1e-10, per_jet=False, seed=0, **kw):
     """Synthetic state into every env and the oracle, then n_actions actions with random jet actions and
     explicit inlet noise, each env re-synced from the oracle before each action (the film is chaotic,
-    SURVEY.md §4); h, q, rhsh, rhsq, obs, rewards and flags compared after each action."""
+    SURVEY.md §4); h, q, rhsh, rhsq, obs, rewards and flags compared after each action.  kw: further
+    oracle constructor arguments (delta, jet_pos), the same the envs were made with."""
     B = envs[0].batch
     L0 = shk_l0(nx, n_jets)
-    orcs = [bo.shkadov(init=False, L0=L0, n_jets=n_jets) for _ in range(B)]
+    orcs = [bo.shkadov(init=False, L0=L0, n_jets=n_jets, **kw) for _ in range(B)]
     for b, o in enumerate(orcs):
         assert o.nx == nx
         o.h[:], o.q[:] = shk_synthetic(nx, b)
