@@ -59,7 +59,10 @@ EXPORTS = (
     "beacon_env_reset", "beacon_env_step", "beacon_env_step_host", "beacon_env_field", "beacon_env_get_state",
     "beacon_env_set_state", "beacon_env_launch_count", "beacon_last_error", "beacon_version",
     "beacon_peer_alloc", "beacon_peer_export", "beacon_peer_open", "beacon_peer_close", "beacon_peer_free",
+    "beacon_env_set_physics", "beacon_env_get_physics",
 )
+# per-env physical parameters of beacon_env_set_physics, by env
+PHYSICS = {"rayleigh": ("ra",), "mixing": ("re", "pe")}
 PEER_HANDLE_BYTES = 64
 
 _lib = None
@@ -95,6 +98,8 @@ def lib():
     L.beacon_env_field.argtypes = [vp, _i32, C.POINTER(C.c_char_p), C.POINTER(C.c_int64), C.POINTER(_i32)]
     L.beacon_env_get_state.argtypes = [vp, C.c_char_p, vp, vp]
     L.beacon_env_set_state.argtypes = [vp, C.c_char_p, vp, vp]
+    L.beacon_env_set_physics.argtypes = [vp, C.c_char_p, dp, vp]
+    L.beacon_env_get_physics.argtypes = [vp, C.c_char_p, dp, vp]
     L.beacon_env_launch_count.argtypes = [vp]
     L.beacon_env_launch_count.restype = C.c_int64
     L.beacon_peer_alloc.argtypes = [_i32, C.c_uint64, C.POINTER(vp)]

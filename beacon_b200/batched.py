@@ -22,6 +22,10 @@ def _dp(a):
     return a.ctypes.data_as(C.POINTER(C.c_double))
 
 
+def _host(x):
+    return x.detach().cpu().numpy() if isinstance(x, torch.Tensor) else x
+
+
 class BatchedEnv:
     """`BatchedEnv("shkadov", batch=1024, n_jets=10)`; kwargs are the reference ctor's.
 
@@ -29,6 +33,11 @@ class BatchedEnv:
     step(actions, noise=None)     -> obs [B, n_obs], rwd [B] (or [B, n_jets]), done [B], trunc [B]
     step_fused(actions[K,B,...])  -> same with a leading K axis: K consecutive actions, one launch
     get_state(name) / set_state(name, tensor)
+
+    Per-env physical parameters (rayleigh `ra`; mixing `re`, `pe`): each may be a scalar, as in the
+    reference, or a 1-D array / list / tensor of length `batch`, one value per env; set_physics(**values)
+    changes them between launches (domain randomisation: draw values for the finished envs, set_physics,
+    reset(mask=done)), get_physics(name) reads them back.  All envs of a batch still share one launch.
 
     ctas_per_env (rayleigh / mixing): how many SMs one environment may occupy.  1 runs each env on one
     CTA (grids up to ~100x100 cells); 2..8 split each env over a thread-block cluster of that many CTAs,
@@ -47,6 +56,11 @@ class BatchedEnv:
             raise capi.BeaconError("beacon_b200 needs a CUDA device (B200, sm_100a); there is no CPU fallback")
         self.name, self.batch, self.dtype, self.ctas_per_env = name, int(batch), dtype, int(ctas_per_env)
         self.device = torch.device("cuda", device)
+        per_env = {}
+        for k in capi.PHYSICS.get(name, ()):
+            if k in kwargs and np.ndim(_host(kwargs[k])) != 0:
+                per_env[k] = self._physics_values(k, kwargs.pop(k))   # the handle is created at the default
+        self._per_env_physics = False
         self.cfg = CFG[name](**kwargs)
         d = self.cfg.d
         if init_state:                       # the reference's load(): fields that replace the shipped initial state
@@ -118,6 +132,8 @@ class BatchedEnv:
             self.fields[nm.value.decode()] = (cnt.value, bool(isint.value))
         self.status = torch.zeros(self.batch, dtype=torch.int32, device=self.device)
         self.last_iters = None
+        if per_env:
+            self.set_physics(**per_env)
 
     # ------------------------------------------------------------------------------------
     def __del__(self):
@@ -314,12 +330,52 @@ class BatchedEnv:
     def state_dict(self):
         """Full device state (binary checkpoint; SURVEY.md §5 'Checkpoint / resume'), including the
         per-env Philox draw counter of the inlet noise ("draws", shkadov / burgers): a restored env
-        continues the same noise stream as an uninterrupted one."""
-        return {k: self.get_state(k).cpu() for k in self.fields}
+        continues the same noise stream as an uninterrupted one.  A handle with per-env physical
+        parameters also carries them ("ra", or "re" and "pe", float64 [B])."""
+        sd = {k: self.get_state(k).cpu() for k in self.fields}
+        if self._per_env_physics:
+            sd.update({k: self.get_physics(k) for k in capi.PHYSICS[self.name]})
+        return sd
 
     def load_state_dict(self, sd):
+        phys = {k: v for k, v in sd.items() if k in capi.PHYSICS.get(self.name, ())}
+        if phys:
+            self.set_physics(**phys)
         for k, v in sd.items():
-            self.set_state(k, v)
+            if k not in phys:
+                self.set_state(k, v)
+
+    # ------------------------------------------------------------------------------------
+    def _physics_values(self, name, values):
+        if name not in capi.PHYSICS.get(self.name, ()):
+            have = capi.PHYSICS.get(self.name)
+            raise ValueError(f"{self.name} has no per-env physical parameter '{name}'" +
+                             (f" (it has {', '.join(have)})" if have else " (only rayleigh and mixing have them)"))
+        v = np.ascontiguousarray(_host(values), dtype=np.float64)
+        if v.shape != (self.batch,):
+            raise ValueError(f"{name}: expected a scalar or {self.batch} per-env values, got shape {v.shape}")
+        if not (np.all(np.isfinite(v)) and np.all(v > 0)):
+            raise ValueError(f"{name}: per-env values must be finite and > 0")
+        return v
+
+    def set_physics(self, **values):
+        """Per-env physical parameters, one array of length `batch` each: rayleigh `ra`; mixing `re`
+        (which also sets the wall speed u_max = re nu / L) and `pe`.  Stream-ordered: the values apply from
+        the next reset or step.  Every value is checked before any is applied."""
+        vals = {k: self._physics_values(k, v) for k, v in values.items()}
+        with torch.cuda.device(self.device):
+            for k, v in vals.items():
+                capi.check(self._lib.beacon_env_set_physics(self._h, k.encode(), _dp(v), self._stream()))
+                self._per_env_physics = True
+
+    def get_physics(self, name):
+        """float64 [B] CPU tensor of the per-env values of `name` (the handle's scalar for every env
+        while none has been set)."""
+        self._physics_values(name, np.ones(self.batch))
+        out = np.empty(self.batch, dtype=np.float64)
+        with torch.cuda.device(self.device):
+            capi.check(self._lib.beacon_env_get_physics(self._h, name.encode(), _dp(out), self._stream()))
+        return torch.from_numpy(out)
 
     @property
     def launches(self):

@@ -228,6 +228,23 @@ int beacon_env_set_state(beacon_env *env, const char *field, const void *buf, be
     return copy_state(env, field, nullptr, buf, stream);
 }
 
+int beacon_env_set_physics(beacon_env *env, const char *name, const double *values, beacon_stream_t stream)
+{
+    return guard([&] {
+        BEACON_REQUIRE(env, "NULL handle");
+        BEACON_CUDA_CHECK(cudaSetDevice(env->impl->common.device));
+        env->impl->set_physics(name, values, (cudaStream_t)stream);
+    });
+}
+int beacon_env_get_physics(beacon_env *env, const char *name, double *values, beacon_stream_t stream)
+{
+    return guard([&] {
+        BEACON_REQUIRE(env, "NULL handle");
+        BEACON_CUDA_CHECK(cudaSetDevice(env->impl->common.device));
+        env->impl->get_physics(name, values, (cudaStream_t)stream);
+    });
+}
+
 int beacon_peer_alloc(int32_t device, uint64_t bytes, void **ptr)
 {
     return guard([&] {

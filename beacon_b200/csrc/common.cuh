@@ -299,6 +299,15 @@ public:
     virtual ~Env() {}
     virtual void reset(const ResetArgs &a) = 0;
     virtual void step(const StepArgs &a) = 0;
+    // per-env physical parameters (beacon_env_set_physics / get_physics): rayleigh and mixing only
+    virtual void set_physics(const char *, const double *, cudaStream_t)
+    {
+        throw Error(BEACON_ERR_INVALID, "per-env physical parameters apply to rayleigh and mixing only");
+    }
+    virtual void get_physics(const char *, double *, cudaStream_t)
+    {
+        throw Error(BEACON_ERR_INVALID, "per-env physical parameters apply to rayleigh and mixing only");
+    }
 
     int real_bytes() const { return info.dtype == BEACON_F64 ? 8 : 4; }
     const Field *find(const char *name) const

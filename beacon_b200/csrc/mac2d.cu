@@ -66,7 +66,21 @@ template <typename R> struct MacArgs {
     int32_t *status;
     int64_t *iters;
     unsigned long long *dbg;   // optional per-phase cycle counters (BEACON_MAC_DEBUG), block 0 only
+    const R *phys;             // per-env instances: [B][3] rows of (dcoef, tcoef, u_max), built by mac_phys_derive
 };
+
+// The physical constants of an env inside the kernel bodies (template switch PHYS): the handle's
+// (a.dcoef, a.tcoef, a.u_max) in the uniform instances, whose machine code is the same as before the
+// switch existed; in the per-env instances the env's row of a.phys, read once per CTA into the static
+// shared array s_coef (MAC_LOAD_COEF, before a CTA barrier) and broadcast from there.  Every CTA of a
+// cluster belongs to one env and reads the same row.  Names, not locals: a new local captured by the
+// bodies' lambdas would change the register allocation of the uniform instances (DESIGN.md 3.7).
+#define MAC_DCOEF (PHYS ? s_coef[0] : a.dcoef)
+#define MAC_TCOEF (PHYS ? s_coef[1] : a.tcoef)
+#define MAC_UMAX (PHYS ? s_coef[2] : a.u_max)
+#define MAC_LOAD_COEF(b)                                  \
+    __shared__ R s_coef[3];                               \
+    if (PHYS && tid < 3) s_coef[tid] = a.phys[3 * (size_t)(b) + tid]
 
 // numpy pairwise sum for n <= 128 (np.mean of the action vector, rayleigh.py:165)
 template <typename R> __device__ R np_pairwise_small(const R *a, int n)
@@ -155,8 +169,8 @@ template <typename R> __device__ __forceinline__ int *handoff_flags(R *phiA, con
     return reinterpret_cast<int *>(handoff_west(phiA, a) + MAC_CLUSTER_MAX_LD);
 }
 
-template <typename R, int TI, int TJ, int T, bool CLUSTER>
-__global__ void __launch_bounds__(T) mac_kernel(const MacArgs<R> a)
+template <typename R, int TI, int TJ, int T, bool CLUSTER, bool PHYS>
+__device__ __forceinline__ void mac_body(const MacArgs<R> a, const unsigned thread_x)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     __shared__ R s_part[2][MAC_CLUSTER_MAX][T / 32];   // residual partials of every rank, by sweep parity
@@ -165,12 +179,13 @@ __global__ void __launch_bounds__(T) mac_kernel(const MacArgs<R> a)
     __shared__ int s_bad[MAC_CLUSTER_MAX];            // per-rank non-finite flags
     __shared__ R s_seg[128];
     __shared__ R s_act[128];
-    const int tid = threadIdx.x, G = CLUSTER ? a.G : 1;
+    const int tid = thread_x, G = CLUSTER ? a.G : 1;
     const unsigned rank = CLUSTER ? cluster_rank() : 0;
     const int b = blockIdx.x / G;
     const int nx = a.nx, ny = a.ny, ld = a.ld;
     const bool resetting = a.mode == 1;
     if (resetting && a.mask && !a.mask[b]) return;     // uniform over the cluster: no DSMEM access yet
+    MAC_LOAD_COEF(b);                                  // read after the env barrier below
     const bool ray = a.kind == BEACON_RAYLEIGH;
     const bool first = rank == 0, last = rank == (unsigned)G - 1;
 
@@ -255,10 +270,10 @@ __global__ void __launch_bounds__(T) mac_kernel(const MacArgs<R> a)
         } else if (tid == 0) {                                     // get_control, mixing.py:212-234
             int ai = ((const int32_t *)a.actions)[orow];
             R ut = 0, ub = 0, vl = 0, vr = 0;
-            if (ai == 0) { ub = a.u_max; ut = -a.u_max; }
-            if (ai == 1) { ub = -a.u_max; ut = a.u_max; }
-            if (ai == 2) { vr = a.u_max; vl = -a.u_max; }
-            if (ai == 3) { vr = -a.u_max; vl = a.u_max; }
+            if (ai == 0) { ub = MAC_UMAX; ut = -MAC_UMAX; }
+            if (ai == 1) { ub = -MAC_UMAX; ut = MAC_UMAX; }
+            if (ai == 2) { vr = MAC_UMAX; vl = -MAC_UMAX; }
+            if (ai == 3) { vr = -MAC_UMAX; vl = MAC_UMAX; }
             s_seg[0] = ut; s_seg[1] = ub; s_seg[2] = vl; s_seg[3] = vr;
             if (first) a.a_int[b] = ai;
         }
@@ -316,7 +331,7 @@ __global__ void __launch_bounds__(T) mac_kernel(const MacArgs<R> a)
                         R vN = R(0.5) * (v[i * ld + j + 1] + v[(i - 1) * ld + j + 1]), vS = R(0.5) * (vc + v[(i - 1) * ld + j]);
                         R conv = (uE * uE - uW * uW) * a.inv_dx + (uN * vN - uS * vS) * a.inv_dy;
                         R diff = ((u[(i + 1) * ld + j] - R(2) * uc + u[(i - 1) * ld + j]) * a.inv_dx2 +
-                                  (u[i * ld + j + 1] - R(2) * uc + u[i * ld + j - 1]) * a.inv_dy2) * a.dcoef;
+                                  (u[i * ld + j + 1] - R(2) * uc + u[i * ld + j - 1]) * a.inv_dy2) * MAC_DCOEF;
                         R pres = (p[i * ld + j] - p[(i - 1) * ld + j]) * a.inv_dx;
                         us[i * ld + j] = uc + a.dt * (diff - conv - pres);
                     }
@@ -326,7 +341,7 @@ __global__ void __launch_bounds__(T) mac_kernel(const MacArgs<R> a)
                         R vN = R(0.5) * (v[i * ld + j + 1] + vc), vS = R(0.5) * (vc + v[i * ld + j - 1]);
                         R conv = (uE * vE - uW * vW) * a.inv_dx + (vN * vN - vS * vS) * a.inv_dy;
                         R diff = ((v[(i + 1) * ld + j] - R(2) * vc + v[(i - 1) * ld + j]) * a.inv_dx2 +
-                                  (v[i * ld + j + 1] - R(2) * vc + v[i * ld + j - 1]) * a.inv_dy2) * a.dcoef;
+                                  (v[i * ld + j + 1] - R(2) * vc + v[i * ld + j - 1]) * a.inv_dy2) * MAC_DCOEF;
                         R pres = (p[i * ld + j] - p[i * ld + j - 1]) * a.inv_dy;
                         R rhs = diff - conv - pres;
                         if (ray) rhs += s[i * ld + j];
@@ -417,7 +432,7 @@ __global__ void __launch_bounds__(T) mac_kernel(const MacArgs<R> a)
             {
                 const int passes = a.tr_pass, rows = (S + passes - 1) / passes;
                 R *cA = phiA, *cW = phiA + rows * ld, *cS = phiA + 2 * rows * ld;
-                const R kx = a.tcoef * a.inv_dx2, ky = a.tcoef * a.inv_dy2;
+                const R kx = MAC_TCOEF * a.inv_dx2, ky = MAC_TCOEF * a.inv_dy2;
                 R *s_west = handoff_west(phiA, a);
                 int *s_flag = handoff_flags(phiA, a);
                 int *right_flag = last ? nullptr : cluster_map(s_flag, rank + 1);
@@ -431,7 +446,7 @@ __global__ void __launch_bounds__(T) mac_kernel(const MacArgs<R> a)
                         if (CELL_OK(i, j) && i >= pb && i <= pe) {
                             const R uE = u[(i + 1) * ld + j], uW = u[i * ld + j], vN = v[i * ld + j + 1], vS = v[i * ld + j];
                             const R sc = s[i * ld + j], sE = s[(i + 1) * ld + j], sN = s[i * ld + j + 1];
-                            R diff0 = ((sE - R(2) * sc) * a.inv_dx2 + (sN - R(2) * sc) * a.inv_dy2) * a.tcoef;
+                            R diff0 = ((sE - R(2) * sc) * a.inv_dx2 + (sN - R(2) * sc) * a.inv_dy2) * MAC_TCOEF;
                             R conv0 = (uE * (R(0.5) * (sE + sc)) - uW * (R(0.5) * sc)) * a.inv_dx +
                                       (vN * (R(0.5) * (sN + sc)) - vS * (R(0.5) * sc)) * a.inv_dy;
                             const int e = (i - pb) * ld + j;
@@ -539,6 +554,13 @@ __global__ void __launch_bounds__(T) mac_kernel(const MacArgs<R> a)
 #undef CELL_LOOP
 #undef CELL_OK
 }
+// The wrappers read threadIdx.x, where __launch_bounds__ bounds it, and mac_body takes MacArgs by value: otherwise
+// the uniform instance compiles to different code (DESIGN.md 3.7).
+template <typename R, int TI, int TJ, int T, bool CLUSTER>
+__global__ void __launch_bounds__(T) mac_kernel(const MacArgs<R> a) { mac_body<R, TI, TJ, T, CLUSTER, false>(a, threadIdx.x); }
+// per-env physical constants (MacArgs::phys)
+template <typename R, int TI, int TJ, int T, bool CLUSTER>
+__global__ void __launch_bounds__(T) mac_phys_kernel(const MacArgs<R> a) { mac_body<R, TI, TJ, T, CLUSTER, true>(a, threadIdx.x); }
 
 
 // ---------------------------------------------------------------------------------------
@@ -671,602 +693,16 @@ __device__ __noinline__ bool residual_converged_exact(R mine, R *s_exact, R tol)
 // half-warp fall into 16 distinct 8-byte banks iff (TI * LDP) mod 16 == 2 (TI = 2: 57, TI = 5: 58).
 constexpr int mac_ldp(int ld, int ti) { int l = ld; while ((ti * l) % 16 != 2) l++; return l; }
 
-template <typename R, int NX, int NY, int TI, int TJ, int T, bool DBG>
-__global__ void __launch_bounds__(T, 2) mac_reg_kernel(const MacArgs<R> a)
-{
-    typedef typename vec2_of<R>::type R2;
-    constexpr int LD = NY + 2, N = (NX + 2) * LD;       // field planes in global memory
-    constexpr int LDP = mac_ldp(LD, TI);                // exchange planes: conflict-free stride (8-byte elements)
-    constexpr int NP = ((NX + 1) * LDP + 3) / 4 * 4;    // rows 0 .. NX (no ghost row NX+1: wall tiles read their own edge)
-    // u and v live INTERLEAVED in one plane of (u, v) pairs: the tile origins of a quarter-warp fall into 8 distinct
-    // 16-byte bank groups iff 2 LDU = 2 mod 8 (LDU = 53), one LDS.128 fetches both components, and every access is
-    // conflict free — two separate planes of stride NY+2 = 52 cannot be (the banks 0, 5, 8, 13 are oversubscribed for
-    // 2x5 tiles whatever the thread mapping; a stride of 57 for each does not fit twice per SM).  T uses the stride
-    // of the exchange planes.  Measured: shared-memory bank conflicts were 25 % of all wavefronts before.
-    constexpr int LDU = ((LD + 2) / 4) * 4 + 1, NU = (NX + 2) * LDU;      // in (u, v) pairs
-    constexpr int LDT = LDP, NT = (NX + 2) * LDT;
-    static_assert(TI != 2 || (2 * LDU) % 8 == 2, "u/v plane stride");
-    constexpr int TILES_J = NY / TJ, TILES = (NX / TI) * TILES_J, NW = T / 32;
-    static_assert(NX % TI == 0 && NY % TJ == 0 && TILES <= T, "tiles must cover the grid exactly");
-    static_assert(NX <= 64, "transport wavefront: two rows per lane");
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    __shared__ __align__(16) float s_part[2][NW];     // fp32 warp partials of the residual (see the Poisson section)
-    __shared__ R s_exact[NW];                         // fp64 warp partials, only when the fp32 total is too close to tol
-    __shared__ R s_seg[32];
-    __shared__ R s_act[32];
-    static_assert((NP * sizeof(R)) % 16 == 0, "planes must stay 16-byte aligned");
-    const int tid = threadIdx.x, b = blockIdx.x;
-    const bool resetting = a.mode == 1;
-    if (resetting && a.mask && !a.mask[b]) return;
-
-    R *PA = reinterpret_cast<R *>(smem_raw), *PB = PA + NP;
-    R2 *UV = reinterpret_cast<R2 *>(PB + NP);
-    R *S = reinterpret_cast<R *>(UV + NU);
-    const size_t row = (size_t)b * N;
-    R *gu = a.u + row, *gv = a.v + row, *gp = a.p + row, *gs = a.s + row;
-
-    const bool has_tile = tid < TILES;
-    const int ti = tid / TILES_J, tj = tid - ti * TILES_J;
-    const int i0 = 1 + ti * TI, j0 = 1 + tj * TJ;
-    const int o = i0 * LD + j0, op = i0 * LDP + j0;     // tile origin in global field / exchange planes
-    const int ou = i0 * LDU + j0, ot = i0 * LDT + j0;   // ... in the (u, v) plane and in the T plane
-    const int opx = has_tile ? op : LDP + 1;             // threads without a tile shadow tile 0 in the sweeps (weight 0)
-    const bool top = has_tile && i0 == 1, bot = has_tile && i0 + TI - 1 == NX;
-    const bool lef = has_tile && j0 == 1, rig = has_tile && j0 + TJ - 1 == NY;
-    const R w_has = has_tile ? R(1) : R(0);
-    const R w_top = top ? R(2) : R(1), w_bot = bot ? R(2) : R(1), w_lef = lef ? R(1) : R(0), w_rig = rig ? R(1) : R(0);
-    // Halo offsets of the Jacobi sweeps.  All ghost cells of phi are Neumann copies of the wall-adjacent cell
-    // (rayleigh.py:436-445), so a wall tile reads that cell — its own edge row / column in the exchange plane —
-    // instead of a ghost: no ghost cell of phi is ever stored (30 predicated stores per thread and sweep, ~10
-    // shared-memory wavefronts per warp and sweep, gone).  Threads without a tile shadow tile 0.
-    const int tix = has_tile ? ti : 0, tjx = has_tile ? tj : 0;
-    const int o_n = tix == 0 ? 0 : -LDP, o_s = tix == NX / TI - 1 ? (TI - 1) * LDP : TI * LDP;
-#define TILE_LOOP                                      \
-    _Pragma("unroll") for (int r = 0; r < TI; r++)     \
-    _Pragma("unroll") for (int k = 0; k < TJ; k++)
-
-    if (resetting) {                                   // rayleigh.py:89-128
-        for (int e = tid; e < N; e += T) { gu[e] = a.u0[e]; gv[e] = a.v0[e]; gp[e] = a.p0[e]; gs[e] = a.s0[e]; }
-        for (int e = tid; e < a.n_sgts; e += T) a.a_cur[(size_t)b * a.n_sgts + e] = R(0);
-        const int per_step = 3 * a.nx_obs_pts * a.ny_obs_pts;
-        R *hist = a.obs_hist + (size_t)b * a.n_obs;
-        for (int e = tid; e < a.n_obs; e += T) {
-            int st = e / per_step, rem = e - st * per_step;
-            R val = R(0);
-            if (st == a.n_obs_steps - 1) {
-                int f = rem / (a.nx_obs_pts * a.ny_obs_pts), q = rem - f * (a.nx_obs_pts * a.ny_obs_pts);
-                int pi = q / a.ny_obs_pts, pj = q - pi * a.ny_obs_pts;
-                int x = a.nx_obs / 2 + pi * a.nx_obs, y = a.ny_obs / 2 + pj * a.ny_obs;
-                val = (f == 0) ? a.s0[x * LD + y] : (f == 1 ? a.u0[x * LD + y] : a.v0[x * LD + y]);
-            }
-            hist[e] = val;
-            a.obs[(size_t)b * a.n_obs + e] = val;
-        }
-        if (tid == 0) a.stp[b] = 0;
-        return;
-    }
-    for (int e = tid; e < 2 * NP; e += T) PA[e] = R(0);   // masked wavefront steps read padding slots: keep them finite
-    // state planes global -> shared, into the padded / interleaved layouts (once per launch)
-    for (int e = tid; e < N; e += T) {
-        const int i = e / LD, j = e - i * LD;
-        R2 w; w.x = gu[e]; w.y = gv[e];
-        UV[i * LDU + j] = w;
-        S[i * LDT + j] = gs[e];
-    }
-    for (int e = tid; e < NX + 2; e += T) {            // padding columns: read by masked wavefront steps, keep them finite
-        for (int j = LD; j < LDU; j++) { R2 z; z.x = R(0); z.y = R(0); UV[e * LDU + j] = z; }
-        for (int j = LD; j < LDT; j++) S[e * LDT + j] = R(0);
-    }
-    __syncthreads();
-    // The pressure stays in global memory (L2).  During the launch the authoritative copy of a thread's tile lives in a
-    // scratch laid out [cell][thread] (the `vs` workspace plane): a tile row is 5 doubles at an odd offset in the plane,
-    // so a tile-wise warp access touches ~13 cache lines, in the scratch consecutive lanes are contiguous (2 lines) and
-    // the neighbour tile's cell is the same slot 1 / TILES_J threads away.  The plane keeps the launch-initial values
-    // until the end: ghost cells of p only ever accumulate the same increments as their wall-adjacent cells (phi
-    // ghosts are copies) and never feed back, so they are brought up to date once, at the end of the launch.
-    static_assert(TI * TJ * T <= N, "the pressure scratch must fit the vs plane");
-    R *const sp = a.vs + row + tid;
-#define PSCR(r, k) sp[((r) * TJ + (k)) * T]
-    if (has_tile) { TILE_LOOP { PSCR(r, k) = gp[o + r * LD + k]; } }
-    int stp = a.stp[b];
-    int status = 0;
-    const R dt = a.dt, inv_dx = a.inv_dx, inv_dy = a.inv_dy;
-    const bool dbg = DBG && a.dbg != nullptr && b == 0 && tid == 0;
-    long long tph[DBG ? 8 : 1] = {0}, tlast = dbg ? clock64() : 0;
-#define PHASE(n) do { if (DBG && dbg) { long long tn_ = clock64(); tph[n] += tn_ - tlast; tlast = tn_; } } while (0)
-
-    for (int act = 0; act < a.n_fused; act++) {
-        const size_t orow = (size_t)act * a.B + b;
-        __syncthreads();
-        if (tid == 0) {                                            // rayleigh.py:164-171
-            const R *ain = (const R *)a.actions + orow * a.n_sgts;
-            const int ns = a.n_sgts;
-            for (int j = 0; j < ns; j++) s_act[j] = ain[j];
-            R mean = np_pairwise_small(s_act, ns) / R(ns);
-            R m = R(1);
-            for (int j = 0; j < ns; j++) { s_act[j] = s_act[j] - mean; m = np_max(m, rabs(s_act[j]) / a.Cmax); }
-            for (int j = 0; j < ns; j++) { s_act[j] = s_act[j] / m; s_seg[j] = a.Th + s_act[j]; a.a_cur[(size_t)b * ns + j] = s_act[j]; }
-        }
-        __syncthreads();
-        long long it_total = 0;
-
-#define UU(i, j) UV[(i) * LDU + (j)].x
-#define VV(i, j) UV[(i) * LDU + (j)].y
-#define SS(i, j) S[(i) * LDT + (j)]
-        // ---- boundary conditions, rayleigh.py:180-202, split by field: the velocity ghosts do not depend on T, the
-        // T ghosts need the transported T.  Executed by the threads t0, t0 + nt, ... of the caller's group.
-        auto bc_uv = [&](const int t0, const int nt, const bool walls) {
-            for (int k = t0; k < 2 * (NX + 2) + 2 * (NY + 2); k += nt) {
-                if (k < NY + 2) {
-                    int j = k;
-                    if (walls && j >= 1 && j <= NY) UU(1, j) = R(0);
-                    if (j >= 2 && j <= NY) VV(0, j) = -VV(1, j);
-                } else if (k < 2 * (NY + 2)) {
-                    int j = k - (NY + 2);
-                    if (walls && j >= 1 && j <= NY) UU(NX + 1, j) = R(0);
-                    if (j >= 2 && j <= NY) VV(NX + 1, j) = -VV(NX, j);
-                } else if (k < 2 * (NY + 2) + (NX + 2)) {
-                    int i = k - 2 * (NY + 2);
-                    if (i >= 1 && i <= NX + 1) UU(i, NY + 1) = (i == 1 || i == NX + 1) ? -R(0) : -UU(i, NY);
-                    if (walls && i >= 1 && i <= NX) VV(i, NY + 1) = R(0);
-                } else {
-                    int i = k - 2 * (NY + 2) - (NX + 2);
-                    if (i >= 1 && i <= NX + 1) UU(i, 0) = (i == 1 || i == NX + 1) ? -R(0) : -UU(i, 1);
-                    if (walls && i >= 1 && i <= NX) VV(i, 1) = R(0);
-                }
-            }
-        };
-        auto bc_s = [&](const int t0, const int nt) {
-            for (int k = t0; k < 2 * (NX + 2) + 2 * (NY + 2); k += nt) {
-                if (k < NY + 2) {
-                    int j = k;
-                    if (j >= 1 && j <= NY) SS(0, j) = SS(1, j);
-                } else if (k < 2 * (NY + 2)) {
-                    int j = k - (NY + 2);
-                    if (j >= 1 && j <= NY) SS(NX + 1, j) = SS(NX, j);
-                } else if (k < 2 * (NY + 2) + (NX + 2)) {
-                    int i = k - 2 * (NY + 2);
-                    if (i >= 1 && i <= NX) SS(i, NY + 1) = R(2) * a.Tc - SS(i, NY);
-                } else {
-                    int i = k - 2 * (NY + 2) - (NX + 2);
-                    if (i >= 1 && i <= NX) {
-                        int sg = (i - 1) / a.nx_sgts;
-                        if (sg < a.n_sgts) SS(i, 0) = R(2) * s_seg[sg] - SS(i, 1);
-                    }
-                }
-            }
-        };
-        // ---- predictor into registers, rayleigh.py:371-407: the right-hand sides of u* and v* (v: WITHOUT the buoyancy
-        // term); u* = u + dt rhs_u and v* = v + dt (rhs_v + T) are formed later with the transported T: the same
-        // operations in the same order as the reference's expressions
-        R us[TI][TJ], vs[TI][TJ];
-        auto predictor = [&]() {
-            const R2 *uv = UV + ou;
-            // Not read (the pressure comes from the scratch).  It keeps gp and o among the lambda's captures, on which
-            // nvcc's code for this kernel depends: without it the fp64 instance spills 8 B more.
-            [[maybe_unused]] const R *p = gp + o;
-            // (u, v) pairs of the tile and its one-cell ring are fetched as 16-byte words where they are used (equal
-            // addresses are merged by the compiler)
-            TILE_LOOP {
-                const R2 *q = uv + r * LDU + k;
-                const R2 c = q[0], E = q[LDU], W = q[-LDU], Nn = q[1], Ss = q[-1];
-                const R uc = c.x, vc = c.y, pc = PSCR(r, k);
-                us[r][k] = R(0); vs[r][k] = R(0);
-                if (r > 0 || !top) {               // i >= 2
-                    R uE = R(0.5) * (E.x + uc), uW = R(0.5) * (uc + W.x);
-                    R uN = R(0.5) * (Nn.x + uc), uS = R(0.5) * (uc + Ss.x);
-                    R vN = R(0.5) * (Nn.y + q[-LDU + 1].y), vS = R(0.5) * (vc + W.y);
-                    R conv = (uE * uE - uW * uW) * inv_dx + (uN * vN - uS * vS) * inv_dy;
-                    R diff = ((E.x - R(2) * uc + W.x) * a.inv_dx2 + (Nn.x - R(2) * uc + Ss.x) * a.inv_dy2) * a.dcoef;
-                    const R pw = r > 0 ? PSCR(r - 1, k) : (sp - TILES_J)[((TI - 1) * TJ + k) * T];
-                    R pres = (pc - pw) * inv_dx;
-                    us[r][k] = diff - conv - pres;
-                }
-                if (k > 0 || !lef) {               // j >= 2
-                    R vE = R(0.5) * (E.y + vc), vW = R(0.5) * (vc + W.y);
-                    R uE = R(0.5) * (E.x + q[LDU - 1].x), uW = R(0.5) * (uc + Ss.x);
-                    R vN = R(0.5) * (Nn.y + vc), vS = R(0.5) * (vc + Ss.y);
-                    R conv = (uE * vE - uW * vW) * inv_dx + (vN * vN - vS * vS) * inv_dy;
-                    R diff = ((E.y - R(2) * vc + W.y) * a.inv_dx2 + (Nn.y - R(2) * vc + Ss.y) * a.inv_dy2) * a.dcoef;
-                    const R ps = k > 0 ? PSCR(r, k - 1) : (sp - 1)[(r * TJ + TJ - 1) * T];
-                    R pres = (pc - ps) * inv_dy;
-                    vs[r][k] = diff - conv - pres;
-                }
-            }
-        };
-        const R kx = a.tcoef * a.inv_dx2, ky = a.tcoef * a.inv_dy2;
-        constexpr int RS = wavefront_row_stride(NY);       // columns 0..NY per row pair (0 unused), padded
-        static_assert(NX % 2 == 0 && NX / 2 <= 32, "wavefront layout: one lane per row pair");
-        static_assert(2 * (NX / 2) * RS <= NP, "wavefront planes must fit the exchange planes");
-        auto wavefront = [&]() {
-            const R hk = R(0.5) * dt * inv_dy, dky = dt * ky;
-            if constexpr (std::is_same<R, double>::value) {
-                transport_wavefront_f64<NX, NY, LDU, LDT>((uint32_t)__cvta_generic_to_shared(PA), (uint32_t)__cvta_generic_to_shared(PB),
-                                                          (uint32_t)__cvta_generic_to_shared(UV), (uint32_t)__cvta_generic_to_shared(S), hk, dky, tid);
-            } else {
-                // Lane l owns rows 2l+1, 2l+2 and does column j = t - l + 1 at step t.  The loop is
-                // uniform: inactive steps (j outside 1..NY) compute on harmless in-bounds garbage and
-                // are masked by ONE predicate (stores, partial sums); per step the dependent chain is
-                // SHFL + 2 DFMA, the coefficients of column j+1 are fetched while it waits.
-                constexpr int LANES = NX / 2, STEPS = NY + LANES - 1;
-                const int lane = tid;
-                const bool on = lane < LANES;
-                const int l = on ? lane : 0;
-                const R2 *Vr0 = UV + (2 * l + 1) * LDU, *Vr1 = Vr0 + LDU;
-                R *Sr0 = S + (2 * l + 1) * LDT, *Sr1 = Sr0 + LDT;
-                const R *AAr = PA + (size_t)l * RS * 2, *WWr = PB + (size_t)l * RS * 2;
-                // column 1: partial sums with the south ghost (column 0, untouched by transport)
-                R p0 = fma(fma(hk, Vr0[1].y, dky), Sr0[0], AAr[2]), p1 = fma(fma(hk, Vr1[1].y, dky), Sr1[0], AAr[3]);
-                R w0 = WWr[2], w1 = WWr[3];
-                R last_new = R(0);
-                // pointers biased by -lane: element [t] is column t - lane + 2 (prefetch) / t - lane + 1 (store)
-                // (lanes beyond the last row pair mimic lane 0 with the predicate off)
-                const R *An = AAr + 2 * (2 - l), *Wn = WWr + 2 * (2 - l);
-                const R2 *V0n = Vr0 + (2 - l), *V1n = Vr1 + (2 - l);
-                R *S0o = Sr0 + (1 - l), *S1o = Sr1 + (1 - l);
-                const int c0 = on ? -lane : -(1 << 20);
-    #pragma unroll 2
-                for (int t = 0; t < STEPS; t++) {
-                    const R wv = __shfl_up_sync(0xffffffffu, last_new, 1);
-                    const bool act_ = (unsigned)(c0 + t) < (unsigned)NY;
-                    const R a0n = An[2 * t], a1n = An[2 * t + 1], w0n = Wn[2 * t], w1n = Wn[2 * t + 1];
-                    const R s0n = fma(hk, V0n[t].y, dky), s1n = fma(hk, V1n[t].y, dky);
-                    const R n0 = fma(w0, wv, p0);
-                    const R n1 = fma(w1, n0, p1);
-                    last_new = n1;
-                    if (act_) {
-                        S0o[t] = n0; S1o[t] = n1;
-                        p0 = fma(s0n, n0, a0n); p1 = fma(s1n, n1, a1n);
-                    }
-                    w0 = w0n; w1 = w1n;
-                }
-            }
-        };
-        // The sub-steps are software pipelined across the CTA's warps: the transport of sub-step it-1 is a one-warp
-        // recurrence (the wavefront, ~9 k cycles) and none of what follows it at the start of sub-step it needs the new
-        // T — the velocity ghost cells and the whole predictor up to the buoyancy term.  So while warp 0 runs the
-        // wavefront, the other warps apply the velocity boundary conditions (walls are not re-written: they stay zero
-        // and the wavefront reads them) and compute the predictor of THEIR tiles; after the barrier warp 0 catches up
-        // with the predictor of its tiles while the others set the T ghosts.  Before: 7 of 8 warps idle for 14 % of the
-        // kernel's time.
-        const int warp = tid >> 5;
-        for (int it = 0; it <= a.ndt_act; it++) {
-            // stage X: transport of the previous sub-step (warp 0) || velocity BCs + predictor of this one (the others);
-            // stage Y: warp 0 catches up with the predictor of its tiles, the others set the T ghost cells.
-            // One two-trip loop so that the predictor exists ONCE in the instruction stream.
-            bool last = false;
-#pragma unroll 1
-            for (int stage = 0; stage < 2; stage++) {
-                bool pred;
-                if (stage == 0) {
-                    if (warp == 0) {
-                        if (it > 0) wavefront();
-                        pred = false;
-                    } else {
-                        pred = it < a.ndt_act;
-                        if (pred) {
-                            bc_uv(tid - 32, T - 32, it == 0);
-                            asm volatile("bar.sync 1, %0;" ::"r"(T - 32) : "memory");   // warps 1.. only: their ghost cells are in place
-                        }
-                    }
-                } else {
-                    pred = warp == 0;
-                    if (!pred) bc_s(tid - 32, T - 32);
-                }
-                if (pred && has_tile) predictor();
-                if (stage == 0) {
-                    __syncthreads();               // T is final; velocity ghosts final
-                    PHASE(0);
-                    if (it == a.ndt_act) { last = true; break; }
-                }
-            }
-            if (last) break;
-            if (has_tile) {                        // u* = u + dt rhs_u, v* = v + dt (rhs_v + T), rayleigh.py:393,404
-                TILE_LOOP {                        // (T of the cell itself, no ghost; the pair is one conflict-free 16-byte load)
-                    const R2 c = UV[ou + r * LDU + k];
-                    us[r][k] = (r > 0 || !top) ? c.x + dt * us[r][k] : c.x;
-                    vs[r][k] = (k > 0 || !lef) ? c.y + dt * (vs[r][k] + S[ot + r * LDT + k]) : c.y;
-                }
-            }
-            __syncthreads();                       // every read of the old u, v is done
-            if (has_tile) { TILE_LOOP { R2 w; w.x = us[r][k]; w.y = vs[r][k]; UV[ou + r * LDU + k] = w; } }
-            __syncthreads();                       // U, V now hold the starred fields (walls: 0)
-            PHASE(1);
-
-            // ---- Poisson: rhs and phi in registers, rayleigh.py:412-456 -------------------------------
-            // phi_new = (xp+xm)*k1 + (yp+ym)*k2 + cn with k1 = dy2/(2(dx2+dy2)), k2 = dx2/(2(dx2+dy2)),
-            // cn = -b dx2 dy2/(2(dx2+dy2)): 2 DADD + 2 DFMA per cell.  phi is one register tile updated
-            // in place; sweep s writes exchange plane P[s&1] (P[1] = PB).
-            // The residual reduction is taken off the critical path: while sweep k is computed, the
-            // warp reduction of sweep k-1's residual is interleaved with it (one shuffle stage per
-            // tile column) and the CTA total of sweep k-2 (warp partials published one barrier ago) is
-            // summed; the convergence decision for sweep k-2 is made before sweep k is committed.  A
-            // converged solve drops the two speculative sweeps and re-reads its tile of phi_{k-2}
-            // from the exchange plane that still holds it, so the sweep count and the result are
-            // exactly those of the reference's `while err > tol` loop.
-            // The reduction itself runs in fp32 (5 SHFL + 2 LDS.128 + 7 FADD per sweep instead of 10 SHFL +
-            // 8 LDS.64 + 12 DADD): its only use is the comparison with tol, and an fp32 sum of 256 positive
-            // terms is within ~1e-6 of the fp64 one.  Whenever the fp32 total lies within 1e-4 tol of tol
-            // (a few solves in a thousand) the decision is retaken from the per-thread fp64 residuals of
-            // that sweep, kept in a register, with the fp64 butterfly + pairwise tree: the stop test is
-            // decided by fp64 arithmetic in every case where fp32 could have changed it.
-            R cn[TI][TJ], phi[TI][TJ];
-            R *const pa = PA + opx, *const pb = PB + opx;
-            auto tile_acc = [&](const R (&rs)[TI], const R (&dl)[TI], const R (&dr)[TI]) -> R {
-                // residual over the ghost-inclusive array: ghost copies re-count the wall-adjacent cells
-                R cl = dl[0] * dl[0], cr = dr[0] * dr[0];
-#pragma unroll
-                for (int r = 1; r < TI; r++) { cl = fma(dl[r], dl[r], cl); cr = fma(dr[r], dr[r], cr); }
-                R mid = R(0);
-#pragma unroll
-                for (int r = 1; r < TI - 1; r++) mid += rs[r];
-                R acc = (TI > 1) ? fma(rs[0], w_top, fma(rs[TI - 1], w_bot, mid)) : rs[0] * (w_top + w_bot - R(1));
-                return fma(cl, w_lef, fma(cr, w_rig, acc)) * w_has;
-            };
-            // one sweep (every thread; threads without a tile work on tile 0's addresses and weigh 0)
-            // + the warp reduction of the previous sweep's residual, one stage per column
-            auto sweep = [&](R (&ph)[TI][TJ], const R *pi, float &wsum) -> R {
-                // in place, column by column: the old values of column k-1 are kept in `po_`, column k+1
-                // is still old when column k is computed (one register tile, no copies)
-                R hn[TJ], hs[TJ], hw[TI], he[TI];    // halo: rows i0-1 / i0+TI, columns j0-1 / j0+TJ (wall tiles: their own edge)
-                const R *pn = pi + o_n, *ps = pi + o_s;
-#pragma unroll
-                for (int k = 0; k < TJ; k++) { hn[k] = pn[k]; hs[k] = ps[k]; }
-                // west / east: every lane loads at the same tile-relative offset (conflict free; clamped offsets would put
-                // the lanes of wall tiles one bank off the others: 2-way conflicts in every warp, measured -3.7 %) and
-                // wall tiles take their own edge column from registers instead
-                const bool lefx = tjx == 0, rigx = tjx == TILES_J - 1;
-#pragma unroll
-                for (int r = 0; r < TI; r++) { hw[r] = pi[r * LDP - 1]; he[r] = pi[r * LDP + TJ]; }
-                R rs[TI], dl[TI], dr[TI], po_[TI];
-#pragma unroll
-                for (int r = 0; r < TI; r++) { rs[r] = R(0); po_[r] = lefx ? ph[r][0] : hw[r]; he[r] = rigx ? ph[r][TJ - 1] : he[r]; }
-#pragma unroll
-                for (int k = 0; k < TJ; k++) {
-                    if (k < 5) wsum += __shfl_xor_sync(0xffffffffu, wsum, 16 >> k);
-                    R old[TI], nv[TI];
-#pragma unroll
-                    for (int r = 0; r < TI; r++) old[r] = ph[r][k];
-#pragma unroll
-                    for (int r = 0; r < TI; r++) {
-                        const R xm = (r > 0) ? old[r - 1] : hn[k], xp = (r < TI - 1) ? old[r + 1] : hs[k];
-                        const R ym = po_[r], yp = (k < TJ - 1) ? ph[r][k + 1] : he[r];
-                        nv[r] = fma(xp + xm, a.pk1, fma(yp + ym, a.pk2, cn[r][k]));
-                        const R d = nv[r] - old[r];
-                        rs[r] = fma(d, d, rs[r]);
-                        if (k == 0) dl[r] = d;
-                        if (k == TJ - 1) dr[r] = d;
-                    }
-#pragma unroll
-                    for (int r = 0; r < TI; r++) { po_[r] = old[r]; ph[r][k] = nv[r]; }
-                }
-#pragma unroll
-                for (int st = TJ; st < 5; st++) wsum += __shfl_xor_sync(0xffffffffu, wsum, 16 >> st);
-                return tile_acc(rs, dl, dr);
-            };
-            auto commit = [&](const R (&nw)[TI][TJ], R *po) {
-                if (has_tile) { TILE_LOOP { po[r * LDP + k] = nw[r][k]; } }
-            };
-            auto total32 = [&](const float *part) -> float {   // same pairwise order in every thread -> uniform decision
-                static_assert(NW % 4 == 0, "warp partials are read as float4");
-                float q[NW];
-#pragma unroll
-                for (int w = 0; w < NW; w += 4) {
-                    const float4 v = *reinterpret_cast<const float4 *>(part + w);
-                    q[w] = v.x; q[w + 1] = v.y; q[w + 2] = v.z; q[w + 3] = v.w;
-                }
-#pragma unroll
-                for (int st = 1; st < NW; st *= 2)
-#pragma unroll
-                    for (int w = 0; w + st < NW; w += 2 * st) q[w] += q[w + st];
-                return q[0];
-            };
-            const float tolf = (float)a.tol, tol_band = 1.0e-4f * (float)a.tol;
-            // `while err > tol` for one sweep: fp32 total when it is clearly on one side of tol, else the fp64 total of
-            // the per-thread residuals `mine` of that sweep (butterfly + pairwise tree, the order of the fp64-only code).
-            // The branch is uniform (every thread holds the same fp32 total); a NaN total takes the fp64 path.
-            auto converged = [&](const float err32, const R mine) -> bool {
-                if (fabsf(err32 - tolf) > tol_band) return !(err32 > tolf);
-                return residual_converged_exact<R, NW>(mine, s_exact, a.tol);      // cold, out of line
-            };
-            R accp, accq = R(0);                          // residuals (this thread) of the last committed sweep and of the one before
-            // sweep 1 starts from phi = 0: phi_1 = cn, no halo reads
-            {
-                R rs[TI], dl[TI], dr[TI];
-#pragma unroll
-                for (int r = 0; r < TI; r++) {
-                    rs[r] = R(0);
-#pragma unroll
-                    for (int k = 0; k < TJ; k++) {
-                        R cv = R(0);
-                        if (has_tile) {
-                            const R ue = (r < TI - 1) ? us[r + 1][k] : UV[ou + (r + 1) * LDU + k].x;
-                            const R vn = (k < TJ - 1) ? vs[r][k + 1] : UV[ou + r * LDU + k + 1].y;
-                            cv = -(((ue - us[r][k]) * inv_dx + (vn - vs[r][k]) * inv_dy) * a.cscale) * a.inv_den;
-                        }
-                        cn[r][k] = cv; phi[r][k] = cv;
-                        rs[r] = fma(cv, cv, rs[r]);
-                        if (k == 0) dl[r] = cv;
-                        if (k == TJ - 1) dr[r] = cv;
-                    }
-                }
-                accp = tile_acc(rs, dl, dr);
-                commit(phi, pb);
-                __syncthreads();
-            }
-            // sweep 2 (speculative until sweep 1's residual is known, two barriers from now)
-            {
-                float ws = (float)accp;
-                const R acc = sweep(phi, pb, ws);
-                commit(phi, pa);
-                if ((tid & 31) == 0) s_part[1][tid >> 5] = ws;
-                __syncthreads();
-                accq = accp; accp = acc;
-            }
-            int itp;
-            const R *pf;                                  // plane holding the final iterate (tile-relative)
-            for (int k = 3;; k += 2) {
-                {   // odd k: phi_{k-1} (in PA) -> phi_k; decide on sweep k-2 (still in PB)
-                    float ws = (float)accp;
-                    const R acc = sweep(phi, pa, ws);
-                    const float err = total32(s_part[1]);
-                    if (k - 2 > a.itmax) { status |= BEACON_STATUS_POISSON_OVERFLOW; itp = k - 2; pf = pb; break; }
-                    if (converged(err, accq)) { itp = k - 2; pf = pb; break; }
-                    commit(phi, pb);
-                    if ((tid & 31) == 0) s_part[0][tid >> 5] = ws;
-                    __syncthreads();
-                    accq = accp; accp = acc;
-                }
-                {   // even k+1: phi_k (in PB) -> phi_{k+1}; decide on sweep k-1 (still in PA)
-                    float ws = (float)accp;
-                    const R acc = sweep(phi, pb, ws);
-                    const float err = total32(s_part[0]);
-                    if (k - 1 > a.itmax) { status |= BEACON_STATUS_POISSON_OVERFLOW; itp = k - 1; pf = pa; break; }
-                    if (converged(err, accq)) { itp = k - 1; pf = pa; break; }
-                    commit(phi, pa);
-                    if ((tid & 31) == 0) s_part[1][tid >> 5] = ws;
-                    __syncthreads();
-                    accq = accp; accp = acc;
-                }
-            }
-            TILE_LOOP { phi[r][k] = pf[r * LDP + k]; }     // the converged iterate
-            it_total += itp;
-            PHASE(2);
-
-            // ---- p += phi (rayleigh.py:219; ghost cells: see the end of the launch) and in-place corrector (:461-464)
-            if (has_tile) {
-                R2 *uv = UV + ou;
-                TILE_LOOP {
-                    PSCR(r, k) += phi[r][k];
-                    R2 w = uv[r * LDU + k];
-                    if (r > 0 || !top) { const R pw = (r > 0) ? phi[r - 1][k] : pf[-LDP + k]; w.x = w.x - dt * (phi[r][k] - pw) * inv_dx; }
-                    if (k > 0 || !lef) { const R ps = (k > 0) ? phi[r][k - 1] : pf[r * LDP - 1]; w.y = w.y - dt * (phi[r][k] - ps) * inv_dy; }
-                    uv[r * LDU + k] = w;
-                }
-            }
-            __syncthreads();
-
-            PHASE(3);
-            // ---- transport, rayleigh.py:469-487:  new(i,j) = A + BW*new(i-1,j) + BS*new(i,j-1) ----------
-            // All threads write A and B_W of their cells into the (now free) exchange planes in the
-            // layout the wavefront warp wants: [lane = row pair][column][row in pair], so that one
-            // LDS.128 fetches both rows of a lane and every address is base(lane) + 16*step.  The
-            // west ghost row (i = 0, never updated) is folded into A of row 1 (B_W := 0 there).
-            {
-                if (has_tile) {
-                    const R2 *uv = UV + ou;
-                    const R *sc = S + ot;
-                    R Av[TI][TJ], Wv[TI][TJ];
-                    TILE_LOOP {
-                        const int e = r * LDT + k;
-                        const R2 c = uv[r * LDU + k];
-                        const R uE = uv[(r + 1) * LDU + k].x, uW = c.x, vN = uv[r * LDU + k + 1].y, vS = c.y;
-                        const R s0 = sc[e], sE = sc[e + LDT], sN = sc[e + 1];
-                        R diff0 = ((sE - R(2) * s0) * a.inv_dx2 + (sN - R(2) * s0) * a.inv_dy2) * a.tcoef;
-                        R conv0 = (uE * (R(0.5) * (sE + s0)) - uW * (R(0.5) * s0)) * inv_dx + (vN * (R(0.5) * (sN + s0)) - vS * (R(0.5) * s0)) * inv_dy;
-                        R A = s0 + dt * (diff0 - conv0);
-                        R BW = dt * (kx + R(0.5) * uW * inv_dx);
-                        if (r == 0 && top) { A = fma(BW, sc[e - LDT], A); BW = R(0); }
-                        Av[r][k] = A; Wv[r][k] = BW;
-                    }
-                    // [row pair][column][row in pair]: with two-row tiles the two rows of a column are ONE 16-byte slot
-                    // (conflict free for a quarter-warp: 58 ti + 5 tj mod 8 is a permutation); other tile heights store
-                    // element by element
-                    if constexpr (TI == 2) {
-                        R2 *A2 = reinterpret_cast<R2 *>(PA) + ti * RS + j0, *W2 = reinterpret_cast<R2 *>(PB) + ti * RS + j0;
-#pragma unroll
-                        for (int k = 0; k < TJ; k++) {
-                            R2 x; x.x = Av[0][k]; x.y = Av[1][k]; A2[k] = x;
-                            R2 y; y.x = Wv[0][k]; y.y = Wv[1][k]; W2[k] = y;
-                        }
-                    } else {
-                        TILE_LOOP {
-                            const int gi = TI * ti + r, idx = ((gi >> 1) * RS + j0 + k) * 2 + (gi & 1);
-                            PA[idx] = Av[r][k];
-                            PB[idx] = Wv[r][k];
-                        }
-                    }
-                }
-                __syncthreads();
-                PHASE(4);
-                PHASE(5);
-            }
-        }   // sub-steps
-
-        // ---- observations and reward, rayleigh.py:243-275 ---------------------------------------------
-        {
-            R *hist = a.obs_hist + (size_t)b * a.n_obs;
-            const int per_step = 3 * a.nx_obs_pts * a.ny_obs_pts;
-            R *out = a.obs + orow * a.n_obs;
-            for (int e = tid; e < a.n_obs; e += T) {
-                int st = e / per_step, rem = e - st * per_step;
-                R val;
-                if (st < a.n_obs_steps - 1) val = hist[e + per_step];
-                else {
-                    int f = rem / (a.nx_obs_pts * a.ny_obs_pts), q = rem - f * (a.nx_obs_pts * a.ny_obs_pts);
-                    int pi = q / a.ny_obs_pts, pj = q - pi * a.ny_obs_pts;
-                    int x = a.nx_obs / 2 + pi * a.nx_obs, y = a.ny_obs / 2 + pj * a.ny_obs;
-                    val = (f == 0) ? SS(x, y) : (f == 1 ? UU(x, y) : VV(x, y));
-                }
-                out[e] = val;
-            }
-            __syncthreads();
-            for (int e = tid; e < a.n_obs; e += T) hist[e] = out[e];
-            bool nonfinite = false;
-            for (int e = tid; e < N; e += T) {
-                const int i = e / LD, j = e - i * LD;
-                const R2 w = UV[i * LDU + j];
-                nonfinite |= !finite_(SS(i, j)) | !finite_(w.x) | !finite_(w.y);
-            }
-            if (__syncthreads_or(nonfinite ? 1 : 0)) status |= BEACON_STATUS_NONFINITE;
-            if (tid == 0) {
-                R nu = R(0);
-                for (int i = 1; i <= NX; i++) nu -= (SS(i, 1) - a.Th) / (R(0.5) * a.dy);
-                nu /= R(NX);
-                a.rwd[orow] = -nu;
-                bool horizon = stp == a.n_act - 1;
-                a.done[orow] = horizon; a.trunc[orow] = horizon;
-                if (a.iters) a.iters[orow] = it_total;
-            }
-            stp += 1;
-        }
-    }   // actions
-
-    __syncthreads();
-    for (int e = tid; e < N; e += T) {                 // state planes shared -> global
-        const int i = e / LD, j = e - i * LD;
-        const R2 w = UV[i * LDU + j];
-        gu[e] = w.x; gv[e] = w.y; gs[e] = SS(i, j);
-    }
-    if (has_tile) {                                    // pressure back to its plane; ghost += adjacent(final) - adjacent(launch start)
-        R *pp = gp + o;
-        if (top) {
-#pragma unroll
-            for (int k = 0; k < TJ; k++) pp[-LD + k] += PSCR(0, k) - pp[k];
-        }
-        if (bot) {
-#pragma unroll
-            for (int k = 0; k < TJ; k++) pp[TI * LD + k] += PSCR(TI - 1, k) - pp[(TI - 1) * LD + k];
-        }
-        if (lef) {
-#pragma unroll
-            for (int r = 0; r < TI; r++) pp[r * LD - 1] += PSCR(r, 0) - pp[r * LD];
-        }
-        if (rig) {
-#pragma unroll
-            for (int r = 0; r < TI; r++) pp[r * LD + TJ] += PSCR(r, TJ - 1) - pp[r * LD + TJ - 1];
-        }
-        TILE_LOOP { pp[r * LD + k] = PSCR(r, k); }
-    }
-    if (tid == 0) { a.stp[b] = stp; if (a.status) a.status[b] = status; }
-    if (DBG && dbg) { for (int n = 0; n < (DBG ? 8 : 1); n++) a.dbg[n] += (unsigned long long)tph[n]; }
-#undef PHASE
-#undef TILE_LOOP
-#undef PSCR
-#undef UU
-#undef VV
-#undef SS
-}
+#define MAC_REG_NAME mac_reg_kernel
+#define MAC_REG_PHYS false
+#include "mac_reg_kernel.cuh"
+#undef MAC_REG_NAME
+#undef MAC_REG_PHYS
+#define MAC_REG_NAME mac_reg_phys_kernel
+#define MAC_REG_PHYS true
+#include "mac_reg_kernel.cuh"
+#undef MAC_REG_NAME
+#undef MAC_REG_PHYS
 
 // ---------------------------------------------------------------------------------------
 // Three-plane transport wavefront, shared memory only (any real type):
@@ -1334,8 +770,8 @@ __device__ __noinline__ void transport_wavefront3(uint32_t offA, uint32_t offW, 
 // L2-resident global memory (Poisson is > 90 % of the work: ~65 sweeps per sub-step), transport in
 // row passes through the three-plane wavefront above.  One CTA per SM.
 // ---------------------------------------------------------------------------------------
-template <typename R, int NX, int NY, int TI, int TJ, int T, int MINB, bool DBG>
-__global__ void __launch_bounds__(T, MINB) mac_big_kernel(const MacArgs<R> a)
+template <typename R, int NX, int NY, int TI, int TJ, int T, int MINB, bool DBG, bool PHYS>
+__device__ __forceinline__ void mac_big_body(const MacArgs<R> &a, const unsigned thread_x)
 {
     constexpr int LD = NY + 2, N = (NX + 2) * LD;
     constexpr int LDP = ((LD + 6) / 8) * 8 + 1;         // exchange planes: stride = 1 mod 8
@@ -1354,7 +790,7 @@ __global__ void __launch_bounds__(T, MINB) mac_big_kernel(const MacArgs<R> a)
     __shared__ R s_red[NW];
     __shared__ R s_seg[128];
     __shared__ R s_act[128];
-    const int tid = threadIdx.x, b = blockIdx.x;
+    const int tid = thread_x, b = blockIdx.x;
     const bool resetting = a.mode == 1;
     if (resetting && a.mask && !a.mask[b]) return;
     const bool ray = a.kind == BEACON_RAYLEIGH;
@@ -1415,6 +851,7 @@ __global__ void __launch_bounds__(T, MINB) mac_big_kernel(const MacArgs<R> a)
     }
     int stp = a.stp[b];
     int status = 0;
+    MAC_LOAD_COEF(b);                                  // read after the barrier that opens each action
     const R dt = a.dt, inv_dx = a.inv_dx, inv_dy = a.inv_dy;
     // The uniform transport wavefront reads a few never-written padding slots of the planes during its
     // masked steps; their values cannot reach a result as long as they are finite (they are multiplied
@@ -1446,10 +883,10 @@ __global__ void __launch_bounds__(T, MINB) mac_big_kernel(const MacArgs<R> a)
         } else if (tid == 0) {                                     // get_control, mixing.py:212-234
             int ai = ((const int32_t *)a.actions)[orow];
             R ut = 0, ub = 0, vl = 0, vr = 0;
-            if (ai == 0) { ub = a.u_max; ut = -a.u_max; }
-            if (ai == 1) { ub = -a.u_max; ut = a.u_max; }
-            if (ai == 2) { vr = a.u_max; vl = -a.u_max; }
-            if (ai == 3) { vr = -a.u_max; vl = a.u_max; }
+            if (ai == 0) { ub = MAC_UMAX; ut = -MAC_UMAX; }
+            if (ai == 1) { ub = -MAC_UMAX; ut = MAC_UMAX; }
+            if (ai == 2) { vr = MAC_UMAX; vl = -MAC_UMAX; }
+            if (ai == 3) { vr = -MAC_UMAX; vl = MAC_UMAX; }
             s_seg[0] = ut; s_seg[1] = ub; s_seg[2] = vl; s_seg[3] = vr;
             a.a_int[b] = ai;
         }
@@ -1529,7 +966,7 @@ __global__ void __launch_bounds__(T, MINB) mac_big_kernel(const MacArgs<R> a)
                         R uN = R(0.5) * (uu[e + 1] + uc), uS = R(0.5) * (uc + uu[e - 1]);
                         R vN = R(0.5) * (vv[e + 1] + vv[e - LD + 1]), vS = R(0.5) * (vc + vv[e - LD]);
                         R conv = (uE * uE - uW * uW) * inv_dx + (uN * vN - uS * vS) * inv_dy;
-                        R diff = ((uu[e + LD] - R(2) * uc + uu[e - LD]) * a.inv_dx2 + (uu[e + 1] - R(2) * uc + uu[e - 1]) * a.inv_dy2) * a.dcoef;
+                        R diff = ((uu[e + LD] - R(2) * uc + uu[e - LD]) * a.inv_dx2 + (uu[e + 1] - R(2) * uc + uu[e - 1]) * a.inv_dy2) * MAC_DCOEF;
                         R pres = (pc - ((r > 0) ? pt[r - 1][k] : pwh[k])) * inv_dx;
                         usr[r][k] = uc + dt * (diff - conv - pres);
                     }
@@ -1538,7 +975,7 @@ __global__ void __launch_bounds__(T, MINB) mac_big_kernel(const MacArgs<R> a)
                         R uE = R(0.5) * (uu[e + LD] + uu[e + LD - 1]), uW = R(0.5) * (uc + uu[e - 1]);
                         R vN = R(0.5) * (vv[e + 1] + vc), vS = R(0.5) * (vc + vv[e - 1]);
                         R conv = (uE * vE - uW * vW) * inv_dx + (vN * vN - vS * vS) * inv_dy;
-                        R diff = ((vv[e + LD] - R(2) * vc + vv[e - LD]) * a.inv_dx2 + (vv[e + 1] - R(2) * vc + vv[e - 1]) * a.inv_dy2) * a.dcoef;
+                        R diff = ((vv[e + LD] - R(2) * vc + vv[e - LD]) * a.inv_dx2 + (vv[e + 1] - R(2) * vc + vv[e - 1]) * a.inv_dy2) * MAC_DCOEF;
                         R pres = (pc - ((k > 0) ? pt[r][k - 1] : psh[r])) * inv_dy;
                         R rhs = diff - conv - pres;
                         if (ray) rhs += sc[e];
@@ -1753,7 +1190,7 @@ __global__ void __launch_bounds__(T, MINB) mac_big_kernel(const MacArgs<R> a)
 
             // ---- transport: rayleigh.py:469-487 / mixing.py:478-495, in PASSES row blocks -------------
             {
-                const R kx = a.tcoef * a.inv_dx2, ky = a.tcoef * a.inv_dy2;
+                const R kx = MAC_TCOEF * a.inv_dx2, ky = MAC_TCOEF * a.inv_dy2;
                 constexpr uint32_t PLANE_B = (uint32_t)((LANES_MAX * RS + 8) * 2 * sizeof(R));
                 R *AA = PA, *WW = reinterpret_cast<R *>(smem_raw + PLANE_B), *SS = reinterpret_cast<R *>(smem_raw + 2 * PLANE_B);
                 for (int ps = 0; ps < PASSES; ps++) {
@@ -1782,7 +1219,7 @@ __global__ void __launch_bounds__(T, MINB) mac_big_kernel(const MacArgs<R> a)
                                 for (int h = 0; h < 2; h++) {
                                     const R uE = h ? u2 : u1, uW = h ? u1 : u0, vN = h ? v11 : v01, vS = h ? v10 : v00;
                                     const R s0 = h ? s10 : s00, sE = h ? s20 : s10, sN = h ? s11 : s01;
-                                    R diff0 = ((sE - R(2) * s0) * a.inv_dx2 + (sN - R(2) * s0) * a.inv_dy2) * a.tcoef;
+                                    R diff0 = ((sE - R(2) * s0) * a.inv_dx2 + (sN - R(2) * s0) * a.inv_dy2) * MAC_TCOEF;
                                     R conv0 = (uE * (R(0.5) * (sE + s0)) - uW * (R(0.5) * s0)) * inv_dx + (vN * (R(0.5) * (sN + s0)) - vS * (R(0.5) * s0)) * inv_dy;
                                     R A = s0 + dt * (diff0 - conv0);
                                     R BW = dt * (kx + R(0.5) * uW * inv_dx);
@@ -1890,6 +1327,11 @@ __global__ void __launch_bounds__(T, MINB) mac_big_kernel(const MacArgs<R> a)
 #undef SC
 #undef TILE_LOOP
 }
+template <typename R, int NX, int NY, int TI, int TJ, int T, int MINB, bool DBG>
+__global__ void __launch_bounds__(T, MINB) mac_big_kernel(const MacArgs<R> a) { mac_big_body<R, NX, NY, TI, TJ, T, MINB, DBG, false>(a, threadIdx.x); }
+// per-env physical constants (MacArgs::phys); a name that tools/sass_census.py's patterns for mac_big_kernel do not match
+template <typename R, int NX, int NY, int TI, int TJ, int T, int MINB>
+__global__ void __launch_bounds__(T, MINB) mac_big_phys_kernel(const MacArgs<R> a) { mac_big_body<R, NX, NY, TI, TJ, T, MINB, false, true>(a, threadIdx.x); }
 
 // ---------------------------------------------------------------------------------------
 // Capacity of mac_kernel with G > 1 CTAs per env: "" when (nx, ny) fits, else the reason.
@@ -1916,12 +1358,33 @@ template <typename R> static int cluster_passes(int Smax, int ld)
     return ps;
 }
 
+// Per-env physical constants: row b of `tab` from the raw per-env values of `raw` ([2][B] float64: rayleigh ra;
+// mixing re, pe), with the host's expressions of MacEnv's constructor, in double, then cast to R: a row holds
+// bitwise the constants of a uniform handle created with that env's values (IEEE division and square root on
+// both sides, no fast-math).  Runs when the values change, never on the step path.
+template <typename R>
+__global__ void mac_phys_derive(const double *raw, R *tab, int B, int ray, double pr, double L, double u_max)
+{
+    const int b = blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= B) return;
+    if (ray) {
+        const double ra = raw[b];
+        tab[3 * b] = (R)std::sqrt(pr / ra); tab[3 * b + 1] = (R)(1.0 / std::sqrt(pr * ra)); tab[3 * b + 2] = (R)u_max;
+    } else {
+        const double re = raw[b], pe = raw[B + b];
+        tab[3 * b] = (R)(1.0 / re); tab[3 * b + 1] = (R)(1.0 / pe); tab[3 * b + 2] = (R)(re * 0.01 / L);   // u_max = re nu / L, params.py
+    }
+}
+
 template <typename R> class MacEnv : public Env {
     beacon_mac_params p;
     int kind, G = 1;
     DeviceBuffer u, v, pp, s, us, vs, cc, a_cur, a_int, obs_hist, stp, u0, v0, p0, s0, dbgbuf;
+    DeviceBuffer phys_raw, phys_tab;   // per-env physical parameters, allocated by the first set_physics
     MacArgs<R> base{};
     void (*kernel)(const MacArgs<R>) = nullptr;
+    void (*phys_kernel)(const MacArgs<R>) = nullptr;   // the per-env instance of `kernel`
+    double mix_L = 0;                                   // mixing: L = nx dx, for u_max = re nu / L
     int T = 0;
     size_t smem = 0;
     bool reg_variant = false, dbg_variant = false, big_variant = false;
@@ -1966,16 +1429,19 @@ public:
             // five planes fit twice per SM: register-resident phi tiles, 2 CTAs/SM
             if (getenv("BEACON_MAC_DEBUG")) kernel = mac_reg_kernel<R, 50, 50, 2, 5, 256, true>;
             else kernel = mac_reg_kernel<R, 50, 50, 2, 5, 256, false>;
+            phys_kernel = mac_reg_phys_kernel<R, 50, 50, 2, 5, 256, false>;
             T = 256; TI = 2; TJ = 5; dbg_variant = true;
             smem = sizeof(R) * (2 * (size_t)((51 * mac_ldp(52, 2) + 3) / 4 * 4) + 2 * 52 * 53 + 52 * mac_ldp(52, 2)); reg_variant = true;
         } else if (nx == 100 && ny == 100 && !getenv("BEACON_MAC_V1")) {
             // register-resident Poisson, fields in L2: one CTA of 500 tile threads per SM
             if (getenv("BEACON_MAC_DEBUG")) kernel = mac_big_kernel<R, 100, 100, 4, 5, 512, 1, true>;
             else kernel = mac_big_kernel<R, 100, 100, 4, 5, 512, 1, false>;
+            phys_kernel = mac_big_phys_kernel<R, 100, 100, 4, 5, 512, 1>;
             T = 512; TI = 4; TJ = 5; dbg_variant = true; big_variant = true;
             smem = sizeof(R) * 2 * (size_t)((102 * 105 + 3) / 4 * 4);
         } else if (2 * plane + 1024 <= 220 * 1024 && ((nx + 3) / 4) * ((ny + 4) / 5) <= 512) {
             kernel = mac_kernel<R, 4, 5, 512, false>; T = 512; TI = 4; TJ = 5; smem = 2 * plane;
+            phys_kernel = mac_phys_kernel<R, 4, 5, 512, false>;
         } else {
             std::string msg = "mac2d: grid too large for the one-CTA-per-env kernel (max ~100x100 cells)";
             for (int g = 2; g <= MAC_CLUSTER_MAX; g++)
@@ -1994,6 +1460,7 @@ public:
             a.tr_pass = cluster_passes<R>(Smax, ld);
             const int rows = (Smax + a.tr_pass - 1) / a.tr_pass;
             kernel = mac_kernel<R, 4, 5, 512, true>; T = 512; TI = 4; TJ = 5;
+            phys_kernel = mac_phys_kernel<R, 4, 5, 512, true>;
             smem = sizeof(R) * (size_t)ld * std::max(2 * a.slab_rows, 3 * rows) + MAC_HANDOFF_BYTES(R);
         }
         raise_dynamic_smem_limit(kernel, smem);
@@ -2040,12 +1507,74 @@ public:
         a.u = u.as<R>(); a.v = v.as<R>(); a.p = pp.as<R>(); a.s = s.as<R>(); a.us = us.as<R>(); a.vs = vs.as<R>(); a.cc = cc.as<R>();
         a.a_cur = a_cur.as<R>(); a.a_int = a_int.as<int32_t>(); a.obs_hist = obs_hist.as<R>(); a.stp = stp.as<int32_t>();
         a.u0 = u0.as<R>(); a.v0 = v0.as<R>(); a.p0 = p0.as<R>(); a.s0 = s0.as<R>();
+        mix_L = (double)nx * dx;
     }
+
+    // ---- per-env physical parameters ------------------------------------------------------------
+    // slot of `name` in phys_raw: rayleigh "ra"; mixing "re", "pe"
+    int phys_slot(const char *name) const
+    {
+        const bool ray = kind == BEACON_RAYLEIGH;
+        const std::string nm = name ? name : "";
+        if (ray && nm == "ra") return 0;
+        if (!ray && nm == "re") return 0;
+        if (!ray && nm == "pe") return 1;
+        throw Error(BEACON_ERR_INVALID, std::string(ray ? "rayleigh" : "mixing") + " has no per-env physical parameter '" + nm +
+                                            "' (it has " + (ray ? "\"ra\")" : "\"re\", \"pe\")"));
+    }
+    double phys_uniform(int slot) const { return kind == BEACON_RAYLEIGH ? p.ra : (slot == 0 ? p.re : p.pe); }
+    void set_physics(const char *name, const double *values, cudaStream_t st) override
+    {
+        const int slot = phys_slot(name), B = info.batch;
+        BEACON_REQUIRE(values != nullptr, "set_physics: values must not be NULL");
+        std::vector<double> h(values, values + B);   // pageable: the copy below has read it when it returns
+        for (int b = 0; b < B; b++)
+            if (!std::isfinite(h[b]) || !(h[b] > 0))
+                throw Error(BEACON_ERR_INVALID, std::string("set_physics: ") + name + "[" + std::to_string(b) + "] = " + std::to_string(h[b]) +
+                                                    ": values must be finite and > 0");
+        if (kind == BEACON_MIXING && slot == 0 && p.re * 0.01 / mix_L != p.u_max)
+            throw Error(BEACON_ERR_UNSUPPORTED, "set_physics: per-env re sets u_max = re * 0.01 / L with L = nx dx; this handle's u_max "
+                                                "does not follow that rule");
+        if (!base.phys) {
+            // first call: the per-env instance takes over every launch of the handle
+            raise_dynamic_smem_limit(phys_kernel, smem);
+            if (G > 1) {
+                cudaLaunchConfig_t cfg = {};
+                cudaLaunchAttribute at[1];
+                cfg.gridDim = dim3(B * G); cfg.blockDim = dim3(T); cfg.dynamicSmemBytes = smem;
+                at[0].id = cudaLaunchAttributeClusterDimension; at[0].val.clusterDim.x = G; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
+                cfg.attrs = at; cfg.numAttrs = 1;
+                int clusters = 0;
+                BEACON_CUDA_CHECK(cudaOccupancyMaxActiveClusters(&clusters, phys_kernel, &cfg));
+                if (clusters < 1) throw Error(BEACON_ERR_UNSUPPORTED, "mac2d: the per-env instance does not fit a cluster of " + std::to_string(G) + " CTAs");
+            }
+            std::vector<double> init(2 * (size_t)B);
+            for (int b = 0; b < B; b++) { init[b] = phys_uniform(0); init[B + b] = phys_uniform(1); }
+            phys_raw.alloc(init.size() * sizeof(double));
+            phys_tab.alloc(3 * (size_t)B * sizeof(R));
+            BEACON_CUDA_CHECK(cudaMemcpy(phys_raw.ptr, init.data(), init.size() * sizeof(double), cudaMemcpyHostToDevice));
+            base.phys = phys_tab.as<R>();
+        }
+        BEACON_CUDA_CHECK(cudaMemcpyAsync(phys_raw.as<double>() + (size_t)slot * B, h.data(), (size_t)B * sizeof(double), cudaMemcpyHostToDevice, st));
+        mac_phys_derive<R><<<(B + 127) / 128, 128, 0, st>>>(phys_raw.as<double>(), phys_tab.as<R>(), B, kind == BEACON_RAYLEIGH, p.pr, mix_L, p.u_max);
+        BEACON_CUDA_CHECK(cudaGetLastError());
+        launches++;
+    }
+    void get_physics(const char *name, double *values, cudaStream_t st) override
+    {
+        const int slot = phys_slot(name), B = info.batch;
+        BEACON_REQUIRE(values != nullptr, "get_physics: values must not be NULL");
+        if (!base.phys) { std::fill(values, values + B, phys_uniform(slot)); return; }
+        BEACON_CUDA_CHECK(cudaMemcpyAsync(values, phys_raw.as<double>() + (size_t)slot * B, (size_t)B * sizeof(double), cudaMemcpyDeviceToHost, st));
+        BEACON_CUDA_CHECK(cudaStreamSynchronize(st));
+    }
+
     void run(const MacArgs<R> &a_, cudaStream_t st)
     {
         MacArgs<R> a = a_;
+        auto kernel = a.phys ? phys_kernel : this->kernel;
         static const bool debug = getenv("BEACON_MAC_DEBUG") != nullptr;
-        if (debug && dbg_variant && a.mode == 0) {                       // tuning aid: cycles per phase of env 0
+        if (debug && dbg_variant && !a.phys && a.mode == 0) {            // tuning aid: cycles per phase of env 0
             if (!dbgbuf.ptr) dbgbuf.alloc(8 * sizeof(unsigned long long));
             BEACON_CUDA_CHECK(cudaMemsetAsync(dbgbuf.ptr, 0, 64, st));
             a.dbg = dbgbuf.as<unsigned long long>();
@@ -2061,7 +1590,7 @@ public:
             kernel<<<a.B, T, smem, st>>>(a);
         BEACON_CUDA_CHECK(cudaGetLastError());
         launches++;
-        if (debug && dbg_variant && a.mode == 0) {
+        if (debug && dbg_variant && !a.phys && a.mode == 0) {
             unsigned long long h[8];
             BEACON_CUDA_CHECK(cudaMemcpyAsync(h, dbgbuf.ptr, 64, cudaMemcpyDeviceToHost, st));
             BEACON_CUDA_CHECK(cudaStreamSynchronize(st));

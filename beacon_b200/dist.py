@@ -7,6 +7,7 @@ the CPU tests).
 The noise an env sees depends on (seed, GLOBAL env index) only, so results do not depend on the
 number of shards (tests/test_gpu_parity.py::test_shkadov_philox_noise_sharding_invariance).
 """
+import numpy as np
 import torch
 import torch.distributed as dist
 
@@ -30,6 +31,13 @@ def make_sharded(name, num_envs, rank=None, world=None, **kwargs):
     rank = dist.get_rank() if rank is None else rank
     world = dist.get_world_size() if world is None else world
     lo, hi = shard_range(num_envs, rank, world)
+    from ._capi import PHYSICS
+    for k in PHYSICS.get(name, ()):          # per-env physical parameters: this rank's slice
+        v = kwargs.get(k)
+        if v is not None and np.ndim(v.detach().cpu() if isinstance(v, torch.Tensor) else v) == 1:
+            if len(v) != num_envs:
+                raise ValueError(f"{k}: expected {num_envs} per-env values, got {len(v)}")
+            kwargs[k] = v[lo:hi]
     dev = kwargs.pop("device", torch.cuda.current_device())
     return BatchedEnv(name, batch=hi - lo, device=dev, env_index_base=lo, **kwargs)
 

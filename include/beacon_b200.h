@@ -222,6 +222,19 @@ BEACON_API int beacon_env_field(const beacon_env *env, int32_t index, const char
 BEACON_API int beacon_env_get_state(beacon_env *env, const char *field, void *buf, beacon_stream_t stream);
 BEACON_API int beacon_env_set_state(beacon_env *env, const char *field, const void *buf, beacon_stream_t stream);
 
+/* ---- per-env physical parameters (rayleigh, mixing) -------------------------------------
+ * Each env of a batch may run at its own Rayleigh (rayleigh "ra"), Reynolds and Péclet number (mixing
+ * "re", "pe"); a handle is created with one value for all of them.  values: HOST float64 [batch], each
+ * finite and > 0.  A set is stream-ordered with the launches: it takes effect at the next reset or step
+ * on `stream`.  From the first set on, the handle's launches use the per-env kernel instances (a
+ * handle that is never set runs exactly as before).  mixing "re" also sets the lid / wall speed
+ * u_max = re * 0.01 / L (L = nx dx), as the constructor does.  An unknown name, a name of the other
+ * environment, any other environment or a bad value return BEACON_ERR_INVALID and change nothing.
+ * get_physics returns the current values (the handle's scalar for every env before the first set)
+ * after the stream has drained. */
+BEACON_API int beacon_env_set_physics(beacon_env *env, const char *name, const double *values, beacon_stream_t stream);
+BEACON_API int beacon_env_get_physics(beacon_env *env, const char *name, double *values, beacon_stream_t stream);
+
 /* ---- learner-rank buffers in peer memory (multi-GPU, one process per GPU) -------------
  * The only exchange of the path is the gather of observations / rewards / flags to the learner
  * rank (SURVEY.md §8e; reference call sites whose outputs travel: get_obs / get_rwd,
