@@ -16,7 +16,7 @@ CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "lib")
 LIB = os.path.join(LIBDIR, "libbeacon_b200.so")
 SOURCES = ["capi.cu", "shkadov.cu", "burgers.cu", "sloshing.cu", "ode.cu", "mac2d.cu"]
-HEADERS = [os.path.join(CSRC, "common.cuh"), os.path.join(CSRC, "mac_reg_kernel.cuh"), os.path.join(HERE, "..", "include", "beacon_b200.h")]
+HEADERS = [os.path.join(CSRC, "common.cuh"), os.path.join(HERE, "..", "include", "beacon_b200.h")]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
