@@ -234,9 +234,8 @@ class BatchedEnv:
         self.last_iters = iters
         if self.rwd_dim == 1:
             rwd = rwd[..., 0]
-        if out is not None:
-            return obs, rwd, done.view(torch.bool), trunc.view(torch.bool)
-        return obs, rwd, done.bool(), trunc.bool()
+        # the kernels write 0 / 1 flags: a bool view costs no conversion kernels on the stream
+        return obs, rwd, done.view(torch.bool), trunc.view(torch.bool)
 
     def step_into(self, actions, obs_ptr, rwd_ptr, done_ptr, trunc_ptr, noise=None):
         """One gym step whose observation / reward / flag rows are written to RAW device addresses

@@ -74,18 +74,6 @@ __device__ __forceinline__ double fdiv(double a, double b)
     const double q0 = a * y;
     return fma(q0, fma(e, e, e), q0);
 }
-// 0.5 a / b with the halving done on the exponent of the reciprocal seed by the integer pipe (the
-// seed is 1/b to 20 bits: never zero or denormal for the finite divisors of these paths).
-__device__ __forceinline__ double fdiv_half(double a, double b)
-{
-    double y;
-    asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(y) : "d"(b));
-    const double e = fma(-b, y, 1.0);
-    const double hy = __hiloint2double(__double2hiint(y) - 0x00100000, 0);
-    const double q0 = a * hy;
-    return fma(q0, fma(e, e, e), q0);
-}
-__device__ __forceinline__ float fdiv_half(float a, float b) { return 0.5f * (a / b); }
 // clamp(r, 0, 1) = max(0, min(r, 1)) decided on the high word with integer compares (the fp64
 // pipe is the bottleneck of these kernels): sign bit -> 0, exponent >= 0 -> 1, else r.
 // -0.0 -> 0.  A NaN ratio gives 0 or 1 instead of NaN (numpy's maximum/minimum would propagate

@@ -85,7 +85,11 @@ __global__ void __launch_bounds__(T, MINB) shkadov_kernel(const ShkArgs<R> a)
     // ---- static per-thread geometry ---------------------------------------------------
     const int a0 = tid * C - a.off;                     // first point of my chunk
     const bool has_jet = (a0 + C - 1 >= a.jz0) && (a0 < a.jz0 + a.jz_len) && nj > 0;
-    const int tl = tid > 0 ? tid - 1 : 0, tr = tid < T - 1 ? tid + 1 : T - 1;
+    // Thread 0 has no left neighbour: its left ghost reads are shifted back by two slot rows onto its own slots, so
+    // that the ghost left of its first point reads that point's own q and q2h (XQL1 -> XQ0, XZL1 -> XZ0), the other
+    // four land on its own values too.  F_SMALL relies on this for the inlet face (see the TVD faces below).
+    static_assert(XQ0 - XQL1 == XZ0 - XZL1 && XHL2 + XQ0 - XQL1 >= 0, "exchange slot order");
+    const int tl = tid > 0 ? tid - 1 : (XQ0 - XQL1) * T, tr = tid < T - 1 ? tid + 1 : T - 1;
     const bool interior_thread = a0 >= 2 && a0 + C - 1 <= nx - 4;   // full stencil, all points updated
     // Warp roles (warp-uniform: no warp executes two variants of the update and stalls the others at
     // the barrier; and as few distinct loop bodies as possible, each compact: the bodies of all
@@ -95,8 +99,9 @@ __global__ void __launch_bounds__(T, MINB) shkadov_kernel(const ShkArgs<R> a)
     //            the two one-sided closures of d3o2u and the not-updated point sit at compile-time
     //            positions and are selected by `is_last`.  Thread 0 holds `off` phantom points, the
     //            inlet point 0 and the faces with phi = 0: selects on per-thread thresholds (zero for
-    //            everybody else), confined to m < 3 when off <= 1 (F_SMALL), or for all m in warp 0
-    //            (F_LARGE) while the other warps run the body without them (F_NONE).  Lanes beyond
+    //            everybody else), confined to the points m < 2 when off <= 1 (F_SMALL, whose faces
+    //            need none), or for all m in warp 0 (F_LARGE) while the other warps run the body
+    //            without them (F_NONE).  Lanes beyond
     //            the domain run the same arithmetic on phantom points (never stored, never read by
     //            a result that is kept);
     //   IDLE     warps entirely beyond the domain only keep the barrier count;
@@ -256,11 +261,20 @@ __global__ void __launch_bounds__(T, MINB) shkadov_kernel(const ShkArgs<R> a)
                     for (int k = 0; k < C + 2; k++) { dq[k] = uq[k + 1] - uq[k]; dz[k] = uz[k + 1] - uz[k]; }
 #pragma unroll
                     for (int m = 0; m < C + 1; m++) {
-                        // half of the minmod limiter, 0.5 max(0, min(r, 1))
-                        R pq = clamp0h(fdiv_half(dq[m], dq[m + 1] + R(1.0e-8)));
-                        R pz = clamp0h(fdiv_half(dz[m], dz[m + 1] + R(1.0e-8)));
+                        // half of the minmod limiter, 0.5 max(0, min(r, 1)) with r = d_m / (d_{m+1} + 1e-8), as
+                        // d_m / (2 d_{m+1} + 2e-8): doubling the divisor is exact and costs nothing (an FMA in place of
+                        // the DADD), and the reciprocal seed of 2b is the seed of b with its exponent lowered by one, so
+                        // the quotient is 0.5 r bit for bit (tools/micro/rcpacc.cu checks the seeds)
+                        R pq = clamp0h(fdiv(dq[m], fma(R(2), dq[m + 1], R(2.0e-8))));
+                        R pz = clamp0h(fdiv(dz[m], fma(R(2), dz[m + 1], R(2.0e-8))));
                         if (UK == ROLE_GENERAL) { if (a0 - 1 + m <= 0) { pq = R(0); pz = R(0); } }   // phi[0] = 0
-                        if (UK == F_LARGE || (UK == F_SMALL && m < 3)) { if (m < zf) { pq = R(0); pz = R(0); } }
+                        // F_SMALL needs no select for phi[0] = 0.  The inlet face is face zf-1 of thread 0, and both of
+                        // its differences are exactly 0 there: with off = 0 the ghost left of the inlet point is that
+                        // point (tl), with off = 1 the phantom point carries the inlet values.  A zero numerator gives
+                        // pq = pz = +0 unless the divisor is exactly 0; for q that cannot happen (q_0 = 1), for q2h it
+                        // needs |q2h_0| < 2^-24, an inlet depth above 1.6e7.  The faces left of it feed only points
+                        // that are not updated.
+                        if (UK == F_LARGE) { if (m < zf) { pq = R(0); pz = R(0); } }
                         Fq[m] = uq[m + 1] + pq * dq[m + 1];
                         Fz[m] = uz[m + 1] + pz * dz[m + 1];
                     }
