@@ -59,10 +59,17 @@ template <typename R> struct ShkArgs {
 // shared-memory exchange slots per thread
 enum { XH0 = 0, XH1, XH2, XHL2, XHL1, XQ0, XQL2, XQL1, XZ0, XZL2, XZL1, XN };
 
-template <typename R, int C, int T, int MINB>
-__global__ void __launch_bounds__(T, MINB) shkadov_kernel(const ShkArgs<R> a)
+// Chunk widths: threads [0, TH) hold C points each, threads [TH, T) hold CN.  CN == C is the uniform
+// layout (TH = T).  CN == C - 1 is the balanced layout (TH = T / 2): warps w and w + T/64 of a CTA run on
+// the same SM sub-partition, so every sub-partition then carries one C-point and one CN-point warp
+// instead of two C-point warps, and fewer phantom points fill the last warp (DESIGN.md §3.1).
+template <typename R, int C, int CN, int T>
+__device__ __forceinline__ void shkadov_body(const ShkArgs<R> &a)
 {
-    static_assert(C >= 3, "halo exchange needs at least 3 points per thread");
+    static_assert(CN >= 3, "halo exchange needs at least 3 points per thread");
+    static_assert(CN == C || (CN == C - 1 && T % 64 == 0), "balanced layout: CN = C - 1, warp-aligned halves");
+    constexpr bool BAL = CN != C;
+    constexpr int TH = BAL ? T / 2 : T;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int tid = threadIdx.x, b = a.order ? a.order[blockIdx.x] : (int)blockIdx.x;
     const int nx = a.nx, nj = a.n_jets;
@@ -83,14 +90,17 @@ __global__ void __launch_bounds__(T, MINB) shkadov_kernel(const ShkArgs<R> a)
     short *s_jj = reinterpret_cast<short *>(s_jw + a.jz_len + 2 * C);   // [jz_len] jet index or -1
 
     // ---- static per-thread geometry ---------------------------------------------------
-    const int a0 = tid * C - a.off;                     // first point of my chunk
-    const bool has_jet = (a0 + C - 1 >= a.jz0) && (a0 < a.jz0 + a.jz_len) && nj > 0;
+    const bool narrow = BAL && tid >= TH;               // warp-uniform
+    const int cw = narrow ? CN : C;                     // points of my chunk
+    auto first_point = [&](int t) { return (BAL && t >= TH ? TH * C + (t - TH) * CN : t * C) - a.off; };
+    const int a0 = first_point(tid);                    // first point of my chunk
+    const bool has_jet = (a0 + cw - 1 >= a.jz0) && (a0 < a.jz0 + a.jz_len) && nj > 0;
     // Thread 0 has no left neighbour: its left ghost reads are shifted back by two slot rows onto its own slots, so
     // that the ghost left of its first point reads that point's own q and q2h (XQL1 -> XQ0, XZL1 -> XZ0), the other
     // four land on its own values too.  F_SMALL relies on this for the inlet face (see the TVD faces below).
     static_assert(XQ0 - XQL1 == XZ0 - XZL1 && XHL2 + XQ0 - XQL1 >= 0, "exchange slot order");
     const int tl = tid > 0 ? tid - 1 : (XQ0 - XQL1) * T, tr = tid < T - 1 ? tid + 1 : T - 1;
-    const bool interior_thread = a0 >= 2 && a0 + C - 1 <= nx - 4;   // full stencil, all points updated
+    const bool interior_thread = a0 >= 2 && a0 + cw - 1 <= nx - 4;  // full stencil, all points updated
     // Warp roles (warp-uniform: no warp executes two variants of the update and stalls the others at
     // the barrier; and as few distinct loop bodies as possible, each compact: the bodies of all
     // resident warps must stay in the instruction cache — three 40 KB bodies measured 0.7x):
@@ -99,21 +109,25 @@ __global__ void __launch_bounds__(T, MINB) shkadov_kernel(const ShkArgs<R> a)
     //            the two one-sided closures of d3o2u and the not-updated point sit at compile-time
     //            positions and are selected by `is_last`.  Thread 0 holds `off` phantom points, the
     //            inlet point 0 and the faces with phi = 0: selects on per-thread thresholds (zero for
-    //            everybody else), confined to the points m < 2 when off <= 1 (F_SMALL, whose faces
-    //            need none), or for all m in warp 0 (F_LARGE) while the other warps run the body
-    //            without them (F_NONE).  Lanes beyond
+    //            everybody else), confined to the points m <= SMALL_OFF when off <= SMALL_OFF (F_SMALL,
+    //            whose faces need none), or for all m in warp 0 (F_LARGE) while the other warps run the
+    //            body without them (F_NONE).  The balanced layout has off <= CN - 1 = SMALL_OFF always:
+    //            both of its widths run F_SMALL, unrolled (its inlet lies in the C half, the outlet in
+    //            the CN half, so each width carries only its own specials).  Lanes beyond
     //            the domain run the same arithmetic on phantom points (never stored, never read by
     //            a result that is kept);
     //   IDLE     warps entirely beyond the domain only keep the barrier count;
     //   GENERAL  anything else (tiny lattices, overlapping / dense jets): per-point index tests.
     enum { F_NONE = 0, F_SMALL, F_LARGE, ROLE_GENERAL, ROLE_IDLE };
-    const int w_lo = (tid & ~31) * C - a.off, w_hi = w_lo + 32 * C - 1;
-    const int last_tid = (nx - 1 + a.off) / C;
+    constexpr int SMALL_OFF = BAL ? CN - 1 : 1;
+    const int w_lo = first_point(tid & ~31);
+    const int lp = nx - 1 + a.off;                      // outlet point counted from the first phantom point
+    const int last_tid = BAL && lp >= TH * C ? TH + (lp - TH * C) / CN : lp / C;
     int role = ROLE_GENERAL;
     if (w_lo >= nx) role = ROLE_IDLE;
     else if (a.tail_aligned && a.jets_simple && nx - 4 >= C) {
         // (warp 0 must not hold the outlet specials too: first thread's chunk ends before nx-3)
-        if (a.off <= 1) role = F_SMALL;
+        if (a.off <= SMALL_OFF) role = F_SMALL;
         else role = w_lo <= 0 ? F_LARGE : F_NONE;
         if (w_lo <= 0 && last_tid == 0) role = ROLE_GENERAL;
     }
@@ -123,14 +137,14 @@ __global__ void __launch_bounds__(T, MINB) shkadov_kernel(const ShkArgs<R> a)
     // jets: when consecutive jet zones are at least C-1 points apart a chunk meets at most one jet
     int myjet = -1;
     if (a.jets_simple && nj > 0) {
-        int j = (a0 + C - 1 - a.jz0) / a.jet_space;      // last jet starting at or before my last point
-        if (a0 + C - 1 >= a.jz0) {
+        int j = (a0 + cw - 1 - a.jz0) / a.jet_space;     // last jet starting at or before my last point
+        if (a0 + cw - 1 >= a.jz0) {
             if (j >= nj) j = nj - 1;
             if (a0 <= a.jz0 + j * a.jet_space + 2 * a.jet_hw) myjet = j;
         }
     }
     const int kb = a0 - a.jz0 + C;                       // my first point in the zero-padded weight table
-    const bool edge_thread = (a0 <= 0) || (a0 <= nx - 1 && a0 + C - 1 >= nx - 1);   // owns point 0 or nx-1
+    const bool edge_thread = (a0 <= 0) || (a0 <= nx - 1 && a0 + cw - 1 >= nx - 1);  // owns point 0 or nx-1
 
     // jet zone tables (shkadov.py:224-232): weight v = (k-s)(e-k)/(0.25 (e-s)^2)
     for (int k = tid; k < a.jz_len; k += T) {
@@ -150,13 +164,13 @@ __global__ void __launch_bounds__(T, MINB) shkadov_kernel(const ShkArgs<R> a)
     for (int k = tid; k < 2 * XN * T; k += T) ex[k] = R(1);   // slots of threads beyond the domain are read (and discarded): keep them finite
 
     // ---- load state into registers ----------------------------------------------------
-    R hv[C], qv[C], rh[C], rq[C];
+    R hv[C], qv[C], rh[C], rq[C];                       // entries m >= cw unused
     const size_t row = (size_t)b * nx;
     const bool resetting = a.mode == 1;
 #pragma unroll
     for (int m = 0; m < C; m++) {
         int i = a0 + m;
-        bool real = i >= 0 && i < nx;
+        bool real = i >= 0 && i < nx && m < cw;
         if (resetting) {                                 // reset_fields + load, shkadov.py:113-151
             hv[m] = real ? a.h_init[i] : R(1);
             qv[m] = real ? a.q_init[i] : R(1);
@@ -193,38 +207,41 @@ __global__ void __launch_bounds__(T, MINB) shkadov_kernel(const ShkArgs<R> a)
         draws += (unsigned long long)a.ndt_act;
         __syncthreads();
 
-        // One sub-step of a chunk, shkadov.py:199-236.  KIND is the warp role.
-        auto substep = [&](const int it, auto kind_tag) {
+        // One sub-step of a chunk, shkadov.py:199-236.  KIND is the warp role, CW the width of the chunk
+        // (C or CN).  In the balanced layout only the C half holds the inlet and only the CN half the outlet.
+        auto substep = [&](const int it, auto kind_tag, auto width_tag) {
             constexpr int KIND = decltype(kind_tag)::value;
+            constexpr int CW = decltype(width_tag)::value;
             constexpr bool FAST = KIND != ROLE_GENERAL;
+            constexpr bool INLET = !(BAL && CW == CN), OUTLET = !(BAL && CW == C);
             const int buf = it & 1;
             R *X = ex + buf * XN * T;
             // ---- boundary conditions, shkadov.py:204-207 -------------------------------
-            if (KIND == F_SMALL || KIND == F_LARGE) {
+            if ((KIND == F_SMALL || KIND == F_LARGE) && INLET) {
                 const R hin = R(1) + s_noise[it];
 #pragma unroll
-                for (int m = 0; m < (KIND == F_SMALL ? 2 : C); m++)
+                for (int m = 0; m < (KIND == F_SMALL ? SMALL_OFF + 1 : CW); m++)
                     if (m < np) { hv[m] = hin; qv[m] = R(1); }           // point 0 (and the phantom points left of it)
             }
             if (FAST) {
-                if (is_last) { hv[C - 1] = hv[C - 2]; qv[C - 1] = qv[C - 2]; }
+                if (OUTLET && is_last) { hv[CW - 1] = hv[CW - 2]; qv[CW - 1] = qv[CW - 2]; }
             } else if (edge_thread) {
 #pragma unroll
-                for (int m = 0; m < C; m++) {
+                for (int m = 0; m < CW; m++) {
                     int i = a0 + m;
                     if (i == 0) { hv[m] = R(1) + s_noise[it]; qv[m] = R(1); }
                     if (m > 0 && i == nx - 1) { hv[m] = hv[m - 1]; qv[m] = qv[m - 1]; }   // off guarantees m > 0
                 }
             }
             // ---- q2h = q*q/(h+eps), shkadov.py:213 --------------------------------------
-            R zv[C];
+            R zv[CW];
 #pragma unroll
-            for (int m = 0; m < C; m++) zv[m] = fdiv(qv[m] * qv[m], hv[m] + a.eps);
+            for (int m = 0; m < CW; m++) zv[m] = fdiv(qv[m] * qv[m], hv[m] + a.eps);
             // ---- publish chunk edges ---------------------------------------------------
             X[XH0 * T + tid] = hv[0]; X[XH1 * T + tid] = hv[1]; X[XH2 * T + tid] = hv[2];
-            X[XHL2 * T + tid] = hv[C - 2]; X[XHL1 * T + tid] = hv[C - 1];
-            X[XQ0 * T + tid] = qv[0]; X[XQL2 * T + tid] = qv[C - 2]; X[XQL1 * T + tid] = qv[C - 1];
-            X[XZ0 * T + tid] = zv[0]; X[XZL2 * T + tid] = zv[C - 2]; X[XZL1 * T + tid] = zv[C - 1];
+            X[XHL2 * T + tid] = hv[CW - 2]; X[XHL1 * T + tid] = hv[CW - 1];
+            X[XQ0 * T + tid] = qv[0]; X[XQL2 * T + tid] = qv[CW - 2]; X[XQL1 * T + tid] = qv[CW - 1];
+            X[XZ0 * T + tid] = zv[0]; X[XZL2 * T + tid] = zv[CW - 2]; X[XZL1 * T + tid] = zv[CW - 1];
             // jet amplitudes of this sub-step, shkadov.py:224-226
             if (!FAST) {
                 if (!a.jets_simple && (tid < nj || nj > T)) {
@@ -241,26 +258,26 @@ __global__ void __launch_bounds__(T, MINB) shkadov_kernel(const ShkArgs<R> a)
                 constexpr int UK = decltype(upd_tag)::value;
                 constexpr bool UFAST = UK == F_NONE || UK == F_SMALL || UK == F_LARGE;
                 // ---- extended stencils ---------------------------------------------------
-                R uh[C + 5];   // h at a0-2 .. a0+C+2
+                R uh[CW + 5];   // h at a0-2 .. a0+CW+2
                 uh[0] = X[XHL2 * T + tl]; uh[1] = X[XHL1 * T + tl];
 #pragma unroll
-                for (int m = 0; m < C; m++) uh[m + 2] = hv[m];
-                uh[C + 2] = X[XH0 * T + tr]; uh[C + 3] = X[XH1 * T + tr]; uh[C + 4] = X[XH2 * T + tr];
-                R uq[C + 3], uz[C + 3];   // q, q2h at a0-2 .. a0+C
+                for (int m = 0; m < CW; m++) uh[m + 2] = hv[m];
+                uh[CW + 2] = X[XH0 * T + tr]; uh[CW + 3] = X[XH1 * T + tr]; uh[CW + 4] = X[XH2 * T + tr];
+                R uq[CW + 3], uz[CW + 3];   // q, q2h at a0-2 .. a0+CW
                 uq[0] = X[XQL2 * T + tl]; uq[1] = X[XQL1 * T + tl];
                 uz[0] = X[XZL2 * T + tl]; uz[1] = X[XZL1 * T + tl];
 #pragma unroll
-                for (int m = 0; m < C; m++) { uq[m + 2] = qv[m]; uz[m + 2] = zv[m]; }
-                uq[C + 2] = X[XQ0 * T + tr]; uz[C + 2] = X[XZ0 * T + tr];
+                for (int m = 0; m < CW; m++) { uq[m + 2] = qv[m]; uz[m + 2] = zv[m]; }
+                uq[CW + 2] = X[XQ0 * T + tr]; uz[CW + 2] = X[XZ0 * T + tr];
 
                 // ---- TVD faces (d1tvd, shkadov.py:494-504): F_f = u_f + 0.5 phi_f (u_{f+1}-u_f) ----
-                R Fq[C + 1], Fz[C + 1];   // faces a0-1 .. a0+C-1
+                R Fq[CW + 1], Fz[CW + 1];   // faces a0-1 .. a0+CW-1
                 {
-                    R dq[C + 2], dz[C + 2];   // differences u_{k+1}-u_k for k = a0-2 .. a0+C-1
+                    R dq[CW + 2], dz[CW + 2];   // differences u_{k+1}-u_k for k = a0-2 .. a0+CW-1
 #pragma unroll
-                    for (int k = 0; k < C + 2; k++) { dq[k] = uq[k + 1] - uq[k]; dz[k] = uz[k + 1] - uz[k]; }
+                    for (int k = 0; k < CW + 2; k++) { dq[k] = uq[k + 1] - uq[k]; dz[k] = uz[k + 1] - uz[k]; }
 #pragma unroll
-                    for (int m = 0; m < C + 1; m++) {
+                    for (int m = 0; m < CW + 1; m++) {
                         // half of the minmod limiter, 0.5 max(0, min(r, 1)) with r = d_m / (d_{m+1} + 1e-8), as
                         // d_m / (2 d_{m+1} + 2e-8): doubling the divisor is exact and costs nothing (an FMA in place of
                         // the DADD), and the reciprocal seed of 2b is the seed of b with its exponent lowered by one, so
@@ -270,7 +287,7 @@ __global__ void __launch_bounds__(T, MINB) shkadov_kernel(const ShkArgs<R> a)
                         if (UK == ROLE_GENERAL) { if (a0 - 1 + m <= 0) { pq = R(0); pz = R(0); } }   // phi[0] = 0
                         // F_SMALL needs no select for phi[0] = 0.  The inlet face is face zf-1 of thread 0, and both of
                         // its differences are exactly 0 there: with off = 0 the ghost left of the inlet point is that
-                        // point (tl), with off = 1 the phantom point carries the inlet values.  A zero numerator gives
+                        // point (tl), with off >= 1 the phantom point left of it carries the inlet values.  A zero numerator gives
                         // pq = pz = +0 unless the divisor is exactly 0; for q that cannot happen (q_0 = 1), for q2h it
                         // needs |q2h_0| < 2^-24, an inlet depth above 1.6e7.  The faces left of it feed only points
                         // that are not updated.
@@ -288,18 +305,18 @@ __global__ void __launch_bounds__(T, MINB) shkadov_kernel(const ShkArgs<R> a)
                 }
                 const R hdt = a.hdt;
 #pragma unroll
-                for (int m = 0; m < C; m++) {
+                for (int m = 0; m < CW; m++) {
                     const int i = a0 + m;
                     R nrh = (Fq[m + 1] - Fq[m]) * a.inv_dx;                       // rhsh = d1tvd(q)
                     const R hh = hv[m];
                     R nrq;
                     if (UFAST) {
                         R d3p1 = (-uh[m + 5] + R(6) * uh[m + 4] - R(12) * uh[m + 3] + R(10) * uh[m + 2] - R(3) * uh[m + 1]) * a.inv_2dx3 + R(1);
-                        if (m == C - 3) {                         // i = nx-3 / nx-2 of the outlet chunk: one-sided closures
+                        if (OUTLET && m == CW - 3) {              // i = nx-3 / nx-2 of the outlet chunk: one-sided closures
                             R c = fma(a.kc, uh[m + 4], R(1)); c = fma(-a.kc3, uh[m + 3], c); c = fma(a.kc3, uh[m + 2], c); c = fma(-a.kc, uh[m + 1], c);
                             if (is_last) d3p1 = c;
                         }
-                        if (m == C - 2) {
+                        if (OUTLET && m == CW - 2) {
                             R c = fma(-a.kc, uh[m], R(1)); c = fma(a.kc3, uh[m + 1], c); c = fma(-a.kc3, uh[m + 2], c); c = fma(a.kc, uh[m + 3], c);
                             if (is_last) d3p1 = c;
                         }
@@ -333,9 +350,9 @@ __global__ void __launch_bounds__(T, MINB) shkadov_kernel(const ShkArgs<R> a)
                         }
                     }
                     bool upd = true;                                              // adams(), :515-518: points 1 .. nx-2
-                    if (UK == F_SMALL && m < 2) upd = m >= np;
+                    if (UK == F_SMALL && INLET && m <= SMALL_OFF) upd = m >= np;
                     if (UK == F_LARGE) upd = m >= np;
-                    if (UFAST && m == C - 1) upd = upd && !is_last;
+                    if (UFAST && OUTLET && m == CW - 1) upd = upd && !is_last;
                     if (UK == ROLE_GENERAL) upd = i >= 1 && i <= nx - 2;
                     if (upd) {
                         hv[m] = hh + hdt * (R(-3) * nrh + rh[m]);
@@ -349,25 +366,40 @@ __global__ void __launch_bounds__(T, MINB) shkadov_kernel(const ShkArgs<R> a)
             else if (interior_thread) update(std::integral_constant<int, -1>{});
             else if (a0 < nx) update(std::integral_constant<int, ROLE_GENERAL>{});
         };
+        using WideC = std::integral_constant<int, C>;
+        using NarrowC = std::integral_constant<int, CN>;
 
         // The single-body case runs the sub-step loop unrolled by two: the register rotation of the state
         // arrays (old values are still needed while the new ones are formed) then costs no copies
         // (+13 % measured).  With two bodies resident (F_LARGE + F_NONE) the unrolled pair does not pay
-        // (instruction-cache footprint), they run one sub-step per trip.
+        // (instruction-cache footprint), they run one sub-step per trip.  The balanced layout has two
+        // unrolled bodies, one per width, of about 15 and 12 KB: both loops come first, next to each other,
+        // and the sub-step an odd ndt_act leaves over after them.
         auto run_fast = [&](auto tag, auto unroll_tag) {
             int it = 0;
             if (decltype(unroll_tag)::value)
-                for (; it + 1 < a.ndt_act; it += 2) { substep(it, tag); substep(it + 1, tag); }
-            for (; it < a.ndt_act; it++) substep(it, tag);
+                for (; it + 1 < a.ndt_act; it += 2) { substep(it, tag, WideC{}); substep(it + 1, tag, WideC{}); }
+            for (; it < a.ndt_act; it++) substep(it, tag, WideC{});
         };
-        if (role == F_SMALL) {
-            run_fast(std::integral_constant<int, F_SMALL>{}, std::true_type{});
-        } else if (role == F_NONE) {
+        if (BAL && role == F_SMALL) {
+            using Small = std::integral_constant<int, F_SMALL>;
+            int it = 0;
+            if (narrow)
+                for (; it + 1 < a.ndt_act; it += 2) { substep(it, Small{}, NarrowC{}); substep(it + 1, Small{}, NarrowC{}); }
+            else
+                for (; it + 1 < a.ndt_act; it += 2) { substep(it, Small{}, WideC{}); substep(it + 1, Small{}, WideC{}); }
+            if (it < a.ndt_act) {
+                if (narrow) substep(it, Small{}, NarrowC{});
+                else substep(it, Small{}, WideC{});
+            }
+        } else if (!BAL && role == F_SMALL) {      // (the host selects the balanced layout only where every warp
+            run_fast(std::integral_constant<int, F_SMALL>{}, std::true_type{});   // holding points runs F_SMALL)
+        } else if (!BAL && role == F_NONE) {
             run_fast(std::integral_constant<int, F_NONE>{}, std::false_type{});
-        } else if (role == F_LARGE) {
+        } else if (!BAL && role == F_LARGE) {
             run_fast(std::integral_constant<int, F_LARGE>{}, std::false_type{});
-        } else if (role == ROLE_GENERAL) {
-            for (int it = 0; it < a.ndt_act; it++) substep(it, std::integral_constant<int, ROLE_GENERAL>{});
+        } else if (!BAL && role == ROLE_GENERAL) {
+            for (int it = 0; it < a.ndt_act; it++) substep(it, std::integral_constant<int, ROLE_GENERAL>{}, WideC{});
         } else {
             for (int it = 0; it < a.ndt_act; it++) {           // beyond the domain: jets table duty, barrier count
                 if (!a.jets_simple) {
@@ -385,7 +417,7 @@ __global__ void __launch_bounds__(T, MINB) shkadov_kernel(const ShkArgs<R> a)
 #pragma unroll
         for (int m = 0; m < C; m++) {
             int i = a0 + m;
-            if (i >= 0 && i < nx) {
+            if (i >= 0 && i < nx && m < cw) {
                 s_h[i] = hv[m];
                 s_q[i] = qv[m];
                 bad |= (hv[m] < a.blow_lo) | (hv[m] > a.blow_hi);              // shkadov.py:176
@@ -441,7 +473,7 @@ __global__ void __launch_bounds__(T, MINB) shkadov_kernel(const ShkArgs<R> a)
         // plain reset: observation of the init state
         __syncthreads();
 #pragma unroll
-        for (int m = 0; m < C; m++) { int i = a0 + m; if (i >= 0 && i < nx) s_q[i] = qv[m]; }
+        for (int m = 0; m < C; m++) { int i = a0 + m; if (i >= 0 && i < nx && m < cw) s_q[i] = qv[m]; }
         __syncthreads();
         R *obs = a.obs + (size_t)b * (size_t)(nj * a.n_obs);
         for (int e = tid; e < nj * a.n_obs; e += T) {
@@ -454,7 +486,7 @@ __global__ void __launch_bounds__(T, MINB) shkadov_kernel(const ShkArgs<R> a)
 #pragma unroll
     for (int m = 0; m < C; m++) {
         int i = a0 + m;
-        if (i >= 0 && i < nx) {
+        if (i >= 0 && i < nx && m < cw) {
             a.h[row + i] = hv[m]; a.q[row + i] = qv[m]; a.rhsh[row + i] = rh[m]; a.rhsq[row + i] = rq[m];
         }
     }
@@ -469,6 +501,14 @@ __global__ void __launch_bounds__(T, MINB) shkadov_kernel(const ShkArgs<R> a)
         if (a.status) a.status[b] = status;
     }
 }
+
+template <typename R, int C, int T, int MINB>
+__global__ void __launch_bounds__(T, MINB) shkadov_kernel(const ShkArgs<R> a) { shkadov_body<R, C, C, T>(a); }
+
+// The balanced layout under a name of its own, so that tools and tuning switches that name
+// shkadov_kernel<R, C, T, MINB> never reach it.
+template <typename R, int C, int CN, int T, int MINB>
+__global__ void __launch_bounds__(T, MINB) shkadov_balanced_kernel(const ShkArgs<R> a) { shkadov_body<R, C, CN, T>(a); }
 
 // Reset order: CTAs are handed to the SMs in blockIdx order, and a reset with random warm steps
 // (shkadov.py:118-123, U{0..400} actions per env) finishes when its longest env does.  One small CTA
@@ -504,14 +544,30 @@ template <typename R> class ShkadovEnv : public Env {
     beacon_shkadov_params p;
     DeviceBuffer h, q, rhsh, rhsq, u_cur, u_prev, stp, draws, h_init, q_init, order;
     ShkArgs<R> base{};
-    int C = 0, T = 0;
+    int C = 0, CN = 0, T = 0;        // threads [0, T/2) hold C points, [T/2, T) hold CN (uniform: CN = C)
     size_t smem = 0;
     void (*kernel)(const ShkArgs<R>) = nullptr;
 
     template <int CC, int TT, int MB> void pick()
     {
-        C = CC; T = TT;
+        C = CN = CC; T = TT;
         kernel = shkadov_kernel<R, CC, TT, MB>;
+    }
+    template <int CC, int CNN, int TT, int MB> void pick_balanced()
+    {
+        C = CC; CN = CNN; T = TT;
+        kernel = shkadov_balanced_kernel<R, CC, CNN, TT, MB>;
+    }
+    // Chunks are shifted left by `off` phantom points so that the outlet point nx-1 is the last point of its
+    // chunk (the FAST warp roles then have their special cases at compile-time positions).  The balanced
+    // layout puts it into the CN half.
+    static int aligned_off(int nx, int c, int cn, int t) { return cn == c ? (c - nx % c) % c : ((t / 2 * c - nx) % cn + cn) % cn; }
+    // jets far enough apart that a chunk of c points meets at most one
+    static bool jets_simple(const beacon_shkadov_params &p, int c)
+    {
+        const int nj = p.n_jets;
+        const bool overlap = nj > 1 && p.jet_space <= 2 * p.jet_hw;
+        return nj > 0 && p.jet_space > 0 && (nj == 1 || p.jet_space - 2 * p.jet_hw - 1 >= c - 1) && !overlap;
     }
 
 public:
@@ -535,20 +591,31 @@ public:
         info.rwd_dim = p.per_jet_rwd ? nj : 1; info.n_act = p.n_act; info.noise_dim = p.ndt_act;
 
         // (points per thread, threads, min CTAs/SM) variants; the first that covers nx is used
-        // unless BEACON_SHKADOV_CFG="C,T,MINB" selects one explicitly (tuning).
-        int wc = 0, wt = 0, wm = 0;
-        if (const char *e = getenv("BEACON_SHKADOV_CFG")) sscanf(e, "%d,%d,%d", &wc, &wt, &wm);
+        // unless BEACON_SHKADOV_CFG="C,T,MINB" (or "C/CN,T,MINB" for the balanced layout) selects one explicitly (tuning).
+        int wc = 0, wn = 0, wt = 0, wm = 0;
+        if (const char *e = getenv("BEACON_SHKADOV_CFG"))
+            if (sscanf(e, "%d/%d,%d,%d", &wc, &wn, &wt, &wm) != 4) { wn = 0; sscanf(e, "%d,%d,%d", &wc, &wt, &wm); }
+        const bool noalign = getenv("BEACON_SHKADOV_NOALIGN") != nullptr;
         bool ok = false;
+        // The balanced layout only where every warp that holds points runs the unrolled single body: outlet
+        // aligned in the CN half (off <= CN-1 always), jets at most one per chunk.
+#define BEACON_SHK_TRY_BAL(CC, CNN, TT, MB)                                                                          \
+        if (!ok && (wc ? (wc == CC && wn == CNN && wt == TT && wm == MB) : true) && !noalign && jets_simple(p, CC)) { \
+            const int o = aligned_off(nx, CC, CNN, TT);                                                                \
+            if (nx + o > TT / 2 * CC && nx + o <= TT / 2 * (CC + CNN)) { pick_balanced<CC, CNN, TT, MB>(); ok = true; } \
+        }
 #define BEACON_SHK_TRY(CC, TT, MB)                                                             \
-        if (!ok && (wc ? (wc == CC && wt == TT && wm == MB) : true) && (long)CC * TT >= nx + (CC - nx % CC) % CC) { pick<CC, TT, MB>(); ok = true; }
-        // measured on B200 (profiles/sweep_shkadov_r1j_*.txt): 10 jets (nx 1350) 6,256,2; 20 jets (nx 1850)
-        // 10,192,2; 41 jets (nx 2900) 6,512,1
+        if (!ok && (wc ? (wc == CC && wn == 0 && wt == TT && wm == MB) : true) && (long)CC * TT >= nx + (CC - nx % CC) % CC) { pick<CC, TT, MB>(); ok = true; }
+        // measured on B200 (profiles/sweep_shkadov_r1j_*.txt, profiles/r3_shkadov_balanced_ab.txt): 10 jets (nx 1350)
+        // 6/5,256,2; 20 jets (nx 1850) 10,192,2; 41 jets (nx 2900) 6,512,1
+        BEACON_SHK_TRY_BAL(6, 5, 256, 2)
         BEACON_SHK_TRY(6, 256, 2)
         if (wc) { BEACON_SHK_TRY(9, 160, 3) BEACON_SHK_TRY(9, 160, 2) BEACON_SHK_TRY(11, 128, 3) BEACON_SHK_TRY(11, 128, 2) BEACON_SHK_TRY(5, 640, 1) BEACON_SHK_TRY(10, 320, 1) }   // tuning only
         BEACON_SHK_TRY(10, 192, 2)
         BEACON_SHK_TRY(6, 512, 1)
         BEACON_SHK_TRY(12, 512, 1)
 #undef BEACON_SHK_TRY
+#undef BEACON_SHK_TRY_BAL
         if (!ok) throw Error(BEACON_ERR_UNSUPPORTED, "shkadov: no kernel variant covers this nx (max about 6130) or BEACON_SHKADOV_CFG is unknown");
 
         size_t nb = (size_t)B * nx * sizeof(R);
@@ -564,18 +631,16 @@ public:
         a.nx = nx; a.ndt_act = p.ndt_act; a.n_act = p.n_act; a.n_interp = p.n_interp; a.n_jets = nj;
         a.jet_pos = p.jet_pos; a.jet_hw = p.jet_hw; a.jet_space = p.jet_space; a.l_obs = p.l_obs; a.n_obs = p.n_obs;
         a.obs_stride = p.obs_stride; a.l_rwd = p.l_rwd; a.per_jet_rwd = p.per_jet_rwd;
-        // Chunks are shifted left by `off` phantom points so that the outlet point nx-1 is the last point
-        // of its chunk (the LAST warp role then has its special cases at compile-time positions).
-        a.off = (C - nx % C) % C;
+        a.off = aligned_off(nx, C, CN, T);
         a.tail_aligned = 1;
-        if ((size_t)T * C < (size_t)nx + a.off || getenv("BEACON_SHKADOV_NOALIGN")) {   // no room: old layout, general path
+        if ((size_t)T * C < (size_t)nx + a.off || noalign) {   // no room: old layout, general path (never balanced)
             a.off = ((nx - 1) % C == 0) ? 1 : 0;         // keep points nx-2 and nx-1 in one chunk
             a.tail_aligned = 0;
         }
-        BEACON_REQUIRE((size_t)T * C - a.off >= (size_t)nx, "shkadov: internal chunking error");
+        BEACON_REQUIRE((size_t)T / 2 * (C + CN) - a.off >= (size_t)nx, "shkadov: internal chunking error");
         a.jets_overlap = (nj > 1 && p.jet_space <= 2 * p.jet_hw) ? 1 : 0;
         a.jz0 = p.jet_pos - p.jet_hw;
-        a.jets_simple = (nj > 0 && p.jet_space > 0 && (nj == 1 || p.jet_space - 2 * p.jet_hw - 1 >= C - 1) && !a.jets_overlap) ? 1 : 0;
+        a.jets_simple = jets_simple(p, C) ? 1 : 0;
         a.jz_len = nj > 0 ? (nj - 1) * p.jet_space + 2 * p.jet_hw + 1 : 0;
         a.inv_dx = (R)(1.0 / p.dx); a.inv_2dx3 = (R)(1.0 / (2.0 * p.dx * p.dx * p.dx)); a.inv_dx3 = (R)(1.0 / (p.dx * p.dx * p.dx));
         {

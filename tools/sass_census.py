@@ -100,7 +100,8 @@ def census():
     # ---- shkadov: the sub-step loop of the single-body kernel is unrolled by two (2 barriers per trip) ------
     f = functions(os.path.join(OBJ, "shkadov.o"))
     for tag, needles in (("shkadov_6_256_2", ("shkadov_kernel", "IdLi6ELi256ELi2E")), ("shkadov_6_512_1", ("shkadov_kernel", "IdLi6ELi512ELi1E")),
-                         ("shkadov_10_192_2", ("shkadov_kernel", "IdLi10ELi192ELi2E"))):
+                         ("shkadov_10_192_2", ("shkadov_kernel", "IdLi10ELi192ELi2E")),
+                         ("shkadov_6_5_256_2", ("shkadov_balanced_kernel", "IdLi6ELi5ELi256ELi2E"))):
         name, ins = find(f, *needles)
         cand = []
         for lo, hi in loops_of(ins):
@@ -113,6 +114,8 @@ def census():
         two = [c for c in cand if c["bar"] == 2]
         one = sorted((c for c in cand if c["bar"] == 1), key=lambda c: c["fp64"])
         out[tag] = {"kernel": name, "substep_unrolled2": two[0] if two else None, "substep_bodies": one}
+        if len(two) > 1:   # balanced layout: one unrolled body per chunk width, the wider (more fp64) first
+            out[tag]["substep_unrolled2_per_width"] = sorted(two, key=lambda c: -c["fp64"])
     # ---- rayleigh / mixing: sweep loop (2 sweeps, 2 barriers per trip) inside the sub-step loop -----------------
     f = functions(os.path.join(OBJ, "mac2d.o"))
     for tag, needles in (("rayleigh_reg", ("mac_reg_kernel", "IdLi50ELi50ELi2ELi5ELi256ELb0E")),
@@ -157,4 +160,6 @@ if __name__ == "__main__":
             else:
                 u2 = v["substep_unrolled2"]
                 print(k, "unrolled2 per sub-step:", u2 and u2["per_substep"], "| one-barrier bodies fp64:", [c["fp64"] for c in v["substep_bodies"]])
+                for c in v.get("substep_unrolled2_per_width", []):
+                    print("   unrolled2 body", c["range"], "instr", c["instr"], "fp64", c["fp64"])
     print("wrote", dst)
