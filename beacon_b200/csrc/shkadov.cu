@@ -60,16 +60,18 @@ template <typename R> struct ShkArgs {
 enum { XH0 = 0, XH1, XH2, XHL2, XHL1, XQ0, XQL2, XQL1, XZ0, XZL2, XZL1, XN };
 
 // Chunk widths: threads [0, TH) hold C points each, threads [TH, T) hold CN.  CN == C is the uniform
-// layout (TH = T).  CN == C - 1 is the balanced layout (TH = T / 2): warps w and w + T/64 of a CTA run on
-// the same SM sub-partition, so every sub-partition then carries one C-point and one CN-point warp
-// instead of two C-point warps, and fewer phantom points fill the last warp (DESIGN.md §3.1).
-template <typename R, int C, int CN, int T>
+// layout (TH = T).  CN == C - 1 is the balanced layout (TH a multiple of 32 below T): warps w and w + 4 of
+// a CTA run on the same SM sub-partition, so a sub-partition then carries at most one C-point warp per
+// CTA instead of two, and fewer phantom points fill the last warp (DESIGN.md §3.1).  SMALL_OFF is the
+// largest chunk shift `off` the host hands to this instance: the inlet selects of thread 0 reach m <= SMALL_OFF.
+template <typename R, int C, int CN, int T, int TH, int SMALL_OFF>
 __device__ __forceinline__ void shkadov_body(const ShkArgs<R> &a)
 {
     static_assert(CN >= 3, "halo exchange needs at least 3 points per thread");
-    static_assert(CN == C || (CN == C - 1 && T % 64 == 0), "balanced layout: CN = C - 1, warp-aligned halves");
+    static_assert(CN == C ? TH == T && SMALL_OFF == 1 : CN == C - 1 && TH % 32 == 0 && 0 < TH && TH < T,
+                  "balanced layout: CN = C - 1, the split warp-aligned");
+    static_assert(SMALL_OFF >= 1 && SMALL_OFF < CN, "inlet reach");
     constexpr bool BAL = CN != C;
-    constexpr int TH = BAL ? T / 2 : T;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int tid = threadIdx.x, b = a.order ? a.order[blockIdx.x] : (int)blockIdx.x;
     const int nx = a.nx, nj = a.n_jets;
@@ -111,15 +113,15 @@ __device__ __forceinline__ void shkadov_body(const ShkArgs<R> &a)
     //            inlet point 0 and the faces with phi = 0: selects on per-thread thresholds (zero for
     //            everybody else), confined to the points m <= SMALL_OFF when off <= SMALL_OFF (F_SMALL,
     //            whose faces need none), or for all m in warp 0 (F_LARGE) while the other warps run the
-    //            body without them (F_NONE).  The balanced layout has off <= CN - 1 = SMALL_OFF always:
-    //            both of its widths run F_SMALL, unrolled (its inlet lies in the C half, the outlet in
-    //            the CN half, so each width carries only its own specials).  Lanes beyond
+    //            body without them (F_NONE).  The balanced layout runs only where the host has
+    //            off <= SMALL_OFF (CN - 1 covers every off, 1 the split whose off is 0 or 1): both of its
+    //            widths run F_SMALL, unrolled (its inlet lies in the C part, the outlet in the CN part, so
+    //            each width carries only its own specials).  Lanes beyond
     //            the domain run the same arithmetic on phantom points (never stored, never read by
     //            a result that is kept);
     //   IDLE     warps entirely beyond the domain only keep the barrier count;
     //   GENERAL  anything else (tiny lattices, overlapping / dense jets): per-point index tests.
     enum { F_NONE = 0, F_SMALL, F_LARGE, ROLE_GENERAL, ROLE_IDLE };
-    constexpr int SMALL_OFF = BAL ? CN - 1 : 1;
     const int w_lo = first_point(tid & ~31);
     const int lp = nx - 1 + a.off;                      // outlet point counted from the first phantom point
     const int last_tid = BAL && lp >= TH * C ? TH + (lp - TH * C) / CN : lp / C;
@@ -208,7 +210,7 @@ __device__ __forceinline__ void shkadov_body(const ShkArgs<R> &a)
         __syncthreads();
 
         // One sub-step of a chunk, shkadov.py:199-236.  KIND is the warp role, CW the width of the chunk
-        // (C or CN).  In the balanced layout only the C half holds the inlet and only the CN half the outlet.
+        // (C or CN).  In the balanced layout only the C part holds the inlet and only the CN part the outlet.
         auto substep = [&](const int it, auto kind_tag, auto width_tag) {
             constexpr int KIND = decltype(kind_tag)::value;
             constexpr int CW = decltype(width_tag)::value;
@@ -503,12 +505,12 @@ __device__ __forceinline__ void shkadov_body(const ShkArgs<R> &a)
 }
 
 template <typename R, int C, int T, int MINB>
-__global__ void __launch_bounds__(T, MINB) shkadov_kernel(const ShkArgs<R> a) { shkadov_body<R, C, C, T>(a); }
+__global__ void __launch_bounds__(T, MINB) shkadov_kernel(const ShkArgs<R> a) { shkadov_body<R, C, C, T, T, 1>(a); }
 
 // The balanced layout under a name of its own, so that tools and tuning switches that name
 // shkadov_kernel<R, C, T, MINB> never reach it.
-template <typename R, int C, int CN, int T, int MINB>
-__global__ void __launch_bounds__(T, MINB) shkadov_balanced_kernel(const ShkArgs<R> a) { shkadov_body<R, C, CN, T>(a); }
+template <typename R, int C, int CN, int T, int MINB, int TH, int SMALL_OFF>
+__global__ void __launch_bounds__(T, MINB) shkadov_balanced_kernel(const ShkArgs<R> a) { shkadov_body<R, C, CN, T, TH, SMALL_OFF>(a); }
 
 // Reset order: CTAs are handed to the SMs in blockIdx order, and a reset with random warm steps
 // (shkadov.py:118-123, U{0..400} actions per env) finishes when its longest env does.  One small CTA
@@ -544,24 +546,24 @@ template <typename R> class ShkadovEnv : public Env {
     beacon_shkadov_params p;
     DeviceBuffer h, q, rhsh, rhsq, u_cur, u_prev, stp, draws, h_init, q_init, order;
     ShkArgs<R> base{};
-    int C = 0, CN = 0, T = 0;        // threads [0, T/2) hold C points, [T/2, T) hold CN (uniform: CN = C)
+    int C = 0, CN = 0, T = 0, TH = 0;   // threads [0, TH) hold C points, [TH, T) hold CN (uniform: CN = C, TH = T)
     size_t smem = 0;
     void (*kernel)(const ShkArgs<R>) = nullptr;
 
     template <int CC, int TT, int MB> void pick()
     {
-        C = CN = CC; T = TT;
+        C = CN = CC; T = TH = TT;
         kernel = shkadov_kernel<R, CC, TT, MB>;
     }
-    template <int CC, int CNN, int TT, int MB> void pick_balanced()
+    template <int CC, int CNN, int TT, int MB, int THH, int SO> void pick_balanced()
     {
-        C = CC; CN = CNN; T = TT;
-        kernel = shkadov_balanced_kernel<R, CC, CNN, TT, MB>;
+        C = CC; CN = CNN; T = TT; TH = THH;
+        kernel = shkadov_balanced_kernel<R, CC, CNN, TT, MB, THH, SO>;
     }
     // Chunks are shifted left by `off` phantom points so that the outlet point nx-1 is the last point of its
     // chunk (the FAST warp roles then have their special cases at compile-time positions).  The balanced
-    // layout puts it into the CN half.
-    static int aligned_off(int nx, int c, int cn, int t) { return cn == c ? (c - nx % c) % c : ((t / 2 * c - nx) % cn + cn) % cn; }
+    // layout puts it into the CN part.
+    static int aligned_off(int nx, int c, int cn, int th) { return cn == c ? (c - nx % c) % c : ((th * c - nx) % cn + cn) % cn; }
     // jets far enough apart that a chunk of c points meets at most one
     static bool jets_simple(const beacon_shkadov_params &p, int c)
     {
@@ -591,24 +593,34 @@ public:
         info.rwd_dim = p.per_jet_rwd ? nj : 1; info.n_act = p.n_act; info.noise_dim = p.ndt_act;
 
         // (points per thread, threads, min CTAs/SM) variants; the first that covers nx is used
-        // unless BEACON_SHKADOV_CFG="C,T,MINB" (or "C/CN,T,MINB" for the balanced layout) selects one explicitly (tuning).
-        int wc = 0, wn = 0, wt = 0, wm = 0;
+        // unless BEACON_SHKADOV_CFG="C,T,MINB" (or "C/CN,T,MINB" for the balanced layout split at T/2, "C/CN@TH,T,MINB"
+        // split at thread TH) selects one explicitly (tuning).
+        int wc = 0, wn = 0, wh = 0, wt = 0, wm = 0;
         if (const char *e = getenv("BEACON_SHKADOV_CFG"))
-            if (sscanf(e, "%d/%d,%d,%d", &wc, &wn, &wt, &wm) != 4) { wn = 0; sscanf(e, "%d,%d,%d", &wc, &wt, &wm); }
+            if (sscanf(e, "%d/%d@%d,%d,%d", &wc, &wn, &wh, &wt, &wm) != 5) {
+                wh = 0;
+                if (sscanf(e, "%d/%d,%d,%d", &wc, &wn, &wt, &wm) != 4) { wn = 0; sscanf(e, "%d,%d,%d", &wc, &wt, &wm); }
+            }
         const bool noalign = getenv("BEACON_SHKADOV_NOALIGN") != nullptr;
         bool ok = false;
         // The balanced layout only where every warp that holds points runs the unrolled single body: outlet
-        // aligned in the CN half (off <= CN-1 always), jets at most one per chunk.
-#define BEACON_SHK_TRY_BAL(CC, CNN, TT, MB)                                                                          \
-        if (!ok && (wc ? (wc == CC && wn == CNN && wt == TT && wm == MB) : true) && !noalign && jets_simple(p, CC)) { \
-            const int o = aligned_off(nx, CC, CNN, TT);                                                                \
-            if (nx + o > TT / 2 * CC && nx + o <= TT / 2 * (CC + CNN)) { pick_balanced<CC, CNN, TT, MB>(); ok = true; } \
+        // aligned in the CN part, off within the instance's inlet reach SO, jets at most one per chunk.
+#define BEACON_SHK_TRY_BAL(CC, CNN, TT, MB, THH, SO)                                                                  \
+        if (!ok && (wc ? (wc == CC && wn == CNN && (wh ? wh : wt / 2) == THH && wt == TT && wm == MB) : true) &&       \
+            !noalign && jets_simple(p, CC)) {                                                                          \
+            const int o = aligned_off(nx, CC, CNN, THH);                                                               \
+            if (o <= SO && nx + o > THH * CC && nx + o <= THH * CC + (TT - THH) * CNN) {                              \
+                pick_balanced<CC, CNN, TT, MB, THH, SO>(); ok = true;                                                  \
+            }                                                                                                          \
         }
 #define BEACON_SHK_TRY(CC, TT, MB)                                                             \
         if (!ok && (wc ? (wc == CC && wn == 0 && wt == TT && wm == MB) : true) && (long)CC * TT >= nx + (CC - nx % CC) % CC) { pick<CC, TT, MB>(); ok = true; }
-        // measured on B200 (profiles/sweep_shkadov_r1j_*.txt, profiles/r3_shkadov_balanced_ab.txt): 10 jets (nx 1350)
-        // 6/5,256,2; 20 jets (nx 1850) 10,192,2; 41 jets (nx 2900) 6,512,1
-        BEACON_SHK_TRY_BAL(6, 5, 256, 2)
+        // measured on B200 (profiles/sweep_shkadov_r1j_*.txt, profiles/r3_shkadov_balanced_ab.txt,
+        // profiles/r3_shkadov_split_ab.txt): 10 jets (nx 1350) 6/5@96,256,2; 20 jets (nx 1850) 10,192,2; 41 jets (nx 2900) 6,512,1.
+        // 6/5@96 (warps 0-2 wide) takes off = (576 - nx) mod 5 <= 1, which needs no inlet selects beyond m = 1; 6/5 split
+        // at 128 takes every off (inlet selects up to m = 4).
+        BEACON_SHK_TRY_BAL(6, 5, 256, 2, 96, 1)
+        BEACON_SHK_TRY_BAL(6, 5, 256, 2, 128, 4)
         BEACON_SHK_TRY(6, 256, 2)
         if (wc) { BEACON_SHK_TRY(9, 160, 3) BEACON_SHK_TRY(9, 160, 2) BEACON_SHK_TRY(11, 128, 3) BEACON_SHK_TRY(11, 128, 2) BEACON_SHK_TRY(5, 640, 1) BEACON_SHK_TRY(10, 320, 1) }   // tuning only
         BEACON_SHK_TRY(10, 192, 2)
@@ -631,13 +643,13 @@ public:
         a.nx = nx; a.ndt_act = p.ndt_act; a.n_act = p.n_act; a.n_interp = p.n_interp; a.n_jets = nj;
         a.jet_pos = p.jet_pos; a.jet_hw = p.jet_hw; a.jet_space = p.jet_space; a.l_obs = p.l_obs; a.n_obs = p.n_obs;
         a.obs_stride = p.obs_stride; a.l_rwd = p.l_rwd; a.per_jet_rwd = p.per_jet_rwd;
-        a.off = aligned_off(nx, C, CN, T);
+        a.off = aligned_off(nx, C, CN, TH);
         a.tail_aligned = 1;
         if ((size_t)T * C < (size_t)nx + a.off || noalign) {   // no room: old layout, general path (never balanced)
             a.off = ((nx - 1) % C == 0) ? 1 : 0;         // keep points nx-2 and nx-1 in one chunk
             a.tail_aligned = 0;
         }
-        BEACON_REQUIRE((size_t)T / 2 * (C + CN) - a.off >= (size_t)nx, "shkadov: internal chunking error");
+        BEACON_REQUIRE((size_t)TH * C + (size_t)(T - TH) * CN - a.off >= (size_t)nx, "shkadov: internal chunking error");
         a.jets_overlap = (nj > 1 && p.jet_space <= 2 * p.jet_hw) ? 1 : 0;
         a.jz0 = p.jet_pos - p.jet_hw;
         a.jets_simple = jets_simple(p, C) ? 1 : 0;

@@ -101,7 +101,8 @@ def census():
     f = functions(os.path.join(OBJ, "shkadov.o"))
     for tag, needles in (("shkadov_6_256_2", ("shkadov_kernel", "IdLi6ELi256ELi2E")), ("shkadov_6_512_1", ("shkadov_kernel", "IdLi6ELi512ELi1E")),
                          ("shkadov_10_192_2", ("shkadov_kernel", "IdLi10ELi192ELi2E")),
-                         ("shkadov_6_5_256_2", ("shkadov_balanced_kernel", "IdLi6ELi5ELi256ELi2E"))):
+                         ("shkadov_6_5_256_2", ("shkadov_balanced_kernel", "IdLi6ELi5ELi256ELi2ELi128ELi4E")),
+                         ("shkadov_6_5_96_256_2", ("shkadov_balanced_kernel", "IdLi6ELi5ELi256ELi2ELi96ELi1E"))):
         name, ins = find(f, *needles)
         cand = []
         for lo, hi in loops_of(ins):
